@@ -2,7 +2,7 @@
 """Benchmark of the per-view acquisition pipeline (BASELINE.json: simulated voxels/s and views/s,
 achieved HBM GB/s vs peak).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3|cfg1|small]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3|cfg1|small] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch: the 6 views of BASELINE config 3
 (1024x1024x512 float32 ground truth, 6 views 60 deg apart (+15), one 128^3 PSF per view, delta 0.01,
@@ -14,6 +14,11 @@ own batch of 6 views (weak scaling, no data-path collective; views are independe
            memory, ground truth H2D + results D2H inside the timed region.
 `roofline`: the dominant kernel (fused z pass) timed live with CUDA events inside the timed region.
 `cpu_baseline`: the CPU oracle (restatement of the reference; no JVM in this image) on a bounded sample.
+
+--dump-outputs DIR writes what the last timed step of the device-resident arm returned to its caller on rank 0 (every view's
+acquired volume and its PSF, normalised in place; for cfg5 the convolved z slab) as DIR/<name>.npy in float32, so that two builds
+can be compared output for output on identical seeded inputs.  --steps sets the timed steps of every arm (each caller thread of
+the pipelined end-to-end mode runs that many).
 """
 import argparse
 import json
@@ -73,6 +78,27 @@ def make_ground_truth(shape, seed=464232194):
     for k in range(z):          # slab-wise to keep the temporary small
         out[k] = vol[k] * ((zz[k] + yy[:, None] + xx[None, :]) <= 1.0)
     return out
+
+
+DUMP_BYTES = 60 << 20          # --dump-outputs writes at most this much array data in all (< 64 MB)
+
+
+def dump_indices(size, n):
+    """The fixed sample of --dump-outputs: n sorted distinct flat indices out of `size`, from a seeded generator, so that runs of
+    the same workload write the same voxels."""
+    return np.sort(np.random.default_rng(20261020).choice(size, n, replace=False))
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array of {name: array} as out_dir/<name>.npy in float32.  An array larger than its even share of DUMP_BYTES
+    is replaced by its values at dump_indices()."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // (4 * len(arrays))
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float32)
+        if a.size > share:
+            a = a.reshape(-1)[dump_indices(a.size, share)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def make_psfs(kshape, sigma, n):
@@ -349,6 +375,12 @@ def run_ours(args, rank, world, local_rank):
     launches = grp.sum(launches)
     ms_step = ms_total / args.steps
     value = world * nv * vox_per_view / (ms_step * 1e-3)           # COLD: every view rebuilds its PSF spectrum like the reference (:257)
+    if args.dump_outputs and rank == 0:        # before the arms below overwrite d_out; out_pin is free until the e2e arm
+        dump = {}
+        for v in range(nv):
+            dump[f"acquired_view{v}"] = d_out[v].download(out_pin[v].array)
+            dump[f"psf_view{v}"] = d_psf[v].download()
+        dump_outputs(args.dump_outputs, dump)
 
     # the same step with the PSF-spectrum cache on (SURVEY C6): the six PSFs repeat from step to step, so every view hits
     ctx.psf_cache(8 << 30)
@@ -366,10 +398,10 @@ def run_ours(args, rank, world, local_rank):
     # ---- end-to-end arm: host buffers through the C ABI ------------------------------------------------
     # Serial: one caller thread, one context: every step = ground truth H2D, 6 views, results D2H (downloads overlap the
     # next view inside the call).  Pipelined: THREE caller threads with one context each (the calling pattern of the
-    # reference's own S/SimulateTileStitching.java:85-117), steps dealt round-robin; the library's per-device upload / compute gates line the
+    # reference's own S/SimulateTileStitching.java:85-117), each running --steps steps; the library's per-device upload / compute gates line the
     # callers up so that the H2D of one step runs under the kernels of another and the D2H tail of a third (PCIe is full duplex).  Every step still moves all of its bytes inside the timed region.
     S = mv.SimulateMultiViewDataset
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.steps
     kvox, ovox = int(np.prod(kshape)), int(np.prod(oshape))
 
     def step_e2e(c=ctx, psfs=psf_pin, outs=out_pin):
@@ -394,7 +426,7 @@ def run_ours(args, rank, world, local_rank):
             break                           # pinned host memory exhausted: fewer callers
     n_callers = int(grp.min(len(callers)))      # the same number on every rank
     callers = callers[:n_callers]
-    pipe_steps = 4 * n_callers
+    pipe_steps = n_callers * args.steps         # every caller thread runs --steps steps
     gt_tensor = torch.empty(shape, dtype=torch.float32, device=torch.device("cuda", local_rank)) if world > 1 else None
     gt_tensor_b = torch.empty_like(gt_tensor) if world > 1 else None
 
@@ -490,7 +522,7 @@ def run_ours(args, rank, world, local_rank):
         return res, chk
 
     MODE_TEXT = {"serial": "1 caller thread per rank, ground truth uploaded by every rank",
-                 "pipelined": f"{n_callers} caller threads x 1 context each per rank, steps dealt round-robin (H2D of one step runs under the kernels and D2H of the others)",
+                 "pipelined": f"{n_callers} caller threads x 1 context each per rank, --steps steps each (H2D of one step runs under the kernels and D2H of the others)",
                  "broadcast": "views of one dataset sharded over the ranks: ground truth uploaded once by rank 0 and NCCL-broadcast over NVLink, 1 caller per rank",
                  "broadcast_prefetch": ("views of one dataset sharded over the ranks, one dataset per step: the next dataset's ground truth is uploaded by rank 0 and "
                                         "NCCL-broadcast on a side stream while the current one is simulated and its results drain, 1 caller per rank")}
@@ -662,6 +694,11 @@ def run_slab(args, rank, world, local_rank):
                   "peak_GBps_per_direction": 900.0, "source": "NVML NVLINK_THROUGHPUT_DATA_TX/RX of rank 0's GPU, all links, around the timed region"}
     stage = {k: round(v[0] / args.steps, 3) for k, v in ctx.stage_times().items() if v[1]}
     chk = float(out[::max(1, sc.z_local // 4), ::97, ::89].double().mean().item())
+    if args.dump_outputs and rank == 0:        # rank 0's slab, sampled on the device (16 GB at config 5 on one GPU)
+        res, share = out, DUMP_BYTES // 4
+        if out.numel() > share:
+            res = out.reshape(-1)[torch.from_numpy(dump_indices(out.numel(), share)).to(dev)]
+        dump_outputs(args.dump_outputs, {"convolved_slab_rank0": res.cpu().numpy()})
     if rank == 0:
         vox = int(np.prod(shape))
         print(json.dumps({"metric": "convolved voxels/s (slab-decomposed FFT convolution)", "value": vox / (ms * 1e-3), "unit": "voxels/s",
@@ -688,7 +725,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--widen-threads", type=int, default=0, help="host threads per context that widen uint16 counts (0 = library default)")
     ap.add_argument("--widen-sweep", type=int, nargs="*", help="also time the uint16 transport with these widening thread counts")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (float32, sampled to "
+                                                          "at most 60 MiB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -6,7 +6,7 @@
     into the C ABI has the header's arity and types -- and links against libmvsim.so with no undefined symbol;
   * every mvsim_* function the stubs call is declared in include/mvsim.h and exported by libmvsim.so;
   * the facades carry the reference's public static signatures (S/SimulateMultiViewDataset.java:80,104,181,195,233,253,318 and
-    S/Tools.java:73,112,143) verbatim -- checked against /root/reference when it is mounted -- and no body is elided.
+    S/Tools.java:73,112,143) verbatim -- REFERENCE_SIGNATURES holds those lines of the reference -- and no body is elided.
 """
 import os
 import re
@@ -19,7 +19,6 @@ JAVA = os.path.join(ROOT, "java", "net", "preibisch", "simulation", "gpu")
 JNI_C = os.path.join(ROOT, "jni", "mvsim_jni.c")
 HEADER = os.path.join(ROOT, "include", "mvsim.h")
 LIB = os.path.join(ROOT, "multiview-simulation_b200", "libmvsim.so")
-REF = "/root/reference/src/main/java/net/preibisch/simulation"
 
 
 def _strip_comments(src):
@@ -143,11 +142,8 @@ def test_facades_carry_the_references_signatures_and_complete_bodies():
     for fname, sigs in REFERENCE_SIGNATURES.items():
         src = open(os.path.join(JAVA, fname)).read()
         flat = _norm(src)
-        for ref_file, line, sig in sigs:
+        for _, _, sig in sigs:
             assert _norm(sig) in flat, f"{fname}: missing {sig}"
-            if os.path.isdir(REF):
-                ref_line = open(os.path.join(REF, ref_file)).read().splitlines()[line - 1]
-                assert _norm(ref_line) == _norm(sig), (ref_file, line, ref_line)
         # no elided bodies: no comment-only or empty method bodies, no "..." placeholders
         code = _strip_comments(src)
         assert "..." not in code

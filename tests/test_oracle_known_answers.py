@@ -1,14 +1,11 @@
 """Known-answer pins for the CPU oracle (SURVEY.md section 4): every expectation here follows from
 the cited reference source semantics alone; the reference ships no tests of its own."""
 import math
-import os
 
 import numpy as np
 import pytest
 
 from helpers import gaussian_psf, rel_err, sphere_phantom
-
-REF_RES = "/root/reference/src/main/resources"
 
 
 # ---- java.util.Random (JDK spec) -------------------------------------------------------------
@@ -233,10 +230,10 @@ def test_poisson_is_deterministic_in_the_seed_and_consumes_the_stream_in_flat_or
 
 
 # ---- fixtures of the reference (inputs only) ------------------------------------------------------------
-@pytest.mark.skipif(not os.path.isdir(REF_RES), reason="reference resources not mounted (GPU box)")
 def test_reference_psf_fixture_statistics():
-    from mvsim_b200 import tiff
-    psf = tiff.read_float_stack(os.path.join(REF_RES, "Angle0.tif"))
+    """Angle0.tif of the reference, through its lossless copy in tests/golden/psf_angle0.npz."""
+    from test_golden import load_psf
+    psf = load_psf()
     assert psf.shape == (51, 51, 51) and psf.dtype == np.float32
     assert psf.max() == pytest.approx(0.99, abs=1e-6) and psf.min() == 0
     assert np.unravel_index(psf.argmax(), psf.shape) == (25, 25, 25)
