@@ -162,6 +162,24 @@ int mvsim_weight_image(mvsim_ctx* ctx, const int64_t dims[3], float* out);
  * sum_out (nullable) receives the sum of the normalised weights (sum_weights.tif, :648-663) */
 int mvsim_normalize_weights(mvsim_ctx* ctx, float* const* weights, int n_views, const int64_t dims[3], float osem, float* sum_out);
 
+/* main()'s aligned outputs without the intermediate volumes (:588-663).  The dataset calls rotate about x only (main() does); other
+ * axes stay with the stage entry points.  mvsim_dev_align_view and mvsim_dev_aligned_weights are declared with the device volumes. */
+typedef struct mvsim_dataset_outputs {
+    float* acq;             /* X*Y*((Z-1)/inc+1): the acquired view, float32 (MVSIM_OPT_COUNT_TRANSPORT does not apply) */
+    float* aligned;         /* X*Y*(((Z-1)/inc)*inc+1): rotateAroundAxis(makeIsotropic(acq, inc), 0, align_degrees) (:588, :591) */
+    float* aligned_psf;     /* KX*KY*KZ: the normalised PSF rotated back (:593) */
+    float* weights;         /* X*Y*Z: the view's normalised, rotated-back weight image (:576, :592, :615-646) */
+} mvsim_dataset_outputs;
+/* main()'s view loop with its post-acquisition chain (:567-663) for views[0..n_views) of a dataset of n_all (1..MVSIM_MAX_WEIGHT_VIEWS)
+ * views.  params and align_degrees (the rotate-back angles, -angle in main()) describe ALL views: the weight normalisation needs every
+ * angle, so any subset of the views -- one rank's share -- gives exactly the volumes of the full set.  psfs[i] and outs[i] belong to
+ * views[i]; psfs are normalised in place like :255; any pointer in outs[i] may be NULL (not produced).  sum_weights (nullable):
+ * sum_weights.tif (:648-663).  Every params[k].axis must be 0 and all views share the ground truth dims.  The ground truth is
+ * uploaded once; at most two views' outputs are held on the device, and the downloads of one view overlap the next view's kernels. */
+int mvsim_simulate_dataset(mvsim_ctx* ctx, int n_all, const mvsim_view_params* params, const int32_t* align_degrees, float osem,
+                           int n_views, const int32_t* views, const float* gt, float* const* psfs, const mvsim_dataset_outputs* outs,
+                           float* sum_weights);
+
 /* ---- input generators either side of the path (SURVEY section 8f rows 2-4) ----------------------------------------
  * java.util.Random is replayed bit-exactly (JDK specification), so the caller's seeds keep their meaning. */
 /* SimulateBeads.randomPoints (S/SimulateBeads.java:150-166), reference seed 535 (:69); host arithmetic; points = n x 3 (x, y, z) */
@@ -207,6 +225,18 @@ int mvsim_dev_simulate_view(mvsim_ctx* ctx, const mvsim_view_params* p, const mv
  * another GPU over NVLink when views are sharded across ranks); PSFs and results are host buffers as in mvsim_simulate_views */
 int mvsim_dev_simulate_views(mvsim_ctx* ctx, int n_views, const mvsim_view_params* params, const mvsim_volume* gt,
                              float* const* psfs, float* const* outs);
+/* mvsim_simulate_dataset on a ground truth that is already resident */
+int mvsim_dev_simulate_dataset(mvsim_ctx* ctx, int n_all, const mvsim_view_params* params, const int32_t* align_degrees, float osem,
+                               int n_views, const int32_t* views, const mvsim_volume* gt, float* const* psfs,
+                               const mvsim_dataset_outputs* outs, float* sum_weights);
+/* rotateAroundAxis(makeIsotropic(acq, inc), 0, degrees) (:588, :591) gathered straight from the acquired planes, bit-identical to
+ * the two stages; acq: X*Y*Za, out: X*Y*((Za-1)*inc+1) */
+int mvsim_dev_align_view(mvsim_ctx* ctx, const mvsim_volume* acq, int inc, int degrees, mvsim_volume* out);
+/* the normalised rotate-back weight images of a dataset of n_all views (:576, :592, :615-646) from the dims and angles alone (the
+ * weight image depends on y only, so no volume is read): writes view views[j] into out[j]; sum_weights (nullable) = :648-663.
+ * Bit-identical to mvsim_normalize_weights over mvsim_rotate_axis(mvsim_weight_image(dims), 0, align_degrees[k]) for all k. */
+int mvsim_dev_aligned_weights(mvsim_ctx* ctx, const int64_t dims[3], int n_all, const int32_t* align_degrees, float osem,
+                              int n_out, const int32_t* views, mvsim_volume* const* out, mvsim_volume* sum_weights);
 /* the generators writing straight into a device-resident volume (the ground truth never visits the host) */
 int mvsim_dev_render_beads(mvsim_ctx* ctx, const double* points, int n, const double sigma[3], const int64_t interval_min[3],
                            const int64_t interval_max[3], mvsim_volume* out);

@@ -75,6 +75,17 @@ final class Mvsim
 			float targetAverage, int inc, float poissonSNR, long seed, long firstStream, boolean strictReference,
 			FloatBuffer gt, FloatBuffer[] psfs, FloatBuffer[] outs );
 
+	/**
+	 * main()'s view loop with its post-acquisition chain (:567-663) for the views `views` of a dataset of degrees.length views:
+	 * degrees (acquisition, angle + angleOffset), alignDegrees (rotate-back, -angle) and seeds (noise of view v, stream v) cover ALL
+	 * views, since the weight normalisation needs every angle.  psfs[i], acq[i], aligned[i], alignedPsf[i] and weights[i] belong to
+	 * views[i]; psfs are normalised in place; any output array, any of its elements and sumWeights may be null (not produced).
+	 */
+	static native int simulateDataset( long ctx, long[] dims, long[] kdims, int[] degrees, int[] alignDegrees, double delta, float minValue,
+			float targetAverage, int inc, float poissonSNR, long[] seeds, boolean strictReference, float osem, int[] views,
+			FloatBuffer gt, FloatBuffer[] psfs, FloatBuffer[] acq, FloatBuffer[] aligned, FloatBuffer[] alignedPsf, FloatBuffer[] weights,
+			FloatBuffer sumWeights );
+
 	/* ---- post-acquisition chain of main() ---- */
 	/** makeIsotropic (:144): out holds X*Y*((Z-1)*inc+1) floats */
 	static native int makeIsotropic( long ctx, FloatBuffer in, long[] dims, int inc, FloatBuffer out );

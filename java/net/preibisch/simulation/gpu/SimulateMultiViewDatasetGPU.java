@@ -356,6 +356,75 @@ public class SimulateMultiViewDatasetGPU
 		return result;
 	}
 
+	/**
+	 * main()'s view loop with its post-acquisition chain (:567-663) in one call: for the views `views` of a dataset with the angles
+	 * `angles` (all of them; the weight normalisation needs every angle), the acquired view at angle + angleOffset, the view rotated
+	 * back by -angle (makeIsotropic + rotateAroundAxis, :588-591), its PSF rotated back (:593) and its normalised weights
+	 * (:576, :592, :615-646).  Returns { aligned views, aligned PSFs, aligned weights } in the order of `views`.  Seeds are drawn
+	 * like main(): one rnd.nextLong() per view of the whole dataset, in view order.  psfs (one per entry of `views`, same dims)
+	 * are normalised in place like :255.
+	 */
+	public static List< List< Img< FloatType > > > simulateDataset( final RandomAccessibleInterval< FloatType > gt, final List< Img< FloatType > > psfs,
+			final int[] angles, final int angleOffset, final int[] views, final double delta, final int inc, final float poissonSNR, final float osem,
+			final Random rnd )
+	{
+		final int nAll = angles.length, n = views.length;
+		if ( psfs.size() != n )
+			throw new IllegalArgumentException( "one PSF per simulated view" );
+		if ( inc < 1 )
+			throw new IllegalArgumentException( "inc must be >= 1" );
+		final long[] d = dims( gt ), kd = dims( psfs.get( 0 ) );
+		final long[] iso = new long[] { d[ 0 ], d[ 1 ], ( ( d[ 2 ] - 1 ) / inc ) * inc + 1 };
+		final int[] degrees = new int[ nAll ], align = new int[ nAll ];
+		final long[] seeds = new long[ nAll ];
+		for ( int v = 0; v < nAll; ++v )
+		{
+			degrees[ v ] = angles[ v ] + angleOffset;
+			align[ v ] = -angles[ v ];
+			seeds[ v ] = rnd.nextLong();
+		}
+		final FloatBuffer src = toPinned( gt );
+		final FloatBuffer[] k = new FloatBuffer[ n ], view = new FloatBuffer[ n ], kview = new FloatBuffer[ n ], w = new FloatBuffer[ n ];
+		final List< Img< FloatType > > views_ = new ArrayList< Img< FloatType > >(), psfs_ = new ArrayList< Img< FloatType > >(),
+				weights_ = new ArrayList< Img< FloatType > >();
+		try
+		{
+			for ( int i = 0; i < n; ++i )
+			{
+				final long[] kv = dims( psfs.get( i ) );
+				if ( kv[ 0 ] != kd[ 0 ] || kv[ 1 ] != kd[ 1 ] || kv[ 2 ] != kd[ 2 ] )
+					throw new IllegalArgumentException( "all PSFs of one call must have the same dimensions" );
+				k[ i ] = toPinned( psfs.get( i ) );
+				view[ i ] = Mvsim.pinnedFloats( numElements( iso ) );
+				kview[ i ] = Mvsim.pinnedFloats( numElements( kd ) );
+				w[ i ] = Mvsim.pinnedFloats( numElements( d ) );
+			}
+			check( Mvsim.simulateDataset( ctx(), d, kd, degrees, align, delta, minValue, avgIntensity, inc, poissonSNR, seeds, strictReference,
+					osem, views, src, k, null, view, kview, w, null ) );
+			for ( int i = 0; i < n; ++i )
+			{
+				copyBack( k[ i ], psfs.get( i ) );
+				views_.add( toArrayImg( view[ i ], iso ) );
+				psfs_.add( toArrayImg( kview[ i ], kd ) );
+				weights_.add( toArrayImg( w[ i ], d ) );
+				view[ i ] = kview[ i ] = w[ i ] = null;
+			}
+		}
+		finally
+		{
+			Mvsim.freePinned( src );
+			for ( int i = 0; i < n; ++i )
+				for ( final FloatBuffer b : new FloatBuffer[] { k[ i ], view[ i ], kview[ i ], w[ i ] } )
+					if ( b != null )
+						Mvsim.freePinned( b );
+		}
+		final List< List< Img< FloatType > > > result = new ArrayList< List< Img< FloatType > > >();
+		result.add( views_ );
+		result.add( psfs_ );
+		result.add( weights_ );
+		return result;
+	}
+
 	/* ------------------------------------------------------------------ post-acquisition chain of main() */
 
 	/** drop-in for makeIsotropic (:144-171): linear z up-sampling by inc over the mirror-single extension */

@@ -289,6 +289,62 @@ MVSIM_JNI(jint, simulateViews)(JNIEnv* env, jclass c, jlong ctx, jlongArray dims
     return mvsim_simulate_views(ctx_of(ctx), (int)n, params, src, kern, dst);
 }
 
+/* element i of an optional array of output buffers: NULL when the array or the element is null; *bad when it is too small */
+static float* opt_floats_of(JNIEnv* env, jobjectArray arr, jsize i, int64_t need, int* bad)
+{
+    if (!arr) return NULL;
+    if ((*env)->GetArrayLength(env, arr) <= i) { *bad = 1; return NULL; }
+    jobject b = (*env)->GetObjectArrayElement(env, arr, i);
+    if (!b) return NULL;
+    float* p = floats_of(env, b, need);
+    if (!p) *bad = 1;
+    return p;
+}
+
+MVSIM_JNI(jint, simulateDataset)(JNIEnv* env, jclass c, jlong ctx, jlongArray dims, jlongArray kdims, jintArray degrees, jintArray align_degrees,
+                                 jdouble delta, jfloat min_value, jfloat target_avg, jint inc, jfloat snr, jlongArray seeds, jboolean strict,
+                                 jfloat osem, jintArray views, jobject gt, jobjectArray psfs, jobjectArray acq, jobjectArray aligned,
+                                 jobjectArray aligned_psf, jobjectArray weights, jobject sum_weights)
+{
+    (void)c;
+    int64_t d[3], k[3];
+    if (dims_of(env, dims, d) || dims_of(env, kdims, k) || inc < 1 || !degrees || !align_degrees || !seeds || !views || !psfs) return MVSIM_EINVAL;
+    const jsize n_all = (*env)->GetArrayLength(env, degrees), n = (*env)->GetArrayLength(env, views);
+    if (n_all < 1 || n_all > MVSIM_MAX_WEIGHT_VIEWS || (*env)->GetArrayLength(env, align_degrees) < n_all ||
+        (*env)->GetArrayLength(env, seeds) < n_all || n > n_all || (*env)->GetArrayLength(env, psfs) < n)
+        return MVSIM_EINVAL;
+    const float* src = floats_of(env, gt, prod3(d));
+    if (!src) return MVSIM_EINVAL;
+    jint deg[MVSIM_MAX_WEIGHT_VIEWS], adeg[MVSIM_MAX_WEIGHT_VIEWS], vw[MVSIM_MAX_WEIGHT_VIEWS];
+    jlong sd[MVSIM_MAX_WEIGHT_VIEWS];
+    (*env)->GetIntArrayRegion(env, degrees, 0, n_all, deg);
+    (*env)->GetIntArrayRegion(env, align_degrees, 0, n_all, adeg);
+    (*env)->GetLongArrayRegion(env, seeds, 0, n_all, sd);
+    (*env)->GetIntArrayRegion(env, views, 0, n, vw);
+    mvsim_view_params params[MVSIM_MAX_WEIGHT_VIEWS];
+    int32_t align[MVSIM_MAX_WEIGHT_VIEWS], sel[MVSIM_MAX_WEIGHT_VIEWS];
+    for (jsize v = 0; v < n_all; ++v) {
+        fill_params(&params[v], d, k, 0, deg[v], delta, min_value, target_avg, inc, snr, sd[v], v, strict);
+        align[v] = adeg[v];
+    }
+    const int64_t aligned_elems = d[0] * d[1] * (((d[2] - 1) / inc) * inc + 1);
+    float* kern[MVSIM_MAX_WEIGHT_VIEWS];
+    mvsim_dataset_outputs outs[MVSIM_MAX_WEIGHT_VIEWS];
+    int bad = 0;
+    for (jsize i = 0; i < n; ++i) {
+        sel[i] = vw[i];
+        kern[i] = floats_of(env, (*env)->GetObjectArrayElement(env, psfs, i), prod3(k));
+        if (!kern[i]) return MVSIM_EINVAL;
+        outs[i].acq = opt_floats_of(env, acq, i, slices_of(d, inc), &bad);
+        outs[i].aligned = opt_floats_of(env, aligned, i, aligned_elems, &bad);
+        outs[i].aligned_psf = opt_floats_of(env, aligned_psf, i, prod3(k), &bad);
+        outs[i].weights = opt_floats_of(env, weights, i, prod3(d), &bad);
+    }
+    float* sum = sum_weights ? floats_of(env, sum_weights, prod3(d)) : NULL;
+    if (bad || (sum_weights && !sum)) return MVSIM_EINVAL;
+    return mvsim_simulate_dataset(ctx_of(ctx), (int)n_all, params, align, osem, (int)n, sel, src, kern, outs, sum);
+}
+
 /* ---- post-acquisition chain ------------------------------------------------------------------------------------------ */
 MVSIM_JNI(jint, makeIsotropic)(JNIEnv* env, jclass c, jlong ctx, jobject in, jlongArray dims, jint inc, jobject out)
 {

@@ -7,7 +7,7 @@ from . import tiff                                     # noqa: F401
 from ._lib import LIB_PATH, MvsimError, ViewParams     # noqa: F401
 from .api import (Context, DeviceVolume, JavaRandom, PinnedBuffer, SimulateBeads, SimulateMultiViewDataset, Tools,   # noqa: F401
                   default_context, make_view_params)
-from .drivers import SimulateTileStitching, default_psf, open_psf, run_main   # noqa: F401
+from .drivers import SimulateTileStitching, default_psf, open_psf, run_main, simulate_dataset   # noqa: F401
 from .distributed import Group                         # noqa: F401
 from .sharding import views_for_rank                   # noqa: F401
 from .slab import SlabConvolution, SlabView            # noqa: F401

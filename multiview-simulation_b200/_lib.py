@@ -29,11 +29,17 @@ class ViewParams(C.Structure):
                 ("reserved", C.c_int32)]
 
 
+class DatasetOutputs(C.Structure):
+    _fields_ = [("acq", C.POINTER(C.c_float)), ("aligned", C.POINTER(C.c_float)), ("aligned_psf", C.POINTER(C.c_float)),
+                ("weights", C.POINTER(C.c_float))]
+
+
 # every symbol include/mvsim.h declares: (name, restype, argtypes)
 _vp = C.c_void_p
 _i64p = C.POINTER(C.c_int64)
 _fp = C.POINTER(C.c_float)
 _dp = C.POINTER(C.c_double)
+_i32p = C.POINTER(C.c_int32)
 SYMBOLS = [
     ("mvsim_version", C.c_int, []),
     ("mvsim_device_count", C.c_int, [C.POINTER(C.c_int)]),
@@ -65,6 +71,12 @@ SYMBOLS = [
     ("mvsim_make_isotropic", C.c_int, [_vp, _fp, _i64p, C.c_int, _fp]),
     ("mvsim_weight_image", C.c_int, [_vp, _i64p, _fp]),
     ("mvsim_normalize_weights", C.c_int, [_vp, C.POINTER(_fp), C.c_int, _i64p, C.c_float, _fp]),
+    ("mvsim_simulate_dataset", C.c_int, [_vp, C.c_int, C.POINTER(ViewParams), _i32p, C.c_float, C.c_int, _i32p, _fp, C.POINTER(_fp),
+                                         C.POINTER(DatasetOutputs), _fp]),
+    ("mvsim_dev_simulate_dataset", C.c_int, [_vp, C.c_int, C.POINTER(ViewParams), _i32p, C.c_float, C.c_int, _i32p, _vp,
+                                             C.POINTER(_fp), C.POINTER(DatasetOutputs), _fp]),
+    ("mvsim_dev_align_view", C.c_int, [_vp, _vp, C.c_int, C.c_int, _vp]),
+    ("mvsim_dev_aligned_weights", C.c_int, [_vp, _i64p, C.c_int, _i32p, C.c_float, C.c_int, _i32p, C.POINTER(_vp), _vp]),
     ("mvsim_random_points", C.c_int, [C.c_int, _i64p, _i64p, C.c_int64, _dp]),
     ("mvsim_transform_points", C.c_int, [_dp, C.c_int, _i64p, _i64p, C.c_int, C.c_int, _dp]),
     ("mvsim_render_beads", C.c_int, [_vp, _dp, C.c_int, _dp, _i64p, _i64p, _fp]),

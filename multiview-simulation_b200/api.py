@@ -23,7 +23,7 @@ import threading
 import numpy as np
 
 from . import _lib
-from ._lib import MvsimError, ViewParams, check, dims3, fptr
+from ._lib import DatasetOutputs, MvsimError, ViewParams, check, dims3, fptr
 
 
 class JavaRandom:
@@ -214,6 +214,29 @@ class DeviceVolume:
         if self.h:
             self.ctx._lib.mvsim_volume_free(self.ctx.h, self.h)
             self.h = None
+
+    def alignView(self, inc, degrees, out=None):
+        """rotateAroundAxis(makeIsotropic(self, inc), 0, degrees) (:588, :591) of this acquired view, gathered on the device
+        without the isotropic volume (mvsim_dev_align_view); returns `out` or a new DeviceVolume of ((Za-1)*inc+1, Y, X)."""
+        za, y, x = self.shape
+        out = DeviceVolume(self.ctx, ((za - 1) * inc + 1, y, x)) if out is None else out
+        check(self.ctx._lib.mvsim_dev_align_view(self.ctx.h, self.h, int(inc), int(degrees), out.h), self.ctx.h)
+        return out
+
+    @staticmethod
+    def alignedWeights(ctx, shape_zyx, align_degrees, osem, views=None, sum_weights=False):
+        """The normalised rotate-back weight images of a dataset whose views are rotated back by `align_degrees` (all of them:
+        the normalisation needs every angle), computed from the dims alone (mvsim_dev_aligned_weights).  Returns the DeviceVolumes
+        of `views` (default: all) and, with sum_weights=True, the sum image as a last element."""
+        n_all = len(align_degrees)
+        views = list(range(n_all)) if views is None else [int(v) for v in views]
+        outs = [DeviceVolume(ctx, shape_zyx) for _ in views]
+        s = DeviceVolume(ctx, shape_zyx) if sum_weights else None
+        i32 = C.c_int32
+        oarr = (C.c_void_p * max(len(outs), 1))(*[o.h.value for o in outs])
+        check(ctx._lib.mvsim_dev_aligned_weights(ctx.h, dims3(shape_zyx), n_all, (i32 * n_all)(*[int(d) for d in align_degrees]), float(osem),
+                                                 len(views), (i32 * max(len(views), 1))(*views), oarr, s.h if s else None), ctx.h)
+        return outs + ([s] if s else [])
 
 
 def make_view_params(shape_zyx, kshape_zyx, axis=0, degrees=15, delta=0.01, min_value=0.0001, target_avg=1.0, inc=3,
@@ -456,6 +479,53 @@ class SimulateMultiViewDataset:
             check(ctx._lib.mvsim_simulate_views(ctx.h, n, params, fptr(gt), parr, oarr), ctx.h)
         return outs
 
+    @staticmethod
+    def simulateDataset(gt, psfs, angles, angleOffset=15, delta=0.01, inc=3, poissonSNR=25.0, osem=3.0, rnd=None, views=None, ctx=None,
+                        outputs=("acq", "aligned", "aligned_psf", "weights"), sum_weights=True, strict_reference=True):
+        """main()'s view loop with its post-acquisition chain (:567-663) in one device call (mvsim_simulate_dataset).
+
+        `angles` are ALL the dataset's angles (main(): 0, angleIncrement, ... < 360); view v is acquired at angles[v] + angleOffset
+        and rotated back by -angles[v].  `views` (default: all) selects the views simulated here, `psfs` holds one PSF per selected
+        view (normalised in place, :255).  `gt` is a (Z, Y, X) array or a DeviceVolume.  Noise seeds are drawn like run_main: one
+        nextLong() per view of `rnd` (default JavaRandom(464232194)) in view order for ALL views, stream = view index, so a view's
+        counts do not depend on which subset is simulated.  Returns {"views", "acq", "aligned", "aligned_psf", "weights",
+        "sum_weights"}: lists in the order of `views` (None for outputs not in `outputs`) and the sum image (or None)."""
+        ctx = ctx or default_context()
+        resident = isinstance(gt, DeviceVolume)
+        if not resident:
+            gt = _vol(gt, "gt")
+        n_all = len(angles)
+        views = list(range(n_all)) if views is None else [int(v) for v in views]
+        n = len(views)
+        if len(psfs) != n:
+            raise ValueError("one PSF per simulated view")
+        rnd = JavaRandom(SimulateMultiViewDataset.seed) if rnd is None else (JavaRandom(rnd) if isinstance(rnd, (int, np.integer)) else rnd)
+        seeds = [_seed_from(rnd) for _ in range(n_all)]
+        z, y, x = gt.shape
+        za = (z - 1) // inc + 1
+        params = (ViewParams * n_all)()
+        for v in range(n_all):
+            params[v] = make_view_params(gt.shape, psfs[views.index(v)].shape if v in views else (1, 1, 1), 0, int(angles[v]) + int(angleOffset),
+                                         delta, SimulateMultiViewDataset.minValue, SimulateMultiViewDataset.avgIntensity, inc,
+                                         poissonSNR, seeds[v] if poissonSNR >= 0 else 0, v, strict_reference)
+        res = {"views": views, "acq": [None] * n, "aligned": [None] * n, "aligned_psf": [None] * n, "weights": [None] * n,
+               "sum_weights": np.empty(gt.shape, dtype=np.float32) if sum_weights else None}
+        outs = (DatasetOutputs * max(n, 1))()
+        for i in range(n):
+            _inplace(psfs[i], "psf")
+            shapes = {"acq": (za, y, x), "aligned": ((za - 1) * inc + 1, y, x), "aligned_psf": psfs[i].shape, "weights": (z, y, x)}
+            for key in outputs:
+                res[key][i] = np.empty(shapes[key], dtype=np.float32)
+                setattr(outs[i], key, fptr(res[key][i]))
+        i32 = C.c_int32
+        fpp = C.POINTER(C.c_float)
+        args = (ctx.h, n_all, params, (i32 * n_all)(*[-int(a) for a in angles]), float(osem), n, (i32 * max(n, 1))(*views))
+        tail = ((fpp * max(n, 1))(*[fptr(p) for p in psfs]), outs, fptr(res["sum_weights"]) if sum_weights else None)
+        if resident:
+            check(ctx._lib.mvsim_dev_simulate_dataset(*args, gt.h, *tail), ctx.h)
+        else:
+            check(ctx._lib.mvsim_simulate_dataset(*args, fptr(gt), *tail), ctx.h)
+        return res
 
 
 class SimulateBeads:

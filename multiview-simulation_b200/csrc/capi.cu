@@ -5,6 +5,7 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <algorithm>
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
@@ -1345,6 +1346,208 @@ int mvsim_dev_simulate_view(mvsim_ctx* ctx, const mvsim_view_params* p, const mv
     if (out->dims[0] != p->dims[0] || out->dims[1] != p->dims[1] || out->dims[2] != (p->dims[2] - 1) / p->inc + 1)
         return set_error(ctx, MVSIM_EINVAL, "dev_simulate_view: out dims must be (X, Y, (Z-1)/inc+1)");
     return dev_simulate_view(ctx, p, gt->d, psf->d, out->d);
+}
+
+// ---- main()'s aligned outputs (:588-663) -------------------------------------------------------------------------------
+static int check_view_list(mvsim_ctx* ctx, int n_all, int n, const int32_t* views, const char* what)
+{
+    if (n_all < 1 || n_all > MVSIM_MAX_WEIGHT_VIEWS) return set_error(ctx, MVSIM_EINVAL, "%s: n_all must be 1..%d", what, MVSIM_MAX_WEIGHT_VIEWS);
+    if (n < 0 || n > n_all || (n > 0 && !views)) return set_error(ctx, MVSIM_EINVAL, "%s: 0..n_all view indices", what);
+    bool seen[MVSIM_MAX_WEIGHT_VIEWS] = {};
+    for (int i = 0; i < n; ++i) {
+        if (views[i] < 0 || views[i] >= n_all) return set_error(ctx, MVSIM_EINVAL, "%s: view index %d out of range", what, (int)views[i]);
+        if (seen[views[i]]) return set_error(ctx, MVSIM_EINVAL, "%s: view index %d repeated", what, (int)views[i]);
+        seen[views[i]] = true;
+    }
+    return MVSIM_OK;
+}
+
+// axis-0 inverses of all views for the weight dims (n_all x 12)
+static void weight_inverses(const int64_t dims[3], int n_all, const int32_t* align_degrees, double* inv)
+{
+    for (int k = 0; k < n_all; ++k) axis_rotation(dims, 0, align_degrees[k], nullptr, inv + 12 * k);
+}
+
+static int dev_align_view(mvsim_ctx* ctx, const float* acq, const int64_t acq_dims[3], int inc, int degrees, float* out)
+{
+    // the inverse affine of the isotropic dims, as rotateAroundAxis(iso, 0, degrees) computes it (:591); about x its row 0 is the
+    // identity, which is what lets the gather follow rotate_axis0_kernel
+    const int64_t iso[3] = { acq_dims[0], acq_dims[1], (acq_dims[2] - 1) * inc + 1 };
+    double inv[12];
+    axis_rotation(iso, 0, degrees, nullptr, inv);
+    return k_align_view(ctx, acq, acq_dims, inc, inv, out);
+}
+
+int mvsim_dev_align_view(mvsim_ctx* ctx, const mvsim_volume* acq, int inc, int degrees, mvsim_volume* out)
+{
+    MVSIM_ENTER(ctx);
+    if (!acq || !out || acq == out || inc < 1) return set_error(ctx, MVSIM_EINVAL, "dev_align_view: bad argument");
+    const int64_t iso[3] = { acq->dims[0], acq->dims[1], (acq->dims[2] - 1) * inc + 1 };
+    MVSIM_TRY(check_dims(ctx, iso, "dev_align_view"));
+    if (out->dims[0] != iso[0] || out->dims[1] != iso[1] || out->dims[2] != iso[2])
+        return set_error(ctx, MVSIM_EINVAL, "dev_align_view: out dims must be (X, Y, (Za-1)*inc+1)");
+    return dev_align_view(ctx, acq->d, acq->dims, inc, degrees, out->d);
+}
+
+int mvsim_dev_aligned_weights(mvsim_ctx* ctx, const int64_t dims[3], int n_all, const int32_t* align_degrees, float osem,
+                              int n_out, const int32_t* views, mvsim_volume* const* out, mvsim_volume* sum_weights)
+{
+    MVSIM_ENTER(ctx);
+    MVSIM_TRY(check_dims(ctx, dims, "dev_aligned_weights"));
+    MVSIM_TRY(check_view_list(ctx, n_all, n_out, views, "dev_aligned_weights"));
+    if (!align_degrees || (n_out > 0 && !out)) return set_error(ctx, MVSIM_EINVAL, "dev_aligned_weights: null argument");
+    float* d[MVSIM_MAX_WEIGHT_VIEWS] = {};
+    for (int j = 0; j < n_out; ++j) {
+        const mvsim_volume* o = out[j];
+        if (!o || o->dims[0] != dims[0] || o->dims[1] != dims[1] || o->dims[2] != dims[2])
+            return set_error(ctx, MVSIM_EINVAL, "dev_aligned_weights: output %d must be a volume of dims", j);
+        d[j] = o->d;
+    }
+    if (sum_weights && (sum_weights->dims[0] != dims[0] || sum_weights->dims[1] != dims[1] || sum_weights->dims[2] != dims[2]))
+        return set_error(ctx, MVSIM_EINVAL, "dev_aligned_weights: sum_weights must be a volume of dims");
+    double inv[12 * MVSIM_MAX_WEIGHT_VIEWS];
+    weight_inverses(dims, n_all, align_degrees, inv);
+    return k_aligned_weights(ctx, dims, n_all, inv, osem, n_out, views, d, sum_weights ? sum_weights->d : nullptr);
+}
+
+// main()'s view loop with its post-acquisition chain (:567-663).  Per view: the whole-view acquisition (dev_simulate_view), then the
+// aligned view, the view's own normalised weights and the rotated-back PSF, into one of TWO device output sets; the downloads of
+// view i run on the copy stream under the kernels of view i + 1, and view i + 2 waits for them before it reuses the set.
+static int simulate_dataset_impl(mvsim_ctx* ctx, int n_all, const mvsim_view_params* params, const int32_t* align_degrees, float osem,
+                                 int n_views, const int32_t* views, const float* gt, const float* d_gt, float* const* psfs,
+                                 const mvsim_dataset_outputs* outs, float* sum_weights)
+{
+    MVSIM_TRY(check_view_list(ctx, n_all, n_views, views, "simulate_dataset"));
+    if (!params || !align_degrees) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: null params or angles");
+    for (int k = 0; k < n_all; ++k) {
+        MVSIM_TRY(check_view(ctx, &params[k]));
+        if (params[k].axis != 0) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: main() rotates about x only (axis 0)");
+        for (int d = 0; d < 3; ++d)
+            if (params[k].dims[d] != params[0].dims[d]) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: all views share the ground truth dims");
+    }
+    if (n_views > 0 && (!psfs || !outs || (!gt && !d_gt))) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: null argument");
+    for (int i = 0; i < n_views; ++i)
+        if (!psfs[i]) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: null PSF for view %d", (int)views[i]);
+    if (n_views == 0 && !sum_weights) return MVSIM_OK;
+    if (!ctx->copy_stream) MVSIM_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
+    const int64_t* dims = params[0].dims;
+    const size_t n = elems(dims);
+    double inv_w[12 * MVSIM_MAX_WEIGHT_VIEWS];
+    weight_inverses(dims, n_all, align_degrees, inv_w);
+    auto acq_elems = [&](const mvsim_view_params* p) { return (size_t)(p->dims[0] * p->dims[1] * ((p->dims[2] - 1) / p->inc + 1)); };
+    auto iso_elems = [&](const mvsim_view_params* p) { return (size_t)(p->dims[0] * p->dims[1] * (((p->dims[2] - 1) / p->inc) * p->inc + 1)); };
+    // sizes of a device output set: the largest of its views
+    size_t acq_max = 0, iso_max = 0, k_max = 0;
+    bool any_iso = false, any_kpsf = false, any_w = false;
+    for (int i = 0; i < n_views; ++i) {
+        const mvsim_view_params* p = &params[views[i]];
+        acq_max = std::max(acq_max, acq_elems(p));
+        iso_max = std::max(iso_max, iso_elems(p));
+        k_max = std::max(k_max, elems(p->kdims));
+        any_iso |= outs[i].aligned != nullptr;
+        any_kpsf |= outs[i].aligned_psf != nullptr;
+        any_w |= outs[i].weights != nullptr;
+    }
+    DeviceGates& gates = gates_for(ctx->device);
+    cudaEvent_t done[2] = {}, freed[2] = {}, copied = nullptr;
+    int st = MVSIM_OK;
+    for (int s = 0; s < 2 && st == MVSIM_OK; ++s)
+        if (cudaEventCreateWithFlags(&done[s], cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&freed[s], cudaEventDisableTiming) != cudaSuccess)
+            st = set_error(ctx, MVSIM_ECUDA, "simulate_dataset: cannot create events");
+    if (st == MVSIM_OK && cudaEventCreateWithFlags(&copied, cudaEventDisableTiming) != cudaSuccess) st = set_error(ctx, MVSIM_ECUDA, "simulate_dataset: cannot create events");
+    std::vector<void*> held;
+    auto alloc = [&](size_t bytes) -> float* {
+        void* q = nullptr;
+        if (st == MVSIM_OK && (st = dev_alloc(ctx, &q, bytes)) == MVSIM_OK) held.push_back(q);
+        return static_cast<float*>(q);
+    };
+    float* g = d_gt || n_views == 0 ? nullptr : alloc(n * sizeof(float));
+    const float* gt_dev = d_gt ? d_gt : g;
+    std::vector<float*> kpsf((size_t)n_views, nullptr);
+    for (int i = 0; i < n_views; ++i) kpsf[(size_t)i] = alloc(elems(params[views[i]].kdims) * sizeof(float));
+    struct OutSet { float *acq, *iso, *kpsf, *w; } set[2] = {};
+    for (int s = 0; s < 2 && s < n_views; ++s) {
+        set[s].acq = alloc(acq_max * sizeof(float));
+        if (any_iso) set[s].iso = alloc(iso_max * sizeof(float));
+        if (any_kpsf) set[s].kpsf = alloc(k_max * sizeof(float));
+        if (any_w) set[s].w = alloc(n * sizeof(float));
+    }
+    float* dsum = sum_weights ? alloc(n * sizeof(float)) : nullptr;
+    // downloads of view i (psfs are normalised in place, :255)
+    auto download = [&](int i) -> int {
+        const int s = i % 2;
+        const mvsim_view_params* p = &params[views[i]];
+        const mvsim_dataset_outputs& o = outs[i];
+        cudaError_t e = cudaStreamWaitEvent(ctx->copy_stream, done[s], 0);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(psfs[i], kpsf[(size_t)i], elems(p->kdims) * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
+        if (e == cudaSuccess && o.acq) e = cudaMemcpyAsync(o.acq, set[s].acq, acq_elems(p) * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
+        if (e == cudaSuccess && o.aligned) e = cudaMemcpyAsync(o.aligned, set[s].iso, iso_elems(p) * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
+        if (e == cudaSuccess && o.aligned_psf) e = cudaMemcpyAsync(o.aligned_psf, set[s].kpsf, elems(p->kdims) * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
+        if (e == cudaSuccess && o.weights) e = cudaMemcpyAsync(o.weights, set[s].w, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
+        if (e == cudaSuccess) e = cudaEventRecord(freed[s], ctx->copy_stream);
+        return e == cudaSuccess ? MVSIM_OK : cuda_fail(ctx, e, "simulate_dataset: download");
+    };
+    if (st == MVSIM_OK && n_views > 0) {
+        // all uploads under the upload gate, as in simulate_views_impl
+        std::lock_guard<std::mutex> lk(gates.upload);
+        if (!d_gt) st = h2d(ctx, g, gt, n * sizeof(float));
+        for (int i = 0; i < n_views && st == MVSIM_OK; ++i) st = h2d(ctx, kpsf[(size_t)i], psfs[i], elems(params[views[i]].kdims) * sizeof(float));
+        if (st == MVSIM_OK && (cudaEventRecord(done[0], ctx->stream) != cudaSuccess || cudaEventSynchronize(done[0]) != cudaSuccess))
+            st = set_error(ctx, MVSIM_ECUDA, "simulate_dataset: upload failed");
+    }
+    if (st == MVSIM_OK) {
+        std::lock_guard<std::mutex> lk(gates.compute);
+        // the sum image depends on the dims and the angles alone (:648-663)
+        if (dsum) st = k_aligned_weights(ctx, dims, n_all, inv_w, osem, 0, nullptr, nullptr, dsum);
+        for (int i = 0; i < n_views && st == MVSIM_OK; ++i) {
+            const int s = i % 2, v = views[i];
+            const mvsim_view_params* p = &params[v];
+            const mvsim_dataset_outputs& o = outs[i];
+            if (i >= 2 && cudaStreamWaitEvent(ctx->stream, freed[s], 0) != cudaSuccess) { st = set_error(ctx, MVSIM_ECUDA, "simulate_dataset: wait"); break; }
+            if ((st = dev_simulate_view(ctx, p, gt_dev, kpsf[(size_t)i], set[s].acq)) != MVSIM_OK) break;                 // :570-585
+            const int64_t acq_dims[3] = { p->dims[0], p->dims[1], (p->dims[2] - 1) / p->inc + 1 };
+            if (o.aligned && (st = dev_align_view(ctx, set[s].acq, acq_dims, p->inc, align_degrees[v], set[s].iso)) != MVSIM_OK) break;   // :588, :591
+            if (o.weights && (st = k_aligned_weights(ctx, dims, n_all, inv_w, osem, 1, &v, &set[s].w, nullptr)) != MVSIM_OK) break;      // :576, :592, :615-646
+            if (o.aligned_psf && (st = dev_rotate(ctx, kpsf[(size_t)i], set[s].kpsf, p->kdims, 0, align_degrees[v])) != MVSIM_OK) break; // :593
+            if (cudaEventRecord(done[s], ctx->stream) != cudaSuccess) { st = set_error(ctx, MVSIM_ECUDA, "simulate_dataset: event"); break; }
+            if (i >= 1) st = download(i - 1);
+        }
+        if (st == MVSIM_OK && n_views > 0) st = download(n_views - 1);
+        if (st == MVSIM_OK && dsum) st = d2h(ctx, sum_weights, dsum, n * sizeof(float));
+        // the gate opens when this call's last kernel has run; the tail of the downloads overlaps the next caller's kernels
+        if (st == MVSIM_OK && n_views > 0 && cudaEventSynchronize(done[(n_views - 1) % 2]) != cudaSuccess) st = set_error(ctx, MVSIM_ECUDA, "simulate_dataset: kernels failed");
+    }
+    // the main stream waits for the copy stream before the buffers go back to the pool
+    if (copied && cudaEventRecord(copied, ctx->copy_stream) == cudaSuccess) cudaStreamWaitEvent(ctx->stream, copied, 0);
+    for (void* q : held) dev_free(ctx, q);
+    const int st2 = sync(ctx);
+    for (int s = 0; s < 2; ++s) {
+        if (done[s]) cudaEventDestroy(done[s]);
+        if (freed[s]) cudaEventDestroy(freed[s]);
+    }
+    if (copied) cudaEventDestroy(copied);
+    return st != MVSIM_OK ? st : st2;
+}
+
+int mvsim_simulate_dataset(mvsim_ctx* ctx, int n_all, const mvsim_view_params* params, const int32_t* align_degrees, float osem,
+                           int n_views, const int32_t* views, const float* gt, float* const* psfs, const mvsim_dataset_outputs* outs,
+                           float* sum_weights)
+{
+    MVSIM_ENTER(ctx);
+    if (n_views > 0 && !gt) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: null ground truth");
+    return simulate_dataset_impl(ctx, n_all, params, align_degrees, osem, n_views, views, gt, nullptr, psfs, outs, sum_weights);
+}
+
+int mvsim_dev_simulate_dataset(mvsim_ctx* ctx, int n_all, const mvsim_view_params* params, const int32_t* align_degrees, float osem,
+                               int n_views, const int32_t* views, const mvsim_volume* gt, float* const* psfs,
+                               const mvsim_dataset_outputs* outs, float* sum_weights)
+{
+    MVSIM_ENTER(ctx);
+    if (n_views > 0 && !gt) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: null ground truth");
+    if (gt && params && n_all >= 1)
+        for (int d = 0; d < 3; ++d)
+            if (gt->dims[d] != params[0].dims[d]) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: ground truth volume dims differ from the view params");
+    return simulate_dataset_impl(ctx, n_all, params, align_degrees, osem, n_views, views, nullptr, gt ? gt->d : nullptr, psfs, outs, sum_weights);
 }
 
 

@@ -110,6 +110,13 @@ int k_extract(mvsim_ctx* ctx, const float* in, const int64_t dims[3], int inc, c
 int k_make_isotropic(mvsim_ctx* ctx, const float* in, const int64_t dims[3], int inc, float* out);
 int k_weight_image(mvsim_ctx* ctx, const int64_t dims[3], float* out);
 int k_normalize_weights(mvsim_ctx* ctx, float* const* d_weights, int n_views, size_t n, float osem, float* d_sum_out);
+// rotateAroundAxis(makeIsotropic(acq, inc), 0, .) straight from the acquired planes; acq_dims = {X, Y, Za}, out: X*Y*((Za-1)*inc+1);
+// inv = axisRotation(iso dims, 0, degrees) inverse
+int k_align_view(mvsim_ctx* ctx, const float* acq, const int64_t acq_dims[3], int inc, const double inv[12], float* out);
+// normalised rotate-back weights of n_all views (inv: n_all x 12, the axis-0 inverses for dims): view views[j] -> outs[j] (j < n_out),
+// the sum of the normalised weights -> sum_out (nullable); no input volume
+int k_aligned_weights(mvsim_ctx* ctx, const int64_t dims[3], int n_all, const double* inv, float osem, int n_out, const int* views,
+                      float* const* outs, float* sum_out);
 int k_poisson(mvsim_ctx* ctx, float* inout, size_t n, double snr, uint64_t seed, uint64_t stream);
 // 128-bit content hash of n floats (order-independent sum of two 64-bit mixes of (bits, index)): d_out[2], enqueued on the stream
 int k_hash128(mvsim_ctx* ctx, const float* in, size_t n, unsigned long long* d_out);

@@ -12,6 +12,7 @@
 #include <type_traits>
 
 #include "ctx.h"
+#include "post.cuh"
 #include "sampler.cuh"
 
 namespace mvsim {
@@ -29,8 +30,6 @@ static inline unsigned blocks_for(size_t n, unsigned threads) { return (unsigned
 // rotate.  Inverse affine applied in FP64 in mpicbg's evaluation order, floor + fractional weights in
 // FP64, blend in FP32 in imglib2's tap order (000,100,110,010,011,111,101,001), zero outside.
 // ---------------------------------------------------------------------------------------------
-struct Affine { double m[12]; };
-
 // axis 0: x_src == x (row 0 of the inverse is the identity), so the source coordinates are constant
 // along a row and the gather is bilinear in (y,z): VEC contiguous voxels per thread, 4 coalesced loads.
 template <int VEC> __global__ void __launch_bounds__(256) rotate_axis0_kernel(const float* __restrict__ in, float* __restrict__ out,
@@ -120,26 +119,12 @@ __global__ void __launch_bounds__(256) rotate_general_kernel(const float* __rest
 // (exactly the arithmetic of rotate_axis0_kernel); the main kernel marches every (x,z) column from
 // y = Y-1 down, gathers the rotated voxel from the ground truth and applies the recurrence of :343-357.
 // ---------------------------------------------------------------------------------------------
-struct __align__(16) RowTaps { int iy, iz; float w00, w10, w11, w01; int pad0, pad1; };
-
-// rows (y, z) of the output planes [z0, z0 + Zl): entry (z - z0) * Y + y
+// rows (y, z) of the output planes [z0, z0 + Zl): entry (z - z0) * Y + y  (RowTaps, axis0_row_taps: post.cuh)
 __global__ void __launch_bounds__(256) rotate_rowtable_kernel(RowTaps* __restrict__ tab, int Y, int z0, int Zl, Affine a)
 {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (long long)Y * Zl) return;
-    const int y = (int)(i % Y), z = z0 + (int)(i / Y);
-    const double ly = (double)y, lz = (double)z;
-    const double py = __dadd_rn(__dadd_rn(__dmul_rn(ly, a.m[5]), __dmul_rn(lz, a.m[6])), a.m[7]);
-    const double pz = __dadd_rn(__dadd_rn(__dmul_rn(ly, a.m[9]), __dmul_rn(lz, a.m[10])), a.m[11]);
-    const double fy = floor(py), fz = floor(pz);
-    const double wy = py - fy, wz = pz - fz;
-    const double wyi = 1.0 - wy, wzi = 1.0 - wz;
-    RowTaps t;
-    t.iy = (int)fmax(fmin(fy, 2.0e9), -2.0e9);
-    t.iz = (int)fmax(fmin(fz, 2.0e9), -2.0e9);
-    t.w00 = (float)(wyi * wzi); t.w10 = (float)(wy * wzi); t.w11 = (float)(wy * wz); t.w01 = (float)(wyi * wz);
-    t.pad0 = t.pad1 = 0;
-    tab[i] = t;
+    tab[i] = axis0_row_taps((int)(i % Y), z0 + (int)(i / Y), a);
 }
 
 template <int VEC> struct VecT;
@@ -874,18 +859,7 @@ int k_extract_slab(mvsim_ctx* ctx, const float* in, const int64_t dims[3], int64
 //   computeWeightImage S/SimulateMultiViewDataset.java:280-316   cosine taper along y
 //   weight normalisation                                 :615-661 the one cross-view reduction
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ int mirror_idx(int i, int n)
-{
-    if ((unsigned)i < (unsigned)n) return i;
-    if (n == 1) return 0;
-    const int p = 2 * (n - 1);
-    int j = i % p;
-    if (j < 0) j += p;
-    return j >= n ? p - j : j;
-}
-
-// x, y are integer positions, so the n-linear interpolation of :150,167 reduces to two taps along z:
-// out = f32(f32(a * (1 - w)) + f32(b * w)), position (float)z / (float)inc widened to double (:165)
+// x, y are integer positions, so the n-linear interpolation of :150,167 reduces to two taps along z (iso_plane, iso_blend: post.cuh)
 __global__ void __launch_bounds__(256) make_isotropic_kernel(const float* __restrict__ in, float* __restrict__ out, long long plane, int Z,
                                                              long long n_out, int inc)
 {
@@ -893,13 +867,8 @@ __global__ void __launch_bounds__(256) make_isotropic_kernel(const float* __rest
     if (i >= n_out) return;
     const int zo = (int)(i / plane);
     const long long r = i - (long long)zo * plane;
-    const double zf = (double)((float)zo / (float)inc);
-    const double f = floor(zf);
-    const double w = zf - f, wi = 1.0 - w;
-    const int iz = (int)f;
-    const float a = __ldg(in + (long long)mirror_idx(iz, Z) * plane + r);
-    const float b = __ldg(in + (long long)mirror_idx(iz + 1, Z) * plane + r);
-    out[i] = __fadd_rn((float)__dmul_rn((double)a, wi), (float)__dmul_rn((double)b, w));
+    const IsoPlane p = iso_plane(zo, inc, Z);
+    out[i] = iso_blend(__ldg(in + (long long)p.pa * plane + r), __ldg(in + (long long)p.pb * plane + r), p);
 }
 
 int k_make_isotropic(mvsim_ctx* ctx, const float* in, const int64_t dims[3], int inc, float* out)
@@ -915,13 +884,7 @@ __global__ void __launch_bounds__(256) weight_image_kernel(float* __restrict__ o
 {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const int y = (int)((i / X) % Y);
-    const int l = Y - y - 1, half = Y / 2, span = 40;       // cosineSpan (:283)
-    float v;
-    if (l < half) v = 1.0f;
-    else if (l > half + span) v = 0.0f;
-    else v = (float)((cos(((double)(l - half) / (double)span) * 3.14159265358979323846) + 1.0) / 2.0);
-    out[i] = v;
+    out[i] = weight_of_row((int)((i / X) % Y), Y);
 }
 
 int k_weight_image(mvsim_ctx* ctx, const int64_t dims[3], float* out)
@@ -962,6 +925,177 @@ int k_normalize_weights(mvsim_ctx* ctx, float* const* d_weights, int n_views, si
     for (int k = 0; k < MVSIM_MAX_WEIGHT_VIEWS; ++k) p.w[k] = k < n_views ? d_weights[k] : nullptr;
     normalize_weights_kernel<<<blocks_for(n, 256), 256, 0, ctx->stream>>>(p, n_views, n, osem, d_sum_out);
     MVSIM_LAUNCH_CHECK(ctx);
+    return MVSIM_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// main()'s aligned outputs without the intermediate volumes (row / tap arithmetic: post.cuh)
+//   align_view       rotateAroundAxis(makeIsotropic(acq, inc), 0, d)                    :588, :591
+//   aligned_weights  normalised rotateAroundAxis(computeWeightImage(dims), 0, d_v)      :576, :592, :615-661
+// Both launch 64 x 4 blocks: 64 threads along x, one output row (y, z) per warp pair, rows on grid x (no 64-bit division).
+// ---------------------------------------------------------------------------------------------
+template <int VEC> __device__ __forceinline__ bool any_negzero(const float (&a)[VEC])
+{
+    bool r = false;
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) r |= __float_as_uint(a[i]) == 0x80000000u;
+    return r;
+}
+
+template <int VEC> __device__ __forceinline__ void copy_vec(float (&d)[VEC], const float (&s)[VEC])
+{
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) d[i] = s[i];
+}
+
+// Values of the up-sampled volume at iso planes iz (p0, valid if z0) and iz+1 (p1, valid if z1) of one source row; rowp points at
+// that row in acquired plane 0.  Each iso plane blends the acquired planes pa and pb.  The next iso plane lies between the same two
+// planes or starts at pb, so two row loads serve both taps.  With w == 0 the blend f32(a + f32(b * 0)) equals a for finite b unless
+// a is -0 (then the sign of b decides), so b is read only when it can change the result.
+template <int VEC> __device__ __forceinline__ void iso_taps(const float* rowp, long long plane, bool z0, bool z1, const IsoPlane& p0,
+                                                           const IsoPlane& p1, float (&v0)[VEC], float (&v1)[VEC])
+{
+    float a[VEC], b[VEC], a1[VEC], b1[VEC];
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) { v0[i] = 0.f; v1[i] = 0.f; b[i] = 0.f; b1[i] = 0.f; }
+    bool hb = false;
+    if (z0) {
+        vload<VEC>(a, rowp + p0.pa * plane, true);
+        if (p0.w != 0.0 || any_negzero<VEC>(a)) { vload<VEC>(b, rowp + p0.pb * plane, true); hb = true; }
+#pragma unroll
+        for (int i = 0; i < VEC; ++i) v0[i] = iso_blend(a[i], b[i], p0);
+    }
+    if (z1) {
+        if (z0 && p1.pa == p0.pa) copy_vec<VEC>(a1, a);
+        else if (hb && p1.pa == p0.pb) copy_vec<VEC>(a1, b);
+        else vload<VEC>(a1, rowp + p1.pa * plane, true);
+        if (p1.w != 0.0 || any_negzero<VEC>(a1)) {
+            if (hb && p1.pb == p0.pb) copy_vec<VEC>(b1, b);
+            else vload<VEC>(b1, rowp + p1.pb * plane, true);
+        }
+#pragma unroll
+        for (int i = 0; i < VEC; ++i) v1[i] = iso_blend(a1[i], b1[i], p1);
+    }
+}
+
+// out: X x Y x Ziso, acq: X x Y x Za; tab: the rotation rows of the iso dims (rotate_rowtable_kernel)
+template <int VEC> __global__ void __launch_bounds__(256) align_view_kernel(const float* __restrict__ acq, float* __restrict__ out,
+                                                                           const RowTaps* __restrict__ tab, int X, int Y, int Ziso,
+                                                                           int Za, int inc)
+{
+    const long long row = (long long)blockIdx.x * blockDim.y + threadIdx.y;
+    const int xv = blockIdx.y * blockDim.x + threadIdx.x;
+    if (row >= (long long)Y * Ziso || xv * VEC >= X) return;
+    const RowTaps t = tab[row];
+    const long long plane = (long long)X * Y, x0 = (long long)xv * VEC;
+    const bool y0 = (unsigned)t.iy < (unsigned)Y, y1 = (unsigned)(t.iy + 1) < (unsigned)Y;
+    const bool z0 = (unsigned)t.iz < (unsigned)Ziso, z1 = (unsigned)(t.iz + 1) < (unsigned)Ziso;
+    IsoPlane p0{}, p1{};
+    if (z0) p0 = iso_plane(t.iz, inc, Za);
+    if (z1) p1 = iso_plane(t.iz + 1, inc, Za);
+    float a0[VEC], a1[VEC], b0[VEC], b1[VEC];          // a: source row iy (taps 00, 01), b: row iy + 1 (taps 10, 11)
+    iso_taps<VEC>(acq + x0 + (long long)X * t.iy, plane, y0 && z0, y0 && z1, p0, p1, a0, a1);
+    iso_taps<VEC>(acq + x0 + (long long)X * (t.iy + 1), plane, y1 && z0, y1 && z1, p0, p1, b0, b1);
+    float r[VEC];
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) r[i] = axis0_blend(a0[i], b0[i], b1[i], a1[i], t);
+    *reinterpret_cast<typename VecT<VEC>::type*>(out + x0 + X * row) = *reinterpret_cast<typename VecT<VEC>::type*>(r);
+}
+
+int k_align_view(mvsim_ctx* ctx, const float* acq, const int64_t acq_dims[3], int inc, const double inv[12], float* out)
+{
+    const int X = (int)acq_dims[0], Y = (int)acq_dims[1], Za = (int)acq_dims[2];
+    const int Ziso = (Za - 1) * inc + 1;
+    Affine a;
+    for (int i = 0; i < 12; ++i) a.m[i] = inv[i];
+    const long long rows = (long long)Y * Ziso;
+    RowTaps* tab = nullptr;
+    MVSIM_TRY(dev_alloc(ctx, (void**)&tab, sizeof(RowTaps) * (size_t)rows));
+    rotate_rowtable_kernel<<<blocks_for((size_t)rows, 256), 256, 0, ctx->stream>>>(tab, Y, 0, Ziso, a);
+    ctx->launches++;
+    const bool vec4 = X % 4 == 0 && (reinterpret_cast<uintptr_t>(acq) | reinterpret_cast<uintptr_t>(out)) % 16 == 0;
+    const int xv = vec4 ? X / 4 : X;
+    const dim3 block(64, 4), grid((unsigned)((rows + 3) / 4), (unsigned)((xv + 63) / 64));
+    if (vec4) align_view_kernel<4><<<grid, block, 0, ctx->stream>>>(acq, out, tab, X, Y, Ziso, Za, inc);
+    else align_view_kernel<1><<<grid, block, 0, ctx->stream>>>(acq, out, tab, X, Y, Ziso, Za, inc);
+    ctx->launches++;
+    cudaError_t e = cudaGetLastError();
+    dev_free(ctx, tab);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "align_view_kernel");
+    return MVSIM_OK;
+}
+
+struct WeightViews { Affine a[MVSIM_MAX_WEIGHT_VIEWS]; int slot[MVSIM_MAX_WEIGHT_VIEWS]; };
+
+// Row (y, z) of the Y x Z plane: the rotated-back weights of all n_all views, summed in view order and normalised exactly as
+// normalize_weights_kernel does.  rows[slot * Y*Z + row] receives view k's normalised weight when wv.slot[k] >= 0, and
+// rows[sum_slot * Y*Z + row] the sum of the normalised weights when sum_slot >= 0.
+__global__ void __launch_bounds__(128) aligned_weight_rows_kernel(float* __restrict__ rows, int Y, int Z, int n_all, float osem, int sum_slot,
+                                                                  WeightViews wv)
+{
+    const long long R = (long long)Y * Z;
+    const long long row = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (row >= R) return;
+    const int y = (int)(row % Y), z = (int)(row / Y);
+    float v[MVSIM_MAX_WEIGHT_VIEWS];
+    float sum = 0.f;
+#pragma unroll
+    for (int k = 0; k < MVSIM_MAX_WEIGHT_VIEWS; ++k)
+        if (k < n_all) { v[k] = aligned_weight(y, z, Y, Z, wv.a[k]); sum = fadd_rn(sum, v[k]); }
+    float s2 = 0.f;
+#pragma unroll
+    for (int k = 0; k < MVSIM_MAX_WEIGHT_VIEWS; ++k)
+        if (k < n_all) {
+            const float o = normalized_weight(v[k], sum, osem);
+            s2 = fadd_rn(s2, o);
+            if (wv.slot[k] >= 0) rows[wv.slot[k] * R + row] = o;
+        }
+    if (sum_slot >= 0) rows[sum_slot * R + row] = s2;
+}
+
+// out[x + X * row] = col[row]: a store-bound broadcast of one value per row
+template <int VEC> __global__ void __launch_bounds__(256) broadcast_rows_kernel(const float* __restrict__ col, float* __restrict__ out, int X, long long R)
+{
+    const long long row = (long long)blockIdx.x * blockDim.y + threadIdx.y;
+    const int xv = blockIdx.y * blockDim.x + threadIdx.x;
+    if (row >= R || xv * VEC >= X) return;
+    const float v = __ldg(col + row);
+    float r[VEC];
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) r[i] = v;
+    *reinterpret_cast<typename VecT<VEC>::type*>(out + (long long)xv * VEC + X * row) = *reinterpret_cast<typename VecT<VEC>::type*>(r);
+}
+
+int k_aligned_weights(mvsim_ctx* ctx, const int64_t dims[3], int n_all, const double* inv, float osem, int n_out, const int* views,
+                      float* const* outs, float* sum_out)
+{
+    const int X = (int)dims[0], Y = (int)dims[1], Z = (int)dims[2];
+    const long long R = (long long)Y * Z;
+    const int n_rows = n_out + (sum_out ? 1 : 0);
+    if (n_rows == 0) return MVSIM_OK;
+    WeightViews wv;
+    for (int k = 0; k < MVSIM_MAX_WEIGHT_VIEWS; ++k) {
+        wv.slot[k] = -1;
+        for (int i = 0; i < 12; ++i) wv.a[k].m[i] = k < n_all ? inv[12 * k + i] : 0.0;
+    }
+    for (int j = 0; j < n_out; ++j) wv.slot[views[j]] = j;
+    float* rows = nullptr;
+    MVSIM_TRY(dev_alloc(ctx, (void**)&rows, sizeof(float) * (size_t)n_rows * (size_t)R));
+    aligned_weight_rows_kernel<<<blocks_for((size_t)R, 128), 128, 0, ctx->stream>>>(rows, Y, Z, n_all, osem, sum_out ? n_out : -1, wv);
+    ctx->launches++;
+    cudaError_t e = cudaGetLastError();
+    for (int j = 0; j < n_rows && e == cudaSuccess; ++j) {
+        float* dst = j < n_out ? outs[j] : sum_out;
+        const bool vec4 = X % 4 == 0 && reinterpret_cast<uintptr_t>(dst) % 16 == 0;
+        const int xv = vec4 ? X / 4 : X;
+        const dim3 block(64, 4), grid((unsigned)((R + 3) / 4), (unsigned)((xv + 63) / 64));
+        if (vec4) broadcast_rows_kernel<4><<<grid, block, 0, ctx->stream>>>(rows + (size_t)j * R, dst, X, R);
+        else broadcast_rows_kernel<1><<<grid, block, 0, ctx->stream>>>(rows + (size_t)j * R, dst, X, R);
+        ctx->launches++;
+        e = cudaGetLastError();
+    }
+    dev_free(ctx, rows);
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "aligned_weights");
     return MVSIM_OK;
 }
 

@@ -9,9 +9,12 @@ and they double as integration tests of the boundary: the tile-stitching driver 
 with one context each and re-samples one convolved volume at many SNRs, exactly the calling pattern the boundary must
 support (SURVEY section 3.2).
 
-    python -m mvsim_b200.drivers --out /tmp/sim [--size 289] [--angles 7] [--psf-dir DIR]
+    simulate_dataset(...)    main() with the view loop in one device call (acquisition + aligned outputs)
+
+    python -m mvsim_b200.drivers --out /tmp/sim [--size 289] [--angles 7] [--psf-dir DIR] [--fused [--rank R --world W]]
 """
 import argparse
+import ctypes as C
 import os
 import threading
 import time
@@ -19,6 +22,7 @@ import time
 import numpy as np
 
 from . import tiff
+from ._lib import check
 from .api import Context, JavaRandom, SimulateMultiViewDataset as S, Tools
 
 # main(): angleIncrement -> osem factor (:536-546)
@@ -103,6 +107,74 @@ def run_main(out_dir=None, size=289, angle_increment=52, osem=None, poissonSNR=2
     if "weights" in keep:
         res["weights"] = weights
     res["sum_weights"] = sum_weights
+    res["seconds"] = time.perf_counter() - t_start
+    log("done")
+    return res
+
+
+def simulate_dataset(out_dir=None, size=289, angle_increment=52, osem=None, poissonSNR=25.0, lightsheetSpacing=3, attenuation=0.01,
+                     angleOffset=15, psf_dir=None, psf=None, ctx=None, log=print, keep=("acq", "view", "weights"), rank=0, world=1):
+    """main() (:524-665) with its view loop in one device call (SimulateMultiViewDataset.simulateDataset): the phantom is rendered
+    on the device and stays there; per view the library runs the whole-view acquisition, the aligned view, the view's normalised
+    weights and the rotated-back PSF, and only those outputs cross the host link.  Writes run_main's file names for what it
+    produces (acq_view_, aligned_view_, aligned_view_psf_, aligned_view_weights, sum_weights, rendered, groundtruth); the
+    intermediate rot / att / con / iso volumes exist only in run_main.
+
+    rank / world: this process simulates the views v with v % world == rank (sharding.views_for_rank).  The normalised weights
+    depend on the angles alone, so no rank needs another's data: there is no collective.  Rank 0 also writes rendered,
+    groundtruth and sum_weights.  Returns run_main's dict for this rank's views ('angles' lists them)."""
+    from .api import DeviceVolume
+    from .sharding import views_for_rank
+    ctx = ctx or Context(0)
+    osem = OSEM.get(angle_increment, 3.0) if osem is None else osem
+    t_start = time.perf_counter()
+
+    def save(vol, name):
+        if out_dir:
+            tiff.write_float_stack(os.path.join(out_dir, name), vol)
+
+    if out_dir:
+        os.makedirs(out_dir, exist_ok=True)
+    angles = list(range(0, 360, angle_increment))                                       # :567
+    mine = views_for_rank(len(angles), rank, world)
+    log("rendering basis for ground truth")
+    gt = DeviceVolume(ctx, (size, size, size))
+    n_small = C.c_int64(0)
+    check(ctx._lib.mvsim_dev_simulate_phantom(ctx.h, size, 0, S.seed, gt.h, C.byref(n_small)), ctx.h)   # :554
+    res = {"angles": [angles[v] for v in mine], "acq": [], "view": [], "weights": [], "psf": [], "sum_weights": None}
+    if rank == 0:
+        log("computing ground truth")
+        obj = DeviceVolume(ctx, gt.shape)
+        check(ctx._lib.mvsim_dev_rotate_axis(ctx.h, gt.h, obj.h, 0, angleOffset), ctx.h)   # :557
+        res["rendered"], res["groundtruth"] = gt.download(), obj.download()
+        obj.free()
+        save(res["rendered"], "rendered.tif")
+        save(res["groundtruth"], "groundtruth.tif")
+    psfs = []
+    for v in mine:
+        angle = angles[v]
+        if psf is not None:
+            psfs.append(np.array(psf, dtype=np.float32, order="C", copy=True))
+        elif psf_dir and os.path.exists(os.path.join(psf_dir, f"Angle{angle}.tif")):
+            psfs.append(open_psf(os.path.join(psf_dir, f"Angle{angle}.tif"), True, ctx=ctx))   # :579
+        else:
+            psfs.append(default_psf())
+    log(f"views {[angles[v] for v in mine]}: acquire, align, weights")
+    r = S.simulateDataset(gt, psfs, angles, angleOffset, attenuation, lightsheetSpacing, poissonSNR, osem, JavaRandom(S.seed),
+                          views=mine, ctx=ctx, sum_weights=rank == 0)
+    gt.free()
+    for i, v in enumerate(mine):
+        angle = angles[v]
+        save(r["acq"][i], f"acq_view_{angle}.tif")                                      # :598-604
+        save(r["aligned"][i], f"aligned_view_{angle}.tif")
+        save(r["aligned_psf"][i], f"aligned_view_psf_{angle}.tif")
+        save(r["weights"][i], f"aligned_view_weights{v * angle_increment}.tif")         # :642-646
+    if rank == 0:
+        save(r["sum_weights"], "sum_weights.tif")                                       # :663
+        res["sum_weights"] = r["sum_weights"]
+    for key, src in (("acq", "acq"), ("view", "aligned"), ("psf", "aligned_psf"), ("weights", "weights")):
+        if key in keep:
+            res[key] = r[src]
     res["seconds"] = time.perf_counter() - t_start
     log("done")
     return res
@@ -193,8 +265,16 @@ def _cli():
     ap.add_argument("--angle-increment", type=int, default=52)
     ap.add_argument("--snr", type=float, default=25.0)
     ap.add_argument("--psf-dir", default=None, help="directory with the reference's Angle<angle>.tif PSFs")
+    ap.add_argument("--fused", action="store_true", help="the whole view loop in one device call (simulate_dataset); "
+                    "writes no rot / att / con / iso volumes")
+    ap.add_argument("--rank", type=int, default=0, help="with --fused: simulate the views v %% world == rank")
+    ap.add_argument("--world", type=int, default=1)
     a = ap.parse_args()
-    r = run_main(a.out, size=a.size, angle_increment=a.angle_increment, poissonSNR=a.snr, psf_dir=a.psf_dir, keep=())
+    if a.fused:
+        r = simulate_dataset(a.out, size=a.size, angle_increment=a.angle_increment, poissonSNR=a.snr, psf_dir=a.psf_dir, keep=(),
+                             rank=a.rank, world=a.world)
+    else:
+        r = run_main(a.out, size=a.size, angle_increment=a.angle_increment, poissonSNR=a.snr, psf_dir=a.psf_dir, keep=())
     print(f"{len(r['angles'])} views of {a.size}^3 in {r['seconds']:.2f} s -> {a.out}")
 
 
