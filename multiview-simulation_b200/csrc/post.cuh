@@ -1,5 +1,7 @@
-// Row and tap arithmetic of the post-acquisition chain of main() (S/SimulateMultiViewDataset.java:576-663): the rotation rows of
-// rotate_axis0_kernel, the z blend of makeIsotropic, the weight taper of computeWeightImage and the weight normalisation.
+// Row and tap arithmetic of the rotation about x and of the attenuation (S/SimulateMultiViewDataset.java:104-135, :318-364) and of
+// the post-acquisition chain of main() (:576-663): the rotation rows and their blend, the attenuation recurrence, the z blend of
+// makeIsotropic, the weight taper of computeWeightImage and the weight normalisation.  Every kernel that rotates about x or
+// attenuates calls these functions, so their results agree bit for bit.
 // __host__ __device__: the kernels in stages.cu and the CPU harness in tests/emu run this same code.  Every operation is an
 // explicitly rounded IEEE operation (intrinsics on the device, plain operators on the host), so nothing is contracted into an FMA.
 #pragma once
@@ -21,6 +23,14 @@ MVSIM_HD double dadd_rn(double a, double b)
     return __dadd_rn(a, b);
 #else
     return a + b;
+#endif
+}
+MVSIM_HD double dsub_rn(double a, double b)
+{
+#ifdef __CUDA_ARCH__
+    return __dsub_rn(a, b);
+#else
+    return a - b;
 #endif
 }
 MVSIM_HD float fmul_rn(float a, float b)
@@ -72,10 +82,57 @@ MVSIM_HD RowTaps axis0_row_taps(int y, int z, const Affine& a)
     return t;
 }
 
-// imglib2's tap order 000, 100, 110, 010 reduced to (y, z): (iy, iz), (iy+1, iz), (iy+1, iz+1), (iy, iz+1)
-MVSIM_HD float axis0_blend(float t00, float t10, float t11, float t01, const RowTaps& t)
+// The row taps of an X x Y x Z volume (< 2^31 voxels) as element offsets from the row's x: the source rows (iy, iz), (iy+1, iz),
+// (iy+1, iz+1), (iy, iz+1).  A tap outside the volume gets weight 0 and the offset of row (0, 0), so a march reads all four rows
+// without a bounds test.  Its product f32(s * 0) with the voxel s of row (0, 0) is +0, like the product of the zero a bounds test
+// substitutes, whenever s is finite and neither negative nor -0.  So for finite source data without negative values, which every
+// generator here produces, the blend is bit-identical to the bounds-tested one.  For other finite data only the sign of a zero can
+// differ: with all four taps outside and a negative voxel in row (0, 0) the blend is -0 where the bounds test gives +0.
+struct alignas(16) RowTapsOff { unsigned o00, o10, o11, o01; float w00, w10, w11, w01; };
+
+MVSIM_HD RowTapsOff axis0_row_offsets(const RowTaps& t, int X, int Y, int Z)
+{
+    const bool y0 = (unsigned)t.iy < (unsigned)Y, y1 = (unsigned)(t.iy + 1) < (unsigned)Y;
+    const bool z0 = (unsigned)t.iz < (unsigned)Z, z1 = (unsigned)(t.iz + 1) < (unsigned)Z;
+    const unsigned sy = (unsigned)X, sz = (unsigned)X * (unsigned)Y;
+    RowTapsOff o;
+    o.o00 = (y0 && z0) ? sy * (unsigned)t.iy + sz * (unsigned)t.iz : 0u;
+    o.o10 = (y1 && z0) ? sy * (unsigned)(t.iy + 1) + sz * (unsigned)t.iz : 0u;
+    o.o11 = (y1 && z1) ? sy * (unsigned)(t.iy + 1) + sz * (unsigned)(t.iz + 1) : 0u;
+    o.o01 = (y0 && z1) ? sy * (unsigned)t.iy + sz * (unsigned)(t.iz + 1) : 0u;
+    o.w00 = (y0 && z0) ? t.w00 : 0.f;
+    o.w10 = (y1 && z0) ? t.w10 : 0.f;
+    o.w11 = (y1 && z1) ? t.w11 : 0.f;
+    o.w01 = (y0 && z1) ? t.w01 : 0.f;
+    return o;
+}
+
+// imglib2's tap order 000, 100, 110, 010 reduced to (y, z): (iy, iz), (iy+1, iz), (iy+1, iz+1), (iy, iz+1); Taps: RowTaps or RowTapsOff
+template <class Taps> MVSIM_HD float axis0_blend(float t00, float t10, float t11, float t01, const Taps& t)
 {
     return fadd_rn(fadd_rn(fadd_rn(fmul_rn(t00, t.w00), fmul_rn(t10, t.w10)), fmul_rn(t11, t.w11)), fmul_rn(t01, t.w01));
+}
+
+// Math.max(d, 0) of :354 for a non-NaN d through the sign bit (one compare + two selects instead of the four instructions of a
+// double-precision fmax on the device); -0.0 gives +0.0 like Math.max
+MVSIM_HD double clamp0(double d)
+{
+#ifdef __CUDA_ARCH__
+    return __double2hiint(d) < 0 ? 0.0 : d;
+#else
+    return signbit(d) ? 0.0 : d;
+#endif
+}
+
+// One row of attenuate's recurrence (:343-357) with n the light left in the column: phi = v * delta * n, n = max(n - phi, 0),
+// result f32(v * n).  SIGN_CLAMP takes the max through clamp0, which equals fmax for every non-NaN difference.
+template <bool SIGN_CLAMP = false> MVSIM_HD float attenuate_step(float v, double delta, double& n)
+{
+    const double dv = (double)v;
+    const double phi = dmul_rn(dmul_rn(dv, delta), n);
+    const double d = dsub_rn(n, phi);
+    n = SIGN_CLAMP ? clamp0(d) : fmax(d, 0.0);
+    return (float)dmul_rn(dv, n);
 }
 
 // makeIsotropic (:144-171) at plane zo of the up-sampled volume: position (float)zo / (float)inc widened to double (:165), two taps

@@ -9,8 +9,6 @@
 // full 128-byte line (float4 where the row length allows).
 #include <stdlib.h>
 
-#include <type_traits>
-
 #include "ctx.h"
 #include "post.cuh"
 #include "sampler.cuh"
@@ -30,6 +28,25 @@ static inline unsigned blocks_for(size_t n, unsigned threads) { return (unsigned
 // rotate.  Inverse affine applied in FP64 in mpicbg's evaluation order, floor + fractional weights in
 // FP64, blend in FP32 in imglib2's tap order (000,100,110,010,011,111,101,001), zero outside.
 // ---------------------------------------------------------------------------------------------
+template <int VEC> struct VecT;
+template <> struct VecT<1> { using type = float; };
+template <> struct VecT<2> { using type = float2; };
+template <> struct VecT<4> { using type = float4; };
+
+template <int VEC> __device__ __forceinline__ void vload(float (&d)[VEC], const float* p, bool ok)
+{
+    using V = typename VecT<VEC>::type;
+    if (ok) {
+        const V v = __ldg(reinterpret_cast<const V*>(p));
+        const float* f = reinterpret_cast<const float*>(&v);
+#pragma unroll
+        for (int i = 0; i < VEC; ++i) d[i] = f[i];
+    } else {
+#pragma unroll
+        for (int i = 0; i < VEC; ++i) d[i] = 0.f;
+    }
+}
+
 // axis 0: x_src == x (row 0 of the inverse is the identity), so the source coordinates are constant
 // along a row and the gather is bilinear in (y,z): VEC contiguous voxels per thread, 4 coalesced loads.
 template <int VEC> __global__ void __launch_bounds__(256) rotate_axis0_kernel(const float* __restrict__ in, float* __restrict__ out,
@@ -42,41 +59,21 @@ template <int VEC> __global__ void __launch_bounds__(256) rotate_axis0_kernel(co
     const int xv = (int)(idx % XV);
     const long long yz = idx / XV;
     const int y = (int)(yz % Y), z = (int)(yz / Y);
-    const double ly = (double)y, lz = (double)z;
-    // l0*m10 + l1*m11 + l2*m12 + m13 with m10 == 0
-    const double py = __dadd_rn(__dadd_rn(__dmul_rn(ly, a.m[5]), __dmul_rn(lz, a.m[6])), a.m[7]);
-    const double pz = __dadd_rn(__dadd_rn(__dmul_rn(ly, a.m[9]), __dmul_rn(lz, a.m[10])), a.m[11]);
-    const double fy = floor(py), fz = floor(pz);
-    const double wy = py - fy, wz = pz - fz;
-    const double wyi = 1.0 - wy, wzi = 1.0 - wz;
-    // clamp before the int conversion: far outside is simply "no tap"
-    const int iy = (int)fmax(fmin(fy, 2.0e9), -2.0e9), iz = (int)fmax(fmin(fz, 2.0e9), -2.0e9);
-    const float w00 = (float)(wyi * wzi), w10 = (float)(wy * wzi), w11 = (float)(wy * wz), w01 = (float)(wyi * wz);
-    const bool y0 = (unsigned)iy < (unsigned)Y, y1 = (unsigned)(iy + 1) < (unsigned)Y;
-    const bool z0 = (unsigned)iz < (unsigned)Z, z1 = (unsigned)(iz + 1) < (unsigned)Z;
+    const RowTaps t = axis0_row_taps(y, z, a);
+    const bool y0 = (unsigned)t.iy < (unsigned)Y, y1 = (unsigned)(t.iy + 1) < (unsigned)Y;
+    const bool z0 = (unsigned)t.iz < (unsigned)Z, z1 = (unsigned)(t.iz + 1) < (unsigned)Z;
     const long long x0 = (long long)xv * VEC;
-    const long long r00 = x0 + (long long)X * (iy + (long long)Y * iz);
+    const long long r00 = x0 + (long long)X * (t.iy + (long long)Y * t.iz);
     const long long sy = X, sz = (long long)X * Y;
     float* o = out + x0 + (long long)X * (y + (long long)Y * z);
-    if (VEC == 4) {
-        const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
-        const float4 t00 = (y0 && z0) ? __ldg(reinterpret_cast<const float4*>(in + r00)) : zero;
-        const float4 t10 = (y1 && z0) ? __ldg(reinterpret_cast<const float4*>(in + r00 + sy)) : zero;
-        const float4 t11 = (y1 && z1) ? __ldg(reinterpret_cast<const float4*>(in + r00 + sy + sz)) : zero;
-        const float4 t01 = (y0 && z1) ? __ldg(reinterpret_cast<const float4*>(in + r00 + sz)) : zero;
-        float4 r;
-        r.x = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(t00.x, w00), __fmul_rn(t10.x, w10)), __fmul_rn(t11.x, w11)), __fmul_rn(t01.x, w01));
-        r.y = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(t00.y, w00), __fmul_rn(t10.y, w10)), __fmul_rn(t11.y, w11)), __fmul_rn(t01.y, w01));
-        r.z = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(t00.z, w00), __fmul_rn(t10.z, w10)), __fmul_rn(t11.z, w11)), __fmul_rn(t01.z, w01));
-        r.w = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(t00.w, w00), __fmul_rn(t10.w, w10)), __fmul_rn(t11.w, w11)), __fmul_rn(t01.w, w01));
-        *reinterpret_cast<float4*>(o) = r;
-    } else {
-        const float t00 = (y0 && z0) ? __ldg(in + r00) : 0.f;
-        const float t10 = (y1 && z0) ? __ldg(in + r00 + sy) : 0.f;
-        const float t11 = (y1 && z1) ? __ldg(in + r00 + sy + sz) : 0.f;
-        const float t01 = (y0 && z1) ? __ldg(in + r00 + sz) : 0.f;
-        *o = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(t00, w00), __fmul_rn(t10, w10)), __fmul_rn(t11, w11)), __fmul_rn(t01, w01));
-    }
+    float t00[VEC], t10[VEC], t11[VEC], t01[VEC], r[VEC];
+    vload<VEC>(t00, in + r00, y0 && z0);
+    vload<VEC>(t10, in + r00 + sy, y1 && z0);
+    vload<VEC>(t11, in + r00 + sy + sz, y1 && z1);
+    vload<VEC>(t01, in + r00 + sz, y0 && z1);
+#pragma unroll
+    for (int i = 0; i < VEC; ++i) r[i] = axis0_blend(t00[i], t10[i], t11[i], t01[i], t);
+    *reinterpret_cast<typename VecT<VEC>::type*>(o) = *reinterpret_cast<typename VecT<VEC>::type*>(r);
 }
 
 __global__ void __launch_bounds__(256) rotate_general_kernel(const float* __restrict__ in, float* __restrict__ out,
@@ -115,9 +112,9 @@ __global__ void __launch_bounds__(256) rotate_general_kernel(const float* __rest
 
 // ---------------------------------------------------------------------------------------------
 // fused rotate (axis 0) + attenuate for the whole-view entry point: the rotated volume never goes to HBM.
-// A tiny pre-pass tabulates, per output row (y,z), the source row pair and the four bilinear weights
-// (exactly the arithmetic of rotate_axis0_kernel); the main kernel marches every (x,z) column from
-// y = Y-1 down, gathers the rotated voxel from the ground truth and applies the recurrence of :343-357.
+// A tiny pre-pass tabulates, per output row (y,z), the row taps of rotate_axis0_kernel (post.cuh); the main
+// kernel marches every (x,z) column from y = Y-1 down, gathers the rotated voxel from the ground truth and
+// applies the recurrence of :343-357.
 // ---------------------------------------------------------------------------------------------
 // rows (y, z) of the output planes [z0, z0 + Zl): entry (z - z0) * Y + y  (RowTaps, axis0_row_taps: post.cuh)
 __global__ void __launch_bounds__(256) rotate_rowtable_kernel(RowTaps* __restrict__ tab, int Y, int z0, int Zl, Affine a)
@@ -127,28 +124,8 @@ __global__ void __launch_bounds__(256) rotate_rowtable_kernel(RowTaps* __restric
     tab[i] = axis0_row_taps((int)(i % Y), z0 + (int)(i / Y), a);
 }
 
-template <int VEC> struct VecT;
-template <> struct VecT<1> { using type = float; };
-template <> struct VecT<2> { using type = float2; };
-template <> struct VecT<4> { using type = float4; };
-
-template <int VEC> __device__ __forceinline__ void vload(float (&d)[VEC], const float* p, bool ok)
-{
-    using V = typename VecT<VEC>::type;
-    if (ok) {
-        const V v = __ldg(reinterpret_cast<const V*>(p));
-        const float* f = reinterpret_cast<const float*>(&v);
-#pragma unroll
-        for (int i = 0; i < VEC; ++i) d[i] = f[i];
-    } else {
-#pragma unroll
-        for (int i = 0; i < VEC; ++i) d[i] = 0.f;
-    }
-}
-
-// IDX32: the volume has < 2^31 voxels (every volume an ImgLib2 ArrayImg can hold), element offsets are 32-bit (wrapping unsigned
-// arithmetic: offsets of taps that are masked off may wrap, the ones that are dereferenced are exact)
-template <int VEC, int U, bool IDX32> __global__ void __launch_bounds__(128) rotate_attenuate_kernel(const float* __restrict__ in, float* __restrict__ out,
+// bounds-tested march: volumes of 2^31 voxels or more, or X % 4 != 0
+template <int VEC, int U> __global__ void __launch_bounds__(128) rotate_attenuate_kernel(const float* __restrict__ in, float* __restrict__ out,
                                                                                         const RowTaps* __restrict__ tab, int X, int Y, int Z,
                                                                                         double delta, int steps, int Zl)
 {
@@ -159,10 +136,9 @@ template <int VEC, int U, bool IDX32> __global__ void __launch_bounds__(128) rot
     const long long col = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (col >= (long long)XV * Zl) return;
     const int x0 = (int)(col % XV) * VEC, z = (int)(col / XV);      // z: local plane
-    using Off = typename std::conditional<IDX32, unsigned, long long>::type;
-    const Off sy = (Off)X, sz = (Off)X * (Off)Y;
+    const long long sy = X, sz = (long long)X * Y;
     const RowTaps* trow = tab + (long long)Y * z;
-    const Off obase = (Off)x0 + sz * (Off)z;
+    const long long obase = x0 + sz * z;
     double n[VEC];
 #pragma unroll
     for (int i = 0; i < VEC; ++i) n[i] = 1.0;
@@ -187,25 +163,18 @@ template <int VEC, int U, bool IDX32> __global__ void __launch_bounds__(128) rot
             const int iy = tp[j].iy, iz = tp[j].iz;
             const bool y0 = (unsigned)iy < (unsigned)Y, y1 = (unsigned)(iy + 1) < (unsigned)Y;
             const bool z0 = (unsigned)iz < (unsigned)Z, z1 = (unsigned)(iz + 1) < (unsigned)Z;
-            const Off r = (Off)x0 + sy * (Off)iy + sz * (Off)iz;
+            const long long r = x0 + sy * iy + sz * iz;
             vload<VEC>(t00[j], in + r, y0 && z0);
-            vload<VEC>(t10[j], in + (Off)(r + sy), y1 && z0);
-            vload<VEC>(t11[j], in + (Off)(r + sy + sz), y1 && z1);
-            vload<VEC>(t01[j], in + (Off)(r + sz), y0 && z1);
+            vload<VEC>(t10[j], in + (r + sy), y1 && z0);
+            vload<VEC>(t11[j], in + (r + sy + sz), y1 && z1);
+            vload<VEC>(t01[j], in + (r + sz), y0 && z1);
         }
 #pragma unroll
         for (int j = 0; j < U; ++j) {
             float res[VEC];
 #pragma unroll
-            for (int i = 0; i < VEC; ++i) {
-                const float v = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(t00[j][i], tp[j].w00), __fmul_rn(t10[j][i], tp[j].w10)),
-                                                    __fmul_rn(t11[j][i], tp[j].w11)), __fmul_rn(t01[j][i], tp[j].w01));
-                const double dv = (double)v;
-                const double phi = __dmul_rn(__dmul_rn(dv, delta), n[i]);
-                n[i] = fmax(__dsub_rn(n[i], phi), 0.0);
-                res[i] = (float)__dmul_rn(dv, n[i]);
-            }
-            *reinterpret_cast<V*>(out + (Off)(obase + sy * (Off)(y - j))) = *reinterpret_cast<V*>(res);
+            for (int i = 0; i < VEC; ++i) res[i] = attenuate_step(axis0_blend(t00[j][i], t10[j][i], t11[j][i], t01[j][i], tp[j]), delta, n[i]);
+            *reinterpret_cast<V*>(out + (obase + sy * (y - j))) = *reinterpret_cast<V*>(res);
         }
 #pragma unroll
         for (int j = 0; j < U; ++j) tp[j] = tn[j];
@@ -214,62 +183,30 @@ template <int VEC, int U, bool IDX32> __global__ void __launch_bounds__(128) rot
         const RowTaps t = trow[y];
         const bool y0 = (unsigned)t.iy < (unsigned)Y, y1 = (unsigned)(t.iy + 1) < (unsigned)Y;
         const bool z0 = (unsigned)t.iz < (unsigned)Z, z1 = (unsigned)(t.iz + 1) < (unsigned)Z;
-        const Off r = (Off)x0 + sy * (Off)t.iy + sz * (Off)t.iz;
+        const long long r = x0 + sy * t.iy + sz * t.iz;
         float a00[VEC], a10[VEC], a11[VEC], a01[VEC], res[VEC];
         vload<VEC>(a00, in + r, y0 && z0);
-        vload<VEC>(a10, in + (Off)(r + sy), y1 && z0);
-        vload<VEC>(a11, in + (Off)(r + sy + sz), y1 && z1);
-        vload<VEC>(a01, in + (Off)(r + sz), y0 && z1);
+        vload<VEC>(a10, in + (r + sy), y1 && z0);
+        vload<VEC>(a11, in + (r + sy + sz), y1 && z1);
+        vload<VEC>(a01, in + (r + sz), y0 && z1);
 #pragma unroll
-        for (int i = 0; i < VEC; ++i) {
-            const float v = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(a00[i], t.w00), __fmul_rn(a10[i], t.w10)), __fmul_rn(a11[i], t.w11)),
-                                      __fmul_rn(a01[i], t.w01));
-            const double dv = (double)v;
-            const double phi = __dmul_rn(__dmul_rn(dv, delta), n[i]);
-            n[i] = fmax(__dsub_rn(n[i], phi), 0.0);
-            res[i] = (float)__dmul_rn(dv, n[i]);
-        }
-        *reinterpret_cast<V*>(out + (Off)(obase + sy * (Off)y)) = *reinterpret_cast<V*>(res);
+        for (int i = 0; i < VEC; ++i) res[i] = attenuate_step(axis0_blend(a00[i], a10[i], a11[i], a01[i], t), delta, n[i]);
+        *reinterpret_cast<V*>(out + (obase + sy * y)) = *reinterpret_cast<V*>(res);
     }
     float zero[VEC];
 #pragma unroll
     for (int i = 0; i < VEC; ++i) zero[i] = 0.f;
-    for (; y >= 0; --y) *reinterpret_cast<V*>(out + (Off)(obase + sy * (Off)y)) = *reinterpret_cast<V*>(zero);
+    for (; y >= 0; --y) *reinterpret_cast<V*>(out + (obase + sy * y)) = *reinterpret_cast<V*>(zero);
 }
 
-// The same march with the tap ADDRESSES tabulated: per output row (y, z) the table holds the four element offsets of the source rows
-// (iy, iz), (iy+1, iz), (iy+1, iz+1), (iy, iz+1) and the four weights; a tap outside the volume gets weight 0 and the offset of row
-// (0, 0), so the march issues four unconditional float4 loads per row and spends no instruction on bounds (ncu r02c: half of the
-// kernel's cycles issue, a quarter of its instructions were offsets, bound predicates and the zero fill of masked taps).  The blend
-// fmul(t, 0) = 0 of such a tap equals the blend of the zero the bounds check substituted (finite source data), so the result is
-// bit-identical to rotate_attenuate_kernel.  Volumes below 2^31 voxels, X % 4 == 0.
-struct __align__(16) RowTapsOff { unsigned o00, o10, o11, o01; float w00, w10, w11, w01; };
-
+// The same march with the tap ADDRESSES tabulated (RowTapsOff, axis0_row_offsets: post.cuh): four unconditional float4 loads per
+// row and no instruction on bounds (ncu r02c: half of the kernel's cycles issue, a quarter of its instructions were offsets, bound
+// predicates and the zero fill of masked taps).  Volumes below 2^31 voxels, X % 4 == 0.
 __global__ void __launch_bounds__(256) rotate_rowtable_off_kernel(RowTapsOff* __restrict__ tab, int X, int Y, int Z, int z0, int Zl, Affine a)
 {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (long long)Y * Zl) return;
-    const int y = (int)(i % Y), z = z0 + (int)(i / Y);
-    const double ly = (double)y, lz = (double)z;
-    const double py = __dadd_rn(__dadd_rn(__dmul_rn(ly, a.m[5]), __dmul_rn(lz, a.m[6])), a.m[7]);
-    const double pz = __dadd_rn(__dadd_rn(__dmul_rn(ly, a.m[9]), __dmul_rn(lz, a.m[10])), a.m[11]);
-    const double fy = floor(py), fz = floor(pz);
-    const double wy = py - fy, wz = pz - fz;
-    const double wyi = 1.0 - wy, wzi = 1.0 - wz;
-    const int iy = (int)fmax(fmin(fy, 2.0e9), -2.0e9), iz = (int)fmax(fmin(fz, 2.0e9), -2.0e9);
-    const bool y0 = (unsigned)iy < (unsigned)Y, y1 = (unsigned)(iy + 1) < (unsigned)Y;
-    const bool z0b = (unsigned)iz < (unsigned)Z, z1 = (unsigned)(iz + 1) < (unsigned)Z;
-    const unsigned sy = (unsigned)X, sz = (unsigned)X * (unsigned)Y;
-    RowTapsOff t;
-    t.o00 = (y0 && z0b) ? sy * (unsigned)iy + sz * (unsigned)iz : 0u;
-    t.o10 = (y1 && z0b) ? sy * (unsigned)(iy + 1) + sz * (unsigned)iz : 0u;
-    t.o11 = (y1 && z1) ? sy * (unsigned)(iy + 1) + sz * (unsigned)(iz + 1) : 0u;
-    t.o01 = (y0 && z1) ? sy * (unsigned)iy + sz * (unsigned)(iz + 1) : 0u;
-    t.w00 = (y0 && z0b) ? (float)(wyi * wzi) : 0.f;
-    t.w10 = (y1 && z0b) ? (float)(wy * wzi) : 0.f;
-    t.w11 = (y1 && z1) ? (float)(wy * wz) : 0.f;
-    t.w01 = (y0 && z1) ? (float)(wyi * wz) : 0.f;
-    tab[i] = t;
+    tab[i] = axis0_row_offsets(axis0_row_taps((int)(i % Y), z0 + (int)(i / Y), a), X, Y, Z);
 }
 
 // esz = sizeof(float) as a RUN-TIME value: tap addresses become one widening multiply-add (IMAD.WIDE.U32) each instead of the shift +
@@ -279,10 +216,8 @@ __device__ __forceinline__ float4 tap4(const float* base, unsigned off, unsigned
     return __ldg(reinterpret_cast<const float4*>(reinterpret_cast<const char*>(base) + (unsigned long long)off * (unsigned long long)esz));
 }
 
-// Math.max(d, 0) of :354 for a non-NaN d through the sign bit (one compare + two selects instead of the four instructions of a
-// double-precision fmax); -0.0 gives +0.0 like Math.max
-__device__ __forceinline__ double clamp0(double d) { return __double2hiint(d) < 0 ? 0.0 : d; }
-
+// The blend of an out-of-volume tap is f32(s * 0) with the voxel s of row (0, 0): bit-identical to rotate_attenuate_kernel for finite
+// source data without negative values (RowTapsOff).  The recurrence clamps through the sign bit (clamp0): the same as fmax there.
 template <int U> __global__ void __launch_bounds__(128) rotate_attenuate_off_kernel(const float* __restrict__ in, float* __restrict__ out,
                                                                                     const RowTapsOff* __restrict__ tab, int X, int Y,
                                                                                     double delta, int steps, int Zl, unsigned esz)
@@ -323,14 +258,7 @@ template <int U> __global__ void __launch_bounds__(128) rotate_attenuate_off_ker
             const float a11[4] = { t11[j].x, t11[j].y, t11[j].z, t11[j].w }, a01[4] = { t01[j].x, t01[j].y, t01[j].z, t01[j].w };
             float res[4];
 #pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const float v = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(a00[i], tp[j].w00), __fmul_rn(a10[i], tp[j].w10)),
-                                                    __fmul_rn(a11[i], tp[j].w11)), __fmul_rn(a01[i], tp[j].w01));
-                const double dv = (double)v;
-                const double phi = __dmul_rn(__dmul_rn(dv, delta), n[i]);
-                n[i] = clamp0(__dsub_rn(n[i], phi));
-                res[i] = (float)__dmul_rn(dv, n[i]);
-            }
+            for (int i = 0; i < 4; ++i) res[i] = attenuate_step<true>(axis0_blend(a00[i], a10[i], a11[i], a01[i], tp[j]), delta, n[i]);
             *reinterpret_cast<float4*>(dst + sy * (unsigned)(y - j)) = make_float4(res[0], res[1], res[2], res[3]);
         }
 #pragma unroll
@@ -343,17 +271,17 @@ template <int U> __global__ void __launch_bounds__(128) rotate_attenuate_off_ker
         const float a11[4] = { b11.x, b11.y, b11.z, b11.w }, a01[4] = { b01.x, b01.y, b01.z, b01.w };
         float res[4];
 #pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const float v = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(a00[i], t.w00), __fmul_rn(a10[i], t.w10)), __fmul_rn(a11[i], t.w11)),
-                                      __fmul_rn(a01[i], t.w01));
-            const double dv = (double)v;
-            const double phi = __dmul_rn(__dmul_rn(dv, delta), n[i]);
-            n[i] = clamp0(__dsub_rn(n[i], phi));
-            res[i] = (float)__dmul_rn(dv, n[i]);
-        }
+        for (int i = 0; i < 4; ++i) res[i] = attenuate_step<true>(axis0_blend(a00[i], a10[i], a11[i], a01[i], t), delta, n[i]);
         *reinterpret_cast<float4*>(dst + sy * (unsigned)y) = make_float4(res[0], res[1], res[2], res[3]);
     }
     for (; y >= 0; --y) *reinterpret_cast<float4*>(dst + sy * (unsigned)y) = make_float4(0.f, 0.f, 0.f, 0.f);
+}
+
+// a rotation about x: row 0 of the inverse is the identity (up to the rounding of (c^2+s^2) * 1/(c^2+s^2), < 1e-15), so x_src == x
+// and the gather is bilinear in (y, z)
+static bool x_identity(int axis, const double inv[12])
+{
+    return axis == 0 && fabs(inv[0] - 1.0) < 1e-12 && inv[1] == 0.0 && inv[2] == 0.0 && inv[3] == 0.0 && inv[4] == 0.0 && inv[8] == 0.0;
 }
 
 // returns MVSIM_EUNSUPPORTED when the fused path does not apply (caller falls back to the two kernels)
@@ -362,9 +290,7 @@ int k_rotate_attenuate(mvsim_ctx* ctx, const float* in, float* out, const int64_
 {
     const int X = (int)dims[0], Y = (int)dims[1], Z = (int)dims[2];
     const int Zl = z_local > 0 ? (int)z_local : Z, zfirst = z_local > 0 ? (int)z0 : 0;
-    const bool x_identity = axis == 0 && fabs(inv[0] - 1.0) < 1e-12 && inv[1] == 0.0 && inv[2] == 0.0 && inv[3] == 0.0 &&
-                            inv[4] == 0.0 && inv[8] == 0.0;
-    if (!x_identity) return MVSIM_EUNSUPPORTED;
+    if (!x_identity(axis, inv)) return MVSIM_EUNSUPPORTED;
     Affine a;
     for (int i = 0; i < 12; ++i) a.m[i] = inv[i];
     const bool aligned = (reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out)) % 16 == 0;
@@ -388,24 +314,19 @@ int k_rotate_attenuate(mvsim_ctx* ctx, const float* in, float* out, const int64_
     MVSIM_TRY(dev_alloc(ctx, (void**)&tab, sizeof(RowTaps) * (size_t)Y * Zl));
     rotate_rowtable_kernel<<<blocks_for((size_t)Y * Zl, 256), 256, 0, ctx->stream>>>(tab, Y, zfirst, Zl, a);
     ctx->launches++;
-    // the march along y is sequential per column, so the grid is small (X*Z/VEC threads): pick the widest
-    // vector whose single wave still fits the machine (config 3: 131072 threads x float4, 2 rows in flight)
-    const bool idx32 = (double)X * Y * Z < 2147483648.0;
+    // the march along y is sequential per column, so the grid is small (X*Z/VEC threads): the widest vector the row allows
     // (L2 prefetch of the source rows was measured and lost in both forms -- issued by thread 0: 0.905 -> 1.11 .. 1.31 ms; by a
     // fifth, paced warp per CTA: 1.04 .. 1.06 ms, profiles/r02_experiments.txt -- the march already keeps 2 rows x 4 taps in
     // flight per thread and re-reads every source row from the L2.)
     if (X % 4 == 0 && aligned) {
         const size_t cols = (size_t)(X / 4) * Zl;
-        // measured on B200, config 3 (profiles/r02_notes.md): <4, 2> 0.904 ms, <4, 3> 0.882, with the row taps of the next batch
-        // requested early <4, 2> 0.96 / <4, 3> 0.857; CTAs of 256 / 512 threads 0.950 / 0.956
-        if (idx32) rotate_attenuate_kernel<4, 3, true><<<blocks_for(cols, 128), 128, 0, ctx->stream>>>(in, out, tab, X, Y, Z, delta, steps, Zl);
-        else rotate_attenuate_kernel<4, 2, false><<<blocks_for(cols, 128), 128, 0, ctx->stream>>>(in, out, tab, X, Y, Z, delta, steps, Zl);
+        rotate_attenuate_kernel<4, 2><<<blocks_for(cols, 128), 128, 0, ctx->stream>>>(in, out, tab, X, Y, Z, delta, steps, Zl);
     } else if (X % 2 == 0 && aligned) {
         const size_t cols = (size_t)(X / 2) * Zl;
-        rotate_attenuate_kernel<2, 4, false><<<blocks_for(cols, 128), 128, 0, ctx->stream>>>(in, out, tab, X, Y, Z, delta, steps, Zl);
+        rotate_attenuate_kernel<2, 4><<<blocks_for(cols, 128), 128, 0, ctx->stream>>>(in, out, tab, X, Y, Z, delta, steps, Zl);
     } else {
         const size_t cols = (size_t)X * Zl;
-        rotate_attenuate_kernel<1, 4, false><<<blocks_for(cols, 128), 128, 0, ctx->stream>>>(in, out, tab, X, Y, Z, delta, steps, Zl);
+        rotate_attenuate_kernel<1, 4><<<blocks_for(cols, 128), 128, 0, ctx->stream>>>(in, out, tab, X, Y, Z, delta, steps, Zl);
     }
     ctx->launches++;
     cudaError_t e = cudaGetLastError();
@@ -419,10 +340,7 @@ int k_rotate(mvsim_ctx* ctx, const float* in, float* out, const int64_t dims[3],
     Affine a;
     for (int i = 0; i < 12; ++i) a.m[i] = inv[i];
     const int X = (int)dims[0], Y = (int)dims[1], Z = (int)dims[2];
-    // row 0 == identity (up to the rounding of (c^2+s^2) * 1/(c^2+s^2), < 1e-15): bilinear fast path
-    const bool x_identity = axis == 0 && fabs(inv[0] - 1.0) < 1e-12 && inv[1] == 0.0 && inv[2] == 0.0 && inv[3] == 0.0 &&
-                            inv[4] == 0.0 && inv[8] == 0.0;
-    if (x_identity) {
+    if (x_identity(axis, inv)) {
         const bool vec4 = (X % 4 == 0) && ((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out)) % 16 == 0);
         if (vec4) {
             const size_t total = (size_t)(X / 4) * Y * Z;
@@ -441,8 +359,8 @@ int k_rotate(mvsim_ctx* ctx, const float* in, float* out, const int64_t dims[3],
 
 // ---------------------------------------------------------------------------------------------
 // attenuate.  One (x,z) column per thread (lanes along x: coalesced), marching from y = Y-1 down;
-// the FP64 recurrence of :343-357 is reproduced operation by operation (no FMA contraction).  The
-// loads do not depend on the recurrence, so they are issued 8 rows ahead.
+// the FP64 recurrence of :343-357 (attenuate_step: post.cuh).  The loads do not depend on the
+// recurrence, so they are issued 8 rows ahead.
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(128) attenuate_kernel(const float* __restrict__ in, float* __restrict__ out, int X, int Y, int Z,
                                                         double delta, int steps)
@@ -460,19 +378,9 @@ __global__ void __launch_bounds__(128) attenuate_kernel(const float* __restrict_
 #pragma unroll
         for (int j = 0; j < 8; ++j) v[j] = __ldg(p + (long long)(y - j) * X);
 #pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            const double dv = (double)v[j];
-            const double phi = __dmul_rn(__dmul_rn(dv, delta), n);
-            n = fmax(__dsub_rn(n, phi), 0.0);
-            o[(long long)(y - j) * X] = (float)__dmul_rn(dv, n);
-        }
+        for (int j = 0; j < 8; ++j) o[(long long)(y - j) * X] = attenuate_step(v[j], delta, n);
     }
-    for (; s < steps; ++s, --y) {
-        const double dv = (double)__ldg(p + (long long)y * X);
-        const double phi = __dmul_rn(__dmul_rn(dv, delta), n);
-        n = fmax(__dsub_rn(n, phi), 0.0);
-        o[(long long)y * X] = (float)__dmul_rn(dv, n);
-    }
+    for (; s < steps; ++s, --y) o[(long long)y * X] = attenuate_step(__ldg(p + (long long)y * X), delta, n);
     for (; y >= 0; --y) o[(long long)y * X] = 0.f;      // rows the reference loop never reaches stay 0 (:321)
 }
 
@@ -911,7 +819,7 @@ __global__ void __launch_bounds__(256) normalize_weights_kernel(WeightPtrs p, in
 #pragma unroll
     for (int k = 0; k < MVSIM_MAX_WEIGHT_VIEWS; ++k)
         if (k < n_views) {
-            const float o = sum == 0.f ? 0.f : fminf(1.0f, __fmul_rn(osem, __fdiv_rn(v[k], sum)));
+            const float o = normalized_weight(v[k], sum, osem);
             p.w[k][i] = o;
             s2 = __fadd_rn(s2, o);
         }

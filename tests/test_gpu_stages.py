@@ -3,6 +3,7 @@
 Tolerances (BASELINE.json north_star): max|a-b| / max|b| <= 1e-4 for rotation, attenuation,
 convolution and adjust; bit exact for voxel indexing / slice selection; Poisson by mean/variance and
 a two-sample KS test against the oracle's replay of the reference sampler."""
+import ctypes as C
 import math
 
 import numpy as np
@@ -67,6 +68,28 @@ def test_attenuate_strict_rejects_x_greater_y(mv, S):
         S.attenuate3d(np.ones((2, 4, 8), dtype=np.float32), 0.01)
     assert e.value.status == 1
     S.attenuate3d(np.ones((2, 4, 8), dtype=np.float32), 0.01, strict_reference=False)
+
+
+# ---- fused rotate + attenuate ------------------------------------------------------------------------
+# one shape per march kernel: X % 4 == 0 (offset table), X % 4 == 2 (float2), odd X (scalar); the phantom is non-negative, the
+# condition under which the offset table's out-of-volume taps give exactly the bounds-tested result
+@pytest.mark.parametrize("shape", [(24, 40, 32), (17, 34, 30), (9, 40, 13)])
+@pytest.mark.parametrize("strict,delta", [(True, 0.01), (False, 0.01), (False, 0.5)])
+def test_fused_rotate_attenuate_equals_rotate_then_attenuate_bitwise(mv, shape, strict, delta):
+    from mvsim_b200._lib import check, dims3
+    ctx = mv.Context(0)
+    lib = ctx._lib
+    gt, rot, att, fused = (mv.DeviceVolume(ctx, shape) for _ in range(4))
+    gt.upload(sphere_phantom(shape, n_spheres=20) * 3)
+    for deg in (0, 15, 60, 90, 135, 200, -52):
+        check(lib.mvsim_dev_rotate_axis(ctx.h, gt.h, rot.h, 0, deg), ctx.h)
+        check(lib.mvsim_dev_attenuate(ctx.h, rot.h, att.h, delta, int(strict)), ctx.h)
+        check(lib.mvsim_slab_rotate_attenuate(ctx.h, C.c_void_p(gt.device_ptr), dims3(shape), 0, deg, delta, int(strict), 0, shape[0],
+                                              C.c_void_p(fused.device_ptr)), ctx.h)
+        assert np.array_equal(fused.download().view(np.uint32), att.download().view(np.uint32)), deg
+    for v in (gt, rot, att, fused):
+        v.free()
+    ctx.close()
 
 
 # ---- normImage / convolve ----------------------------------------------------------------------------
