@@ -219,6 +219,13 @@ int mvsim_dev_psf_normalize(mvsim_ctx* ctx, mvsim_volume* psf, double* sum_out /
 int mvsim_dev_convolve(mvsim_ctx* ctx, const mvsim_volume* img, const mvsim_volume* psf, mvsim_volume* out);
 int mvsim_dev_adjust(mvsim_ctx* ctx, mvsim_volume* img, float min_value, float target_avg, double* correction_out /* nullable: no sync */);
 int mvsim_dev_extract_slices(mvsim_ctx* ctx, const mvsim_volume* in, int inc, float snr, uint64_t seed, uint64_t stream, mvsim_volume* out);
+/* extractSlices (:195-231) of Views.zeroMin(Views.interval(in, min, max)) (S/SimulateTileStitching.java:152-153,174) without
+ * materialising the view: min/max inclusive (x, y, z); out dims (max0-min0+1, max1-min1+1, (max2-min2)/inc+1).  Bit-identical to
+ * mvsim_dev_extract_slices of the dense cut with the same seed / stream.  MVSIM_EINVAL for a null pointer, in == out, inc < 1,
+ * an interval outside in (min < 0, max >= dims or min > max on any axis) or mismatched out dims; MVSIM_EUNSUPPORTED for a tile
+ * plane (max0-min0+1)*(max1-min1+1) of 2^32 voxels or more. */
+int mvsim_dev_extract_interval(mvsim_ctx* ctx, const mvsim_volume* in, const int64_t min[3], const int64_t max[3], int inc,
+                               float snr, uint64_t seed, uint64_t stream, mvsim_volume* out);
 /* gt: ground truth, psf: raw PSF (normalised in place), out: X*Y*((Z-1)/inc+1) */
 int mvsim_dev_simulate_view(mvsim_ctx* ctx, const mvsim_view_params* p, const mvsim_volume* gt, mvsim_volume* psf, mvsim_volume* out);
 /* the view loop (:567-613) on a ground truth that is already resident (uploaded once, generated on the device, or received from

@@ -94,6 +94,33 @@ final class Mvsim
 	/** weight normalisation of main() (:615-661), in place; sumOut may be null */
 	static native int normalizeWeights( long ctx, FloatBuffer[] weights, long[] dims, float osem, FloatBuffer sumOut );
 
+	/* ---- device-resident volumes (mvsim_volume handles cross as long; 0 = none) ----
+	 * Keep intermediates in GPU memory between calls, e.g. the two convolved volumes of the tile-stitching pair generator
+	 * (SimulateTileStitchingGPU): only what the caller downloads crosses the host link.  A handle belongs to the context it was
+	 * created on.  Uploads and downloads are asynchronous on the context's stream for pinned buffers: ctxSynchronize before the
+	 * host touches them. */
+	/** mvsim_volume_create: the handle, or 0 on failure (see lastError( ctx )) */
+	static native long volumeCreate( long ctx, long[] dims );
+	/** mvsim_volume_free */
+	static native int volumeFree( long ctx, long vol );
+	/** mvsim_volume_upload: host holds at least X*Y*Z floats of the volume's dims */
+	static native int volumeUpload( long ctx, long vol, FloatBuffer host );
+	/** mvsim_volume_download: host holds at least X*Y*Z floats of the volume's dims */
+	static native int volumeDownload( long ctx, long vol, FloatBuffer host );
+	/** simulate( halfPixelOffset, rnd ) (S/SimulateMultiViewDataset.java:371-392) into a size^3 volume; nSmallOut may be null */
+	static native int devSimulatePhantom( long ctx, int size, boolean halfPixelOffset, long seed, long out, long[] nSmallOut );
+	/** Tools.normImage (S/Tools.java:112) in place; sumOut may be null (then the call does not synchronise) */
+	static native int devPsfNormalize( long ctx, long psf, double[] sumOut );
+	/** attenuate3d (:318) */
+	static native int devAttenuate( long ctx, long in, long out, double delta, boolean strictReference );
+	/** convolve (:253) with a PSF already normalised by devPsfNormalize */
+	static native int devConvolve( long ctx, long img, long psf, long out );
+	/** Tools.adjustImage (S/Tools.java:143) in place; correctionOut may be null (then the call does not synchronise) */
+	static native int devAdjust( long ctx, long img, float minValue, float targetAverage, double[] correctionOut );
+	/** extractSlices (:195) of Views.zeroMin( Views.interval( in, min, max ) ) (S/SimulateTileStitching.java:152-153,174) read in
+	 * place: min / max inclusive (x, y, z); out dims (max0-min0+1, max1-min1+1, (max2-min2)/inc+1) */
+	static native int devExtractInterval( long ctx, long in, long[] min, long[] max, int inc, float poissonSNR, long seed, long stream, long out );
+
 	/** pinned off-heap float buffer of n elements, native byte order */
 	static FloatBuffer pinnedFloats( final long n )
 	{

@@ -383,3 +383,106 @@ MVSIM_JNI(jint, normalizeWeights)(JNIEnv* env, jclass c, jlong ctx, jobjectArray
     if (sum_out && !sum) return MVSIM_EINVAL;
     return mvsim_normalize_weights(ctx_of(ctx), w, (int)n, d, osem, sum);
 }
+
+/* ---- device-resident volumes ---------------------------------------------------------------------------------------- */
+static mvsim_volume* vol_of(jlong h) { return (mvsim_volume*)(intptr_t)h; }
+
+/* direct buffer address when it holds the whole volume, else NULL */
+static float* volume_floats_of(JNIEnv* env, jlong vol, jobject buf)
+{
+    int64_t d[3];
+    if (!vol || mvsim_volume_dims(vol_of(vol), d) != MVSIM_OK) return NULL;
+    return floats_of(env, buf, prod3(d));
+}
+
+/* three longs, any sign (interval bounds: the library checks them against the volume) */
+static int longs3_of(JNIEnv* env, jlongArray arr, int64_t v[3])
+{
+    if (!arr || (*env)->GetArrayLength(env, arr) < 3) return MVSIM_EINVAL;
+    jlong tmp[3];
+    (*env)->GetLongArrayRegion(env, arr, 0, 3, tmp);
+    for (int i = 0; i < 3; ++i) v[i] = (int64_t)tmp[i];
+    return MVSIM_OK;
+}
+
+MVSIM_JNI(jlong, volumeCreate)(JNIEnv* env, jclass c, jlong ctx, jlongArray dims)
+{
+    (void)c;
+    int64_t d[3];
+    mvsim_volume* v = NULL;
+    if (dims_of(env, dims, d) || mvsim_volume_create(ctx_of(ctx), d, &v) != MVSIM_OK) return 0;
+    return (jlong)(intptr_t)v;
+}
+
+MVSIM_JNI(jint, volumeFree)(JNIEnv* env, jclass c, jlong ctx, jlong vol)
+{
+    (void)env; (void)c;
+    return mvsim_volume_free(ctx_of(ctx), vol_of(vol));
+}
+
+MVSIM_JNI(jint, volumeUpload)(JNIEnv* env, jclass c, jlong ctx, jlong vol, jobject host)
+{
+    (void)c;
+    const float* src = volume_floats_of(env, vol, host);
+    if (!src) return MVSIM_EINVAL;
+    return mvsim_volume_upload(ctx_of(ctx), vol_of(vol), src);
+}
+
+MVSIM_JNI(jint, volumeDownload)(JNIEnv* env, jclass c, jlong ctx, jlong vol, jobject host)
+{
+    (void)c;
+    float* dst = volume_floats_of(env, vol, host);
+    if (!dst) return MVSIM_EINVAL;
+    return mvsim_volume_download(ctx_of(ctx), vol_of(vol), dst);
+}
+
+MVSIM_JNI(jint, devSimulatePhantom)(JNIEnv* env, jclass c, jlong ctx, jint size, jboolean half, jlong seed, jlong out, jlongArray n_small_out)
+{
+    (void)c;
+    int64_t n = 0;
+    const int st = mvsim_dev_simulate_phantom(ctx_of(ctx), size, half ? 1 : 0, (int64_t)seed, vol_of(out), &n);
+    if (st == MVSIM_OK && n_small_out && (*env)->GetArrayLength(env, n_small_out) >= 1) {
+        const jlong v = (jlong)n;
+        (*env)->SetLongArrayRegion(env, n_small_out, 0, 1, &v);
+    }
+    return st;
+}
+
+MVSIM_JNI(jint, devPsfNormalize)(JNIEnv* env, jclass c, jlong ctx, jlong psf, jdoubleArray sum_out)
+{
+    (void)c;
+    double sum = 0.0;
+    const int st = mvsim_dev_psf_normalize(ctx_of(ctx), vol_of(psf), sum_out ? &sum : NULL);
+    if (st == MVSIM_OK && sum_out && (*env)->GetArrayLength(env, sum_out) >= 1) (*env)->SetDoubleArrayRegion(env, sum_out, 0, 1, &sum);
+    return st;
+}
+
+MVSIM_JNI(jint, devAttenuate)(JNIEnv* env, jclass c, jlong ctx, jlong in, jlong out, jdouble delta, jboolean strict)
+{
+    (void)env; (void)c;
+    return mvsim_dev_attenuate(ctx_of(ctx), vol_of(in), vol_of(out), delta, strict ? 1 : 0);
+}
+
+MVSIM_JNI(jint, devConvolve)(JNIEnv* env, jclass c, jlong ctx, jlong img, jlong psf, jlong out)
+{
+    (void)env; (void)c;
+    return mvsim_dev_convolve(ctx_of(ctx), vol_of(img), vol_of(psf), vol_of(out));
+}
+
+MVSIM_JNI(jint, devAdjust)(JNIEnv* env, jclass c, jlong ctx, jlong img, jfloat min_value, jfloat target_avg, jdoubleArray corr_out)
+{
+    (void)c;
+    double corr = 0.0;
+    const int st = mvsim_dev_adjust(ctx_of(ctx), vol_of(img), min_value, target_avg, corr_out ? &corr : NULL);
+    if (st == MVSIM_OK && corr_out && (*env)->GetArrayLength(env, corr_out) >= 1) (*env)->SetDoubleArrayRegion(env, corr_out, 0, 1, &corr);
+    return st;
+}
+
+MVSIM_JNI(jint, devExtractInterval)(JNIEnv* env, jclass c, jlong ctx, jlong in, jlongArray min, jlongArray max, jint inc, jfloat snr, jlong seed,
+                                    jlong stream, jlong out)
+{
+    (void)c;
+    int64_t mn[3], mx[3];
+    if (longs3_of(env, min, mn) || longs3_of(env, max, mx)) return MVSIM_EINVAL;
+    return mvsim_dev_extract_interval(ctx_of(ctx), vol_of(in), mn, mx, inc, snr, (uint64_t)seed, (uint64_t)stream, vol_of(out));
+}

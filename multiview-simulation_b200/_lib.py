@@ -99,6 +99,7 @@ SYMBOLS = [
     ("mvsim_dev_convolve", C.c_int, [_vp, _vp, _vp, _vp]),
     ("mvsim_dev_adjust", C.c_int, [_vp, _vp, C.c_float, C.c_float, _dp]),
     ("mvsim_dev_extract_slices", C.c_int, [_vp, _vp, C.c_int, C.c_float, C.c_uint64, C.c_uint64, _vp]),
+    ("mvsim_dev_extract_interval", C.c_int, [_vp, _vp, _i64p, _i64p, C.c_int, C.c_float, C.c_uint64, C.c_uint64, _vp]),
     ("mvsim_dev_simulate_view", C.c_int, [_vp, C.POINTER(ViewParams), _vp, _vp, _vp]),
     ("mvsim_dev_simulate_views", C.c_int, [_vp, C.c_int, C.POINTER(ViewParams), _vp, C.POINTER(_fp), C.POINTER(_fp)]),
     ("mvsim_slabconv_create", C.c_int, [_vp, _i64p, _i64p, C.c_int, C.c_int, C.POINTER(_vp)]),

@@ -215,6 +215,35 @@ class DeviceVolume:
             self.ctx._lib.mvsim_volume_free(self.ctx.h, self.h)
             self.h = None
 
+    def extractSlices(self, inc, poissonSNR, rnd=None, stream=0, interval=None, out=None):
+        """extractSlices (:195-231) on the device: every inc-th plane, Poisson noise when poissonSNR >= 0.  interval = (min_xyz,
+        max_xyz), inclusive (SimulateTileStitching.getInterval's form), samples Views.zeroMin(Views.interval(self, min, max))
+        (S/SimulateTileStitching.java:152-153,174) in place, without a dense copy of the tile (mvsim_dev_extract_interval); the
+        result equals extractSlices of the dense cut, bit for bit.  None = the whole volume (mvsim_dev_extract_slices).  The seed
+        is drawn like SimulateMultiViewDataset.extractSlices.  Returns `out` or a new DeviceVolume of ((bz-1)//inc+1, by, bx)."""
+        if inc < 1:
+            raise MvsimError(_lib.MVSIM_EINVAL, "inc must be >= 1")
+        seed = _seed_from(rnd) if poissonSNR >= 0 else 0
+        if interval is None:
+            z, y, x = self.shape
+            out = DeviceVolume(self.ctx, ((z - 1) // inc + 1, y, x)) if out is None else out
+            check(self.ctx._lib.mvsim_dev_extract_slices(self.ctx.h, self.h, int(inc), float(poissonSNR), seed, int(stream), out.h),
+                  self.ctx.h)
+            return out
+        mn, mx = (tuple(int(v) for v in t) for t in interval)
+        new = out is None
+        if new:
+            out = DeviceVolume(self.ctx, ((mx[2] - mn[2]) // inc + 1, mx[1] - mn[1] + 1, mx[0] - mn[0] + 1))
+        i3 = C.c_int64 * 3
+        try:
+            check(self.ctx._lib.mvsim_dev_extract_interval(self.ctx.h, self.h, i3(*mn), i3(*mx), int(inc), float(poissonSNR), seed,
+                                                           int(stream), out.h), self.ctx.h)
+        except MvsimError:
+            if new:
+                out.free()
+            raise
+        return out
+
     def alignView(self, inc, degrees, out=None):
         """rotateAroundAxis(makeIsotropic(self, inc), 0, degrees) (:588, :591) of this acquired view, gathered on the device
         without the isotropic volume (mvsim_dev_align_view); returns `out` or a new DeviceVolume of ((Za-1)*inc+1, Y, X)."""

@@ -1336,6 +1336,20 @@ int mvsim_dev_extract_slices(mvsim_ctx* ctx, const mvsim_volume* in, int inc, fl
     return k_extract(ctx, in->d, in->dims, inc, nullptr, 0.f, snr, seed, stream, out->d);
 }
 
+int mvsim_dev_extract_interval(mvsim_ctx* ctx, const mvsim_volume* in, const int64_t min[3], const int64_t max[3], int inc,
+                               float snr, uint64_t seed, uint64_t stream, mvsim_volume* out)
+{
+    MVSIM_ENTER(ctx);
+    if (!in || !out || !min || !max || in == out || inc < 1) return set_error(ctx, MVSIM_EINVAL, "dev_extract_interval: bad argument");
+    for (int d = 0; d < 3; ++d)
+        if (min[d] < 0 || max[d] >= in->dims[d] || min[d] > max[d])
+            return set_error(ctx, MVSIM_EINVAL, "dev_extract_interval: interval must satisfy 0 <= min <= max < dims");
+    if (out->dims[0] != max[0] - min[0] + 1 || out->dims[1] != max[1] - min[1] + 1 || out->dims[2] != (max[2] - min[2]) / inc + 1)
+        return set_error(ctx, MVSIM_EINVAL, "dev_extract_interval: out dims must be (max0-min0+1, max1-min1+1, (max2-min2)/inc+1)");
+    StageTimer t(ctx, MVSIM_T_SAMPLE);
+    return k_extract_interval(ctx, in->d, in->dims, min, max, inc, snr, seed, stream, out->d);
+}
+
 int mvsim_dev_simulate_view(mvsim_ctx* ctx, const mvsim_view_params* p, const mvsim_volume* gt, mvsim_volume* psf, mvsim_volume* out)
 {
     MVSIM_ENTER(ctx);

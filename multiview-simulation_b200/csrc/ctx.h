@@ -107,6 +107,9 @@ int k_extract_u16(mvsim_ctx* ctx, const float* in, const int64_t dims[3], int in
 // out[x,y,cz] = f(in[x,y,cz*inc]); d_corr != null fuses adjustImage; snr >= 0 adds Poisson noise
 int k_extract(mvsim_ctx* ctx, const float* in, const int64_t dims[3], int inc, const double* d_corr, float min_value,
               float snr, uint64_t seed, uint64_t stream, float* out);
+// k_extract of the dense cut [min, max] (inclusive, x y z) of `in`, read in place; the bounds are the caller's to check
+int k_extract_interval(mvsim_ctx* ctx, const float* in, const int64_t dims[3], const int64_t min[3], const int64_t max[3], int inc,
+                       float snr, uint64_t seed, uint64_t stream, float* out);
 int k_make_isotropic(mvsim_ctx* ctx, const float* in, const int64_t dims[3], int inc, float* out);
 int k_weight_image(mvsim_ctx* ctx, const int64_t dims[3], float* out);
 int k_normalize_weights(mvsim_ctx* ctx, float* const* d_weights, int n_views, size_t n, float osem, float* d_sum_out);

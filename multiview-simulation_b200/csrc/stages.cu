@@ -12,6 +12,7 @@
 #include "ctx.h"
 #include "post.cuh"
 #include "sampler.cuh"
+#include "tile.cuh"
 
 namespace mvsim {
 
@@ -596,11 +597,16 @@ template <int G> struct WarpSamplerShared {
     int count;
 };
 
-template <bool VEC4, int G> __global__ void __launch_bounds__(kWarpSamplerThreads) extract_warp_kernel(const float* __restrict__ in, float* __restrict__ out, long long plane,
+// Source addressing: TILE = false reads output plane cz from input plane cz*inc + in_plane0 of a volume with the output's rows
+// (float4 loads when VEC4); TILE = true reads the output, a dense tile, from an interval of a larger parent through `tile`
+// (tile.cuh; scalar loads: tile rows start anywhere), with plane = bx*by, in_plane0 = group0 = 0, no d_corr and no out16.  VEC4
+// selects float4 stores in both.  `tile` is the last parameter, so the dense instantiations keep their code.
+template <bool VEC4, int G, bool TILE> __global__ void __launch_bounds__(kWarpSamplerThreads) extract_warp_kernel(const float* __restrict__ in, float* __restrict__ out, long long plane,
                                                                           long long n_out, int inc, const double* __restrict__ d_corr,
                                                                           float min_value, int noise, double mul, PoissonKey key,
                                                                           long long in_plane0, long long group0,
-                                                                          unsigned short* __restrict__ out16, int* __restrict__ overflow)
+                                                                          unsigned short* __restrict__ out16, int* __restrict__ overflow,
+                                                                          TileMap tile)
 {
     __shared__ WarpSamplerShared<G> shw[kWarpSamplerThreads / 32];
     const unsigned lane = threadIdx.x & 31u, w = threadIdx.x >> 5;
@@ -616,7 +622,13 @@ template <bool VEC4, int G> __global__ void __launch_bounds__(kWarpSamplerThread
 #pragma unroll
         for (int j = 0; j < 4; ++j) v[k][j] = 0.f;
         if (valid[k]) {
-            if (VEC4) {
+            if (TILE) {
+                long long off[4];
+                tile_group_offsets(tile, (uint64_t)i0, off);
+#pragma unroll
+                for (int j = 0; j < 4; ++j)
+                    if (i0 + j < n_out) v[k][j] = __ldg(in + off[j]);
+            } else if (VEC4) {
                 // inc == 1 (the whole-view call hands over the kept slices compacted): output voxel i reads input voxel
                 // i + in_plane0 * plane -- no 64-bit division (a library call of ~60 instructions per group, ncu r02j)
                 long long src_i = i0 + in_plane0 * plane;
@@ -755,8 +767,28 @@ int k_extract_slab(mvsim_ctx* ctx, const float* in, const int64_t dims[3], int64
     const long long in_plane0 = k0 * inc - z0, group0 = first / 4;
     if (out16 && (reinterpret_cast<uintptr_t>(out16) % 8 != 0 || !d_overflow)) return set_error(ctx, MVSIM_EINVAL, "extract: uint16 buffer must be 8-byte aligned");
     const unsigned wblocks = blocks_for((size_t)((n_out + 3) / 4), (unsigned)(kWarpSamplerThreads * 2));
-    if (vec4) extract_warp_kernel<true, 2><<<wblocks, kWarpSamplerThreads, 0, ctx->stream>>>(in, out, plane, n_out, inc, d_corr, min_value, noise, mul, key, in_plane0, group0, out16, d_overflow);
-    else extract_warp_kernel<false, 2><<<wblocks, kWarpSamplerThreads, 0, ctx->stream>>>(in, out, plane, n_out, inc, d_corr, min_value, noise, mul, key, in_plane0, group0, out16, d_overflow);
+    if (vec4) extract_warp_kernel<true, 2, false><<<wblocks, kWarpSamplerThreads, 0, ctx->stream>>>(in, out, plane, n_out, inc, d_corr, min_value, noise, mul, key, in_plane0, group0, out16, d_overflow, TileMap{});
+    else extract_warp_kernel<false, 2, false><<<wblocks, kWarpSamplerThreads, 0, ctx->stream>>>(in, out, plane, n_out, inc, d_corr, min_value, noise, mul, key, in_plane0, group0, out16, d_overflow, TileMap{});
+    MVSIM_LAUNCH_CHECK(ctx);
+    return MVSIM_OK;
+}
+
+// extractSlices of the interval [min, max] (inclusive, x y z) of a volume with dims, straight from the volume: the output and its
+// Philox counters (tile-local flat indices) are those of k_extract on the dense cut of the interval
+int k_extract_interval(mvsim_ctx* ctx, const float* in, const int64_t dims[3], const int64_t min[3], const int64_t max[3], int inc,
+                       float snr, uint64_t seed, uint64_t stream, float* out)
+{
+    const long long plane = (max[0] - min[0] + 1) * (max[1] - min[1] + 1);
+    if (plane > (long long)UINT32_MAX) return set_error(ctx, MVSIM_EUNSUPPORTED, "extract (interval): tile plane must hold < 2^32 voxels");
+    const long long n_out = plane * ((max[2] - min[2]) / inc + 1);
+    const TileMap tile = make_tile_map(dims, min, max, inc);
+    const bool vec4 = n_out % 4 == 0 && reinterpret_cast<uintptr_t>(out) % 16 == 0;
+    const int noise = snr >= 0.0f ? 1 : 0;
+    const double mul = snr_to_mul((double)snr);
+    const PoissonKey key = make_poisson_key(seed, stream);
+    const unsigned wblocks = blocks_for((size_t)((n_out + 3) / 4), (unsigned)(kWarpSamplerThreads * 2));
+    if (vec4) extract_warp_kernel<true, 2, true><<<wblocks, kWarpSamplerThreads, 0, ctx->stream>>>(in, out, plane, n_out, inc, nullptr, 0.f, noise, mul, key, 0, 0, nullptr, nullptr, tile);
+    else extract_warp_kernel<false, 2, true><<<wblocks, kWarpSamplerThreads, 0, ctx->stream>>>(in, out, plane, n_out, inc, nullptr, 0.f, noise, mul, key, 0, 0, nullptr, nullptr, tile);
     MVSIM_LAUNCH_CHECK(ctx);
     return MVSIM_OK;
 }

@@ -23,7 +23,7 @@ import numpy as np
 
 from . import tiff
 from ._lib import check
-from .api import Context, JavaRandom, SimulateMultiViewDataset as S, Tools
+from .api import Context, DeviceVolume, JavaRandom, SimulateMultiViewDataset as S, Tools
 
 # main(): angleIncrement -> osem factor (:536-546)
 OSEM = {60: 3.0, 52: 3.0, 45: 4.0}
@@ -182,7 +182,11 @@ def simulate_dataset(out_dir=None, size=289, angle_increment=52, osem=None, pois
 
 class SimulateTileStitching:
     """S/SimulateTileStitching.java:58-258: two convolved phantoms (with and without a half-pixel shift) are built by two
-    threads, then pairs of overlapping tiles are cut out of them and sampled (every 3rd slice + Poisson noise) at any SNR."""
+    threads, then pairs of overlapping tiles are cut out of them and sampled (every 3rd slice + Poisson noise) at any SNR.
+
+    Both convolved volumes stay on the device, each with the context of the thread that built it: a pair samples its two
+    tiles straight from them (DeviceVolume.extractSlices over the tile's interval) and only the tiles cross the host link.
+    `con` / `conHalfPixel` download the volumes on first access.  close() frees the volumes and the contexts."""
 
     lightsheetSpacing = 3           # :52
     attenuation = 0.01              # :53
@@ -192,33 +196,76 @@ class SimulateTileStitching:
         self.psf = default_psf() if psf is None else np.array(psf, dtype=np.float32, order="C", copy=True)              # :71
         self.size = size
         self.device = device
+        self._ctx, self._vol, self._host, self._tiles = {}, {}, {}, []
         self.init(overlapRatio, halfPixelOffset)
 
     def init(self, overlapRatio, halfPixelOffset):
+        self.close()
+        self._host = {}
         self.halfPixelOffset = halfPixelOffset
         seed = self.rnd.nextInt()                                                       # :83, same phantom for both
-        out = {}
+        raw = self.psf.copy()
+        errors = []
 
         def task(half, key):                                                            # :85-114: one pipeline per thread
-            ctx = Context(self.device)
-            gt = S.simulate(half, seed, size=self.size, ctx=ctx)
-            att = S.attenuate3d(gt, self.attenuation, ctx=ctx)
-            con = S.convolve(att, self.psf if key == "con" else self.psf.copy(), None, ctx=ctx)
-            Tools.adjustImage(con, S.minValue, S.avgIntensity, ctx=ctx)
-            out[key] = con
-            ctx.close()
+            shape = (self.size,) * 3
+            tmp = []
+            try:
+                ctx = self._ctx[key] = Context(self.device)
+                for shp, host in ((shape, None), (shape, None), (raw.shape, raw)):
+                    tmp.append(DeviceVolume(ctx, shp, host))
+                gt, att, psf = tmp
+                con = self._vol[key] = DeviceVolume(ctx, shape)
+                check(ctx._lib.mvsim_dev_simulate_phantom(ctx.h, self.size, int(half), seed, gt.h, C.byref(C.c_int64())), ctx.h)
+                check(ctx._lib.mvsim_dev_attenuate(ctx.h, gt.h, att.h, self.attenuation, 1), ctx.h)
+                check(ctx._lib.mvsim_dev_psf_normalize(ctx.h, psf.h, None), ctx.h)
+                check(ctx._lib.mvsim_dev_convolve(ctx.h, att.h, psf.h, con.h), ctx.h)
+                check(ctx._lib.mvsim_dev_adjust(ctx.h, con.h, S.minValue, S.avgIntensity, None), ctx.h)
+                if key == "con":
+                    psf.download(self.psf)                                              # convolve normalises its PSF in place (:255)
+                ctx.synchronize()
+            except Exception as e:
+                errors.append(e)
+            finally:
+                for v in tmp:
+                    v.free()
         threads = [threading.Thread(target=task, args=(False, "con")), threading.Thread(target=task, args=(True, "conHalfPixel"))]
         for t in threads:
             t.start()
         for t in threads:
             t.join()
-        self.con, self.conHalfPixel = out["con"], out["conHalfPixel"]
-        dims = self.con.shape[::-1]                                                     # x, y, z
+        if errors:
+            self.close()
+            raise errors[0]
+        dims = self._dims()
         self.overlap = [int(np.floor(dims[d] * overlapRatio[d] / 2 + 0.5)) for d in range(3)]   # Math.round, :121
+        # the two tiles' device outputs, on the context of the volume each is cut from; reused by every pair
+        for i, vol in enumerate(self._sources()):
+            mn, mx = self.getInterval(i)
+            self._tiles.append(DeviceVolume(vol.ctx, ((mx[2] - mn[2]) // self.lightsheetSpacing + 1, mx[1] - mn[1] + 1, mx[0] - mn[0] + 1)))
+
+    def _dims(self):
+        return self._vol["con"].shape[::-1]                                             # x, y, z
+
+    def _sources(self):
+        return [self._vol["con"], self._vol["conHalfPixel" if self.halfPixelOffset else "con"]]
+
+    def _host_volume(self, key):
+        if key not in self._host:
+            self._host[key] = self._vol[key].download()
+        return self._host[key]
+
+    @property
+    def con(self):
+        return self._host_volume("con")
+
+    @property
+    def conHalfPixel(self):
+        return self._host_volume("conHalfPixel")
 
     def getInterval(self, tile):
         """(:214-233) -> (min_xyz, max_xyz), inclusive.  Tile 1 starts at dimension(0)/2 - overlap in EVERY dimension, as written."""
-        dims = self.con.shape[::-1]
+        dims = self._dims()
         mn, mx = [0, 0, 0], [d - 1 for d in dims]
         if tile == 0:
             mx = [dims[d] // 2 + self.overlap[d] for d in range(3)]
@@ -226,26 +273,13 @@ class SimulateTileStitching:
             mn = [dims[0] // 2 - self.overlap[d] for d in range(3)]
         return mn, mx
 
-    def _cut(self, vol, tile):
-        mn, mx = self.getInterval(tile)
-        return np.ascontiguousarray(vol[mn[2]:mx[2] + 1, mn[1]:mx[1] + 1, mn[0]:mx[0] + 1])   # Views.zeroMin(Views.interval(...))
-
     def getNextPair(self, snr):
-        """(:131-189): two tiles, each sampled by its own thread / context with its own seed."""
+        """(:131-189): two tiles, each with its own seed and Philox stream, sampled from Views.zeroMin(Views.interval(...)) of the
+        resident volumes without a dense copy; the results equal extractSlices of the numpy cuts, bit for bit."""
         seeds = [self.rnd.nextInt(), self.rnd.nextInt()]
-        src = [self.con, self.conHalfPixel if self.halfPixelOffset else self.con]
-        out = [None, None]
-
-        def task(i):
-            ctx = Context(self.device)
-            out[i] = S.extractSlices(self._cut(src[i], i), self.lightsheetSpacing, snr, rnd=JavaRandom(seeds[i]), ctx=ctx, stream=i)
-            ctx.close()
-        threads = [threading.Thread(target=task, args=(i,)) for i in range(2)]
-        for t in threads:
-            t.start()
-        for t in threads:
-            t.join()
-        return out[0], out[1]
+        for i, vol in enumerate(self._sources()):       # asynchronous on the volumes' contexts: the two samplers may overlap
+            vol.extractSlices(self.lightsheetSpacing, snr, rnd=JavaRandom(seeds[i]), stream=i, interval=self.getInterval(i), out=self._tiles[i])
+        return self._tiles[0].download(), self._tiles[1].download()
 
     def getCorrectTranslation(self):
         """(:191-212)"""
@@ -256,6 +290,14 @@ class SimulateTileStitching:
             t[1] -= 0.5
         t[2] /= self.lightsheetSpacing
         return t
+
+    def close(self):
+        """Frees the resident volumes and the two contexts (downloaded `con` / `conHalfPixel` arrays stay valid)."""
+        for v in self._tiles + list(self._vol.values()):
+            v.free()
+        for ctx in self._ctx.values():
+            ctx.close()
+        self._tiles, self._vol, self._ctx = [], {}, {}
 
 
 def _cli():
