@@ -51,6 +51,11 @@ constexpr int x_rows_per_block(int a, int b, bool inverse) { return x_rows_for(i
     MVSIM_FFT_SIZES_SMALL(X) MVSIM_FFT_SIZES_G1(X) MVSIM_FFT_SIZES_G2(X) MVSIM_FFT_SIZES_G3(X) MVSIM_FFT_SIZES_G4(X)
 #endif
 
+// the decimated and polyphase fused z kernels are built only for z lines of these lengths (build time, fft_group.cu): covers the
+// BASELINE configs (339 -> 360 with inc 3, 639 -> 640 with inc 5).  Here rather than in fft_launch.h so that the CPU emulation
+// (tests/emu) enumerates the same instantiations.
+constexpr int kDecMinLine = 300, kDecMaxLine = 660;
+
 // compile-time lookup in the FULL table (also under MVSIM_EMU_SMALL_ONLY): {0, 0, 0} when n is not a supported size
 constexpr FftSize fft_size_lookup(int n)
 {

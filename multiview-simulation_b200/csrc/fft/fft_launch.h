@@ -11,9 +11,6 @@ enum FftKind { FFT_XFWD = 0, FFT_XINV = 1, FFT_SFWD = 2, FFT_SINV = 3, FFT_ZFUSE
                FFT_ZFUSED_DEC3 = 6, FFT_ZFUSED_DEC5 = 7,     // decimated inverse (ZFusedDec): the planner's (a, b) with 3 | a resp. 5 | a
                FFT_ZFUSED_POLY3 = 8, FFT_ZFUSED_POLY5 = 9 }; // polyphase form (ZFusedPoly): 3 resp. 5 phases of n / inc points
 
-// the decimated fused z kernels are built only for z lines of these lengths (build time): covers the BASELINE
-// configs (339 -> 360 with inc 3, 639 -> 640 with inc 5)
-constexpr int kDecMinLine = 300, kDecMaxLine = 660;
 // Lanes (T) = neighbouring kx columns a CTA of the strided passes owns: 8 complex = 64-byte segments.
 // (T = 4 with 4 CTAs/SM was measured on B200 and gave the same throughput; only T = 8 is built.)
 int strided_lanes();

@@ -1,8 +1,11 @@
 // CPU emulation of the CUDA line-FFT kernels: runs the very same __host__ __device__ phase
 // functions (multiview-simulation_b200/csrc/fft/line_fft.cuh) thread by thread, block by block,
 // with a barrier between phases, driven by the same host logic (conv_driver.h).  Built with g++
-// by tests/test_emu_conv.py; this is a test of the index arithmetic, not a product path.
+// by tests/test_emu_conv.py (the small size table) and tests/test_emu_fft_sizes.py (-DMVSIM_EMU_FULL_TABLE: every
+// line length the library ships); this is a test of the index arithmetic, not a product path.
+#ifndef MVSIM_EMU_FULL_TABLE
 #define MVSIM_EMU_SMALL_ONLY 1
+#endif
 #define MVSIM_PACKED_FFT 1
 #include "fft/conv_driver.h"
 
@@ -141,8 +144,18 @@ struct EmuLauncher {
 
 int EmuLauncher::decimated_launches = 0;
 extern "C" int emu_decimated_launches() { return EmuLauncher::decimated_launches; }
-// which (line length, inc) pairs the polyphase fused z kernel is built for, and how many PSF taps its border groups take
-extern "C" int emu_poly_ok(int n, int inc) { return (n % inc == 0 && fft_size_lookup(n).n == n && zfused_poly_ok(n, inc)) ? zfused_poly_max_taps(n, inc) : 0; }
+// which (line length, inc) pairs the polyphase fused z kernel is built for (fft_group.cu), and how many PSF taps its border groups take
+extern "C" int emu_poly_ok(int n, int inc)
+{
+    const bool built = n >= kDecMinLine && n <= kDecMaxLine && fft_size_lookup(n).n == n;
+    return (built && n % inc == 0 && zfused_poly_ok(n, inc)) ? zfused_poly_max_taps(n, inc) : 0;
+}
+// which (line length, inc) pairs the decimated fused z kernel is built for (fft_group.cu: ZFusedDec<b, a, T, inc> of the split n = a * b)
+extern "C" int emu_dec_ok(int n, int inc)
+{
+    const FftSize s = fft_size_lookup(n);
+    return (n >= kDecMinLine && n <= kDecMaxLine && s.n == n && zfused_dec_ok(s.a, s.b, inc)) ? 1 : 0;
+}
 int EmuLauncher::polyphase_launches = 0;
 extern "C" int emu_polyphase_launches() { return EmuLauncher::polyphase_launches; }
 
@@ -281,4 +294,76 @@ extern "C" double emu_check_pruned_ffts()
     MVSIM_CHK(16) MVSIM_CHK(18) MVSIM_CHK(20) MVSIM_CHK(24) MVSIM_CHK(25) MVSIM_CHK(27) MVSIM_CHK(30) MVSIM_CHK(32) MVSIM_CHK(36) MVSIM_CHK(40)
 #undef MVSIM_CHK
     return e;
+}
+
+// One generated sub-transform on the caller's input (2n floats, interleaved re / im), for the float64 DFT comparison of
+// tests/test_emu_fft_sizes.py.  family 0: RegFFT<n, dir> (scalar), 1: RegFFTP<n, dir> (packed), 2: RegFFTPZ<n> (forward transform
+// of x[0..K), x[K..n) is not read; dir ignored), 3: RegFFTPD<n, dir, r> (inverse of which only o[j] = X[r + dir * j] is computed,
+// into out[0..n / dir)).  Returns 0, or -1 when that variant is not generated.
+template <int N, int INC, int R> static int regfft_dec(const float2 (&x)[N], float* out)
+{
+    if constexpr (N % INC == 0 && N / INC >= 2 && R < INC) {
+        float2 o[N / INC];
+        RegFFTPD<N, INC, R>::run(x, o);
+        for (int j = 0; j < N / INC; ++j) { out[2 * j] = o[j].x; out[2 * j + 1] = o[j].y; }
+        return 0;
+    } else {
+        return -1;
+    }
+}
+
+template <int N> static int regfft_one(int family, int dir, int r, const float* in, float* out)
+{
+    float2 x[N];
+    for (int i = 0; i < N; ++i) x[i] = make_float2(in[2 * i], in[2 * i + 1]);
+    if (family == 3) {
+        if (dir == 3) {
+            switch (r) {
+            case 0: return regfft_dec<N, 3, 0>(x, out);
+            case 1: return regfft_dec<N, 3, 1>(x, out);
+            case 2: return regfft_dec<N, 3, 2>(x, out);
+            }
+        } else if (dir == 5) {
+            switch (r) {
+            case 0: return regfft_dec<N, 5, 0>(x, out);
+            case 1: return regfft_dec<N, 5, 1>(x, out);
+            case 2: return regfft_dec<N, 5, 2>(x, out);
+            case 3: return regfft_dec<N, 5, 3>(x, out);
+            case 4: return regfft_dec<N, 5, 4>(x, out);
+            }
+        }
+        return -1;
+    }
+    if (family == 2) RegFFTPZ<N>::run(x);
+    else if (family == 0 && dir == -1) RegFFT<N, -1>::run(x);
+    else if (family == 0 && dir == 1) RegFFT<N, 1>::run(x);
+    else if (family == 1 && dir == -1) RegFFTP<N, -1>::run(x);
+    else if (family == 1 && dir == 1) RegFFTP<N, 1>::run(x);
+    else return -1;
+    for (int i = 0; i < N; ++i) { out[2 * i] = x[i].x; out[2 * i + 1] = x[i].y; }
+    return 0;
+}
+
+// the generated sub-transform sizes: SIZES of tools/gen_regfft.py (a size added there fails the DFT test until it is listed here)
+#define MVSIM_REGFFT_SIZES(X) X(2) X(3) X(4) X(5) X(6) X(8) X(9) X(10) X(12) X(15) X(16) X(18) X(20) X(24) X(25) X(27) X(30) X(32) X(36) X(40)
+
+extern "C" int emu_regfft(int family, int n, int dir, int r, const float* in, float* out)
+{
+    switch (n) {
+#define MVSIM_X(n_) case n_: return regfft_one<n_>(family, dir, r, in, out);
+        MVSIM_REGFFT_SIZES(MVSIM_X)
+#undef MVSIM_X
+    }
+    return -1;
+}
+
+// K of RegFFTPZ<n>: the leading inputs the pruned forward transform reads (-1: no such size)
+extern "C" int emu_regfft_pz_k(int n)
+{
+    switch (n) {
+#define MVSIM_X(n_) case n_: return RegFFTPZ<n_>::K;
+        MVSIM_REGFFT_SIZES(MVSIM_X)
+#undef MVSIM_X
+    }
+    return -1;
 }

@@ -8,27 +8,17 @@ import subprocess
 import numpy as np
 import pytest
 
+import fft_cases
 from helpers import rel_err
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-SO = os.path.join(HERE, "emu", "libemu_conv.so")
-SRC = os.path.join(HERE, "emu", "emu_conv.cpp")
 CSRC = os.path.join(ROOT, "multiview-simulation_b200", "csrc")
 
 
 @pytest.fixture(scope="module")
 def emu():
-    deps = [SRC] + [os.path.join(CSRC, "fft", f) for f in os.listdir(os.path.join(CSRC, "fft"))]
-    if not os.path.exists(SO) or os.path.getmtime(SO) < max(os.path.getmtime(d) for d in deps):
-        # -fno-gnu-unique / -Bsymbolic: the emulator is built with the small size table; its inline statics must not become
-        # process-wide unique symbols that libmvsim.so (loaded later in the same pytest process) would bind to
-        subprocess.check_call(["g++", "-O1", "-std=c++17", "-shared", "-fPIC", "-fno-gnu-unique", "-Wl,-Bsymbolic", "-I", CSRC, SRC, "-o", SO])
-    L = C.CDLL(SO)
-    i64p, fp = C.POINTER(C.c_int64), C.POINTER(C.c_float)
-    L.emu_convolve.argtypes = [fp, i64p, fp, i64p, fp, C.POINTER(C.c_double), C.c_int, C.c_int, C.c_int, C.c_int]
-    L.emu_plan.argtypes = [i64p, i64p, C.POINTER(C.c_int), C.c_int]
-    return L
+    return fft_cases.build_emu(full=False)
 
 
 @pytest.fixture(autouse=True, params=["materialised-H", "on-the-fly"])

@@ -155,7 +155,7 @@ def test_view_loop_on_resident_and_wrapped_ground_truth(mv):
     ((330, 48, 40), (31, 9, 7), 3, 3),       # z line 360: polyphase (3 x 120), decimated inverse (18 | 3) and full spectral kernel
     ((330, 40, 24), (31, 7, 5), 5, 2),       # 360 at inc 5: polyphase (5 x 72); no decimated kernel for this split -> full spectral
     ((512, 32, 24), (128, 9, 5), 5, 3),      # BASELINE config 3's z line: 640 = 5 x 128
-    # the other line lengths the polyphase kernel is built for (one instantiation each)
+    # other line lengths the polyphase kernel is built for
     ((300, 24, 16), (25, 5, 3), 3, 3),       # 324 = 3 x 108 (9 x 12), 36 groups
     ((360, 24, 16), (25, 5, 3), 3, 2),       # 384 = 3 x 128 (8 x 16), 24 groups, two rounds of level-1 items; no decimated kernel (3 does not divide 16)
     ((380, 24, 16), (21, 5, 3), 5, 3),       # 400 = 5 x 80 (8 x 10), 40 groups, two rounds
@@ -164,7 +164,8 @@ def test_view_loop_on_resident_and_wrapped_ground_truth(mv):
 ])
 def test_fused_z_kernel_variants_agree(mv, shape, kshape, inc, distinct):
     """MVSIM_OPT_Z_KERNEL: the polyphase, decimated-inverse and full spectral fused z kernels compute the same view (kept planes AND,
-    through adjustImage's mean, the sum of the dropped planes) to float32 rounding -- and are really different kernels."""
+    through adjustImage's mean, the sum of the dropped planes) to float32 rounding -- and are really different kernels.  Every built
+    instantiation against the direct-sum oracle: tests/test_gpu_fft_sizes.py::test_every_built_whole_view_kernel."""
     S = mv.SimulateMultiViewDataset
     rng = np.random.default_rng(31)
     gt = rng.random(shape, dtype=np.float32)
