@@ -179,23 +179,26 @@ struct DevBuf {
     float* f() { return static_cast<float*>(p); }
 };
 
-struct Activate {
-    int prev; bool ok;
-    explicit Activate(mvsim_ctx* ctx) : prev(-1), ok(false)
+// device buffers of one call with a deferred failure: after the first failed allocation alloc() returns null and st keeps that
+// status, so a call allocates all it needs and checks once
+struct DevBufs {
+    mvsim_ctx* ctx;
+    int st = MVSIM_OK;
+    std::vector<void*> held;
+    explicit DevBufs(mvsim_ctx* c) : ctx(c) {}
+    ~DevBufs() { free_all(); }
+    template <class T> T* alloc(size_t n)
     {
-        if (cudaGetDevice(&prev) != cudaSuccess) return;
-        ok = cudaSetDevice(ctx->device) == cudaSuccess;
-        // drop a stale, non-sticky error an earlier call of this host thread left behind (ours or the caller's): the launch
-        // checks of this entry point read cudaGetLastError() and must report their own failures only
-        if (ok) cudaGetLastError();
+        void* q = nullptr;
+        if (st == MVSIM_OK && (st = dev_alloc(ctx, &q, n * sizeof(T))) == MVSIM_OK) held.push_back(q);
+        return static_cast<T*>(q);
     }
-    ~Activate() { if (prev >= 0) cudaSetDevice(prev); }
+    void free_all() { for (void* q : held) dev_free(ctx, q); held.clear(); }
 };
 
-#define MVSIM_ENTER(ctx)                                                                     \
-    if (!(ctx)) return mvsim::set_error(nullptr, MVSIM_EINVAL, "null context");             \
-    mvsim::Activate act__(ctx);                                                              \
-    if (!act__.ok) return mvsim::set_error((ctx), MVSIM_ECUDA, "cannot select CUDA device %d", (ctx)->device)
+// planes z = 0, inc, 2 inc, ... that the sampler keeps of a view of dims, and the voxels they hold
+static int64_t kept_planes(const int64_t dims[3], int inc) { return (dims[2] - 1) / inc + 1; }
+static size_t kept_elems(const int64_t dims[3], int inc) { return (size_t)(dims[0] * dims[1] * kept_planes(dims, inc)); }
 
 // ---- host side of the uint16 count transport ------------------------------------------------------------------------
 // uint16 -> float32, streaming stores (the destination is written once and not read back by these threads)
@@ -395,11 +398,124 @@ static int dev_simulate_view(mvsim_ctx* ctx, const mvsim_view_params* p, const f
     StageTimer t(ctx, MVSIM_T_SAMPLE);                                                         // :585
     if (planes != p->dims[2]) {
         // the convolution already delivered the kept slices compacted (plus the sum plane, unused here)
-        const int64_t kept[3] = { p->dims[0], p->dims[1], (p->dims[2] - 1) / p->inc + 1 };
+        const int64_t kept[3] = { p->dims[0], p->dims[1], kept_planes(p->dims, p->inc) };
         return k_extract_u16(ctx, a.f(), kept, 1, ctx->d_scalars + 2, p->min_value, p->snr, p->seed, p->stream, out, out16, d_overflow);
     }
     return k_extract_u16(ctx, a.f(), p->dims, p->inc, ctx->d_scalars + 2, p->min_value, p->snr, p->seed, p->stream, out, out16, d_overflow);
 }
+
+// every view of a batch valid, all of them on the dims of the one ground truth (and of its resident volume, if there is one)
+static int check_views(mvsim_ctx* ctx, int n, const mvsim_view_params* params, const mvsim_volume* vol, const char* what)
+{
+    for (int v = 0; v < n; ++v) {
+        MVSIM_TRY(check_view(ctx, &params[v]));
+        for (int d = 0; d < 3; ++d)
+            if (params[v].dims[d] != params[0].dims[d] || (vol && vol->dims[d] != params[0].dims[d]))
+                return set_error(ctx, MVSIM_EINVAL, "%s: all views share the ground truth dims", what);
+    }
+    return MVSIM_OK;
+}
+
+// Per-device phase gates of the batch calls: callers that run contexts concurrently on one GPU (the reference's tile
+// stitching driver does, S/SimulateTileStitching.java:85-117) fall into a pipeline -- one uploads while the other computes.
+struct DeviceGates { std::mutex upload, compute; };
+static DeviceGates& gates_for(int device)
+{
+    static DeviceGates gates[64];
+    return gates[(unsigned)device % 64];
+}
+
+// The protocol of the batch calls (DESIGN section 9): buffers and events first, then upload(), compute() and finish().  A
+// failure is deferred: st keeps the first one, the later phases are skipped, and finish() still drains and frees, and returns it.
+class BatchCall : public DevBufs {
+public:
+    BatchCall(mvsim_ctx* c, const char* what) : DevBufs(c), what_(what), gates_(gates_for(c->device))
+    {
+        stamp("enter");
+        cudaError_t e = cudaSuccess;
+        if (!ctx->copy_stream && (e = cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking)) != cudaSuccess) {
+            ctx->copy_stream = nullptr;
+            st = cuda_fail(ctx, e, "cudaStreamCreateWithFlags");
+        }
+        mark_ = event();
+    }
+    ~BatchCall() { for (cudaEvent_t e : events_) cudaEventDestroy(e); }
+
+    // an event of this call, destroyed with it; null after a failure
+    cudaEvent_t event()
+    {
+        cudaEvent_t e = nullptr;
+        if (st == MVSIM_OK && cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess)
+            st = set_error(ctx, MVSIM_ECUDA, "%s: cannot create events", what_);
+        if (st != MVSIM_OK) return nullptr;
+        events_.push_back(e);
+        return e;
+    }
+
+    // the ground truth on the device: the resident volume, or a buffer that upload() fills from `host` before anything else
+    const float* ground_truth(const float* host, const mvsim_volume* vol, size_t n)
+    {
+        if (vol) return vol->d;
+        gt_host_ = host; gt_bytes_ = n * sizeof(float);
+        return gt_dev_ = alloc<float>(n);
+    }
+
+    // Upload gate: two contexts never share the host->device link, so the second caller's upload runs at full rate under the
+    // first caller's kernels instead of both uploads at half rate followed by both kernel phases.  ALL of a call's uploads
+    // happen here (enqueue() issues those after the ground truth): a PSF upload issued later would queue on the copy engine
+    // behind the other caller's 2 GB ground truth and stall this context's kernels for the length of that transfer.
+    template <class Enqueue> void upload(Enqueue enqueue)
+    {
+        if (st != MVSIM_OK) return;
+        {
+            std::lock_guard<std::mutex> lk(gates_.upload);
+            stamp("upload gate");
+            if (gt_host_) st = h2d(ctx, gt_dev_, gt_host_, gt_bytes_);
+            if (st == MVSIM_OK) st = enqueue();
+            if (st == MVSIM_OK && (cudaEventRecord(mark_, ctx->stream) != cudaSuccess || cudaEventSynchronize(mark_) != cudaSuccess))
+                st = set_error(ctx, MVSIM_ECUDA, "%s: upload failed", what_);
+        }
+        if (st == MVSIM_OK) stamp("upload done");
+    }
+
+    // Compute gate: body(&last) enqueues the kernels and downloads and names the event recorded after the last kernel.  The
+    // gate opens when that event has completed; the tail of the downloads overlaps the next caller's kernels.
+    template <class Body> void compute(Body body)
+    {
+        if (st != MVSIM_OK) return;
+        std::lock_guard<std::mutex> lk(gates_.compute);
+        stamp("compute gate");
+        cudaEvent_t last = nullptr;
+        st = body(&last);
+        if (st == MVSIM_OK && last && cudaEventSynchronize(last) != cudaSuccess) st = set_error(ctx, MVSIM_ECUDA, "%s: kernels failed", what_);
+        stamp("kernels done");
+    }
+
+    int finish()
+    {
+        // the main stream waits for the copy stream before the buffers go back to the pool
+        if (mark_ && cudaEventRecord(mark_, ctx->copy_stream) == cudaSuccess) cudaStreamWaitEvent(ctx->stream, mark_, 0);
+        free_all();
+        const int st2 = sync(ctx);
+        stamp("downloads done");
+        return st != MVSIM_OK ? st : st2;
+    }
+
+    void stamp(const char* what) const
+    {
+        static const bool trace = getenv("MVSIM_TRACE") != nullptr;
+        if (trace) fprintf(stderr, "[mvsim %p] %10.3f ms %s\n", (void*)ctx, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(), what);
+    }
+
+private:
+    const char* what_;
+    DeviceGates& gates_;
+    std::vector<cudaEvent_t> events_;
+    cudaEvent_t mark_ = nullptr;            // end of the uploads, then end of the copy stream's work
+    const float* gt_host_ = nullptr;
+    float* gt_dev_ = nullptr;
+    size_t gt_bytes_ = 0;
+};
 
 }  // namespace mvsim
 
@@ -427,6 +543,8 @@ static int ctx_create(int device, bool own, void* cuda_stream, mvsim_ctx** out)
         return set_error(nullptr, MVSIM_ECUDA, "no CUDA device available (%s); libmvsim has no CPU fallback",
                          e == cudaSuccess ? "device count 0" : cudaGetErrorString(e));
     if (device < 0 || device >= n) return set_error(nullptr, MVSIM_EINVAL, "device %d out of range [0,%d)", device, n);
+    DeviceScope scope(device);
+    if (!scope.ok) return set_error(nullptr, MVSIM_ECUDA, "cannot select CUDA device %d", device);
     mvsim_ctx* ctx = new mvsim_ctx();
     ctx->device = device;
     ctx->stream = nullptr;
@@ -451,11 +569,8 @@ static int ctx_create(int device, bool own, void* cuda_stream, mvsim_ctx** out)
     ctx->profiling = false;
     memset(ctx->acc_ms, 0, sizeof(ctx->acc_ms));
     memset(ctx->acc_n, 0, sizeof(ctx->acc_n));
-    int prev = -1;
-    cudaGetDevice(&prev);
     int st = MVSIM_OK;
     do {
-        if ((e = cudaSetDevice(device)) != cudaSuccess) { st = cuda_fail(nullptr, e, "cudaSetDevice"); break; }
         if (!own) ctx->stream = static_cast<cudaStream_t>(cuda_stream);     // NULL = the legacy default stream
         else {
             if ((e = cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking)) != cudaSuccess) { st = cuda_fail(nullptr, e, "cudaStreamCreate"); break; }
@@ -474,7 +589,6 @@ static int ctx_create(int device, bool own, void* cuda_stream, mvsim_ctx** out)
         uint64_t keep = ~0ull;
         cudaMemPoolSetAttribute(ctx->mempool, cudaMemPoolAttrReleaseThreshold, &keep);
     } while (0);
-    if (prev >= 0) cudaSetDevice(prev);
     if (st != MVSIM_OK) {
         if (ctx->mempool) cudaMemPoolDestroy(ctx->mempool);
         if (ctx->d_scalars) cudaFree(ctx->d_scalars);
@@ -492,7 +606,7 @@ int mvsim_ctx_create_on_stream(int device, void* cuda_stream, mvsim_ctx** out) {
 int mvsim_ctx_destroy(mvsim_ctx* ctx)
 {
     if (!ctx) return MVSIM_OK;
-    Activate act(ctx);
+    DeviceScope scope(ctx->device);
     cudaStreamSynchronize(ctx->stream);
     for (auto& kv : ctx->tables) cudaFree(kv.second.tw);
     for (auto& kv : ctx->dec_tables) cudaFree(kv.second);
@@ -729,7 +843,7 @@ int mvsim_extract_slices(mvsim_ctx* ctx, const float* in, const int64_t dims[3],
     MVSIM_TRY(check_dims(ctx, dims, "extract_slices"));
     if (inc < 1) return set_error(ctx, MVSIM_EINVAL, "extract_slices: inc must be >= 1");
     const size_t bytes = elems(dims) * sizeof(float);
-    const size_t obytes = (size_t)(dims[0] * dims[1] * ((dims[2] - 1) / inc + 1)) * sizeof(float);
+    const size_t obytes = kept_elems(dims, inc) * sizeof(float);
     DevBuf a(ctx), b(ctx);
     MVSIM_TRY(a.alloc(bytes));
     MVSIM_TRY(b.alloc(obytes));
@@ -764,7 +878,7 @@ int mvsim_simulate_view(mvsim_ctx* ctx, const mvsim_view_params* p, const float*
     MVSIM_TRY(check_view(ctx, p));
     if (!gt || !psf || !out) return set_error(ctx, MVSIM_EINVAL, "simulate_view: null buffer");
     const size_t bytes = elems(p->dims) * sizeof(float), kbytes = elems(p->kdims) * sizeof(float);
-    const size_t obytes = (size_t)(p->dims[0] * p->dims[1] * ((p->dims[2] - 1) / p->inc + 1)) * sizeof(float);
+    const size_t obytes = kept_elems(p->dims, p->inc) * sizeof(float);
     DevBuf g(ctx), k(ctx), o(ctx);
     MVSIM_TRY(g.alloc(bytes));
     MVSIM_TRY(k.alloc(kbytes));
@@ -777,79 +891,44 @@ int mvsim_simulate_view(mvsim_ctx* ctx, const mvsim_view_params* p, const float*
     return sync(ctx);
 }
 
-// Per-device phase gates of the batch call: callers that run contexts concurrently on one GPU (the reference's tile
-// stitching driver does, S/SimulateTileStitching.java:85-117) fall into a pipeline -- one uploads while the other computes.
-namespace {
-struct DeviceGates { std::mutex upload, compute; };
-DeviceGates& gates_for(int device)
-{
-    static DeviceGates gates[64];
-    return gates[(unsigned)device % 64];
-}
-}  // namespace
-
-// gt: host ground truth (uploaded under the upload gate) or, when d_gt is given, already resident on the device
-static int simulate_views_impl(mvsim_ctx* ctx, int n_views, const mvsim_view_params* params, const float* gt, const float* d_gt,
+// gt: host ground truth (uploaded under the upload gate) or, when vol is given, already resident on the device
+static int simulate_views_impl(mvsim_ctx* ctx, int n_views, const mvsim_view_params* params, const float* gt, const mvsim_volume* vol,
                                float* const* psfs, float* const* outs)
 {
-    if (n_views < 0 || (n_views > 0 && (!params || (!gt && !d_gt) || !psfs || !outs))) return set_error(ctx, MVSIM_EINVAL, "simulate_views: null argument");
+    if (n_views < 0 || (n_views > 0 && (!params || (!gt && !vol) || !psfs || !outs))) return set_error(ctx, MVSIM_EINVAL, "simulate_views: null argument");
     if (n_views == 0) return MVSIM_OK;
-    for (int v = 0; v < n_views; ++v) {
-        MVSIM_TRY(check_view(ctx, &params[v]));
+    MVSIM_TRY(check_views(ctx, n_views, params, vol, "simulate_views"));
+    for (int v = 0; v < n_views; ++v)
         if (!psfs[v] || !outs[v]) return set_error(ctx, MVSIM_EINVAL, "simulate_views: null buffer for view %d", v);
-        for (int d = 0; d < 3; ++d)
-            if (params[v].dims[d] != params[0].dims[d]) return set_error(ctx, MVSIM_EINVAL, "simulate_views: all views share the ground truth dims");
-    }
-    if (!ctx->copy_stream) MVSIM_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-    const size_t bytes = elems(params[0].dims) * sizeof(float);
-    DeviceGates& gates = gates_for(ctx->device);
-    static const bool trace = getenv("MVSIM_TRACE") != nullptr;
-    auto stamp = [&](const char* what) {
-        if (trace) fprintf(stderr, "[mvsim %p] %10.3f ms %s\n", (void*)ctx, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(), what);
-    };
-    stamp("enter");
-    cudaEvent_t done = nullptr, copied = nullptr;
-    if (cudaEventCreateWithFlags(&done, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&copied, cudaEventDisableTiming) != cudaSuccess) {
-        if (done) cudaEventDestroy(done);
-        return set_error(ctx, MVSIM_ECUDA, "simulate_views: cannot create events");
-    }
-    DevBuf g(ctx);
-    int st = d_gt ? MVSIM_OK : g.alloc(bytes);
-    const float* gt_dev = d_gt ? d_gt : g.f();
-    std::vector<void*> held;            // per-view device buffers (psf, out) stay alive until their download is done
-    for (int v = 0; v < n_views && st == MVSIM_OK; ++v) {
-        void *k = nullptr, *o = nullptr;
-        if ((st = dev_alloc(ctx, &k, elems(params[v].kdims) * sizeof(float))) != MVSIM_OK) break;
-        held.push_back(k);
-        const size_t obytes = (size_t)(params[v].dims[0] * params[v].dims[1] * ((params[v].dims[2] - 1) / params[v].inc + 1)) * sizeof(float);
-        if ((st = dev_alloc(ctx, &o, obytes)) != MVSIM_OK) break;
-        held.push_back(o);
+    BatchCall bc(ctx, "simulate_views");
+    const float* gt_dev = bc.ground_truth(gt, vol, elems(params[0].dims));
+    cudaEvent_t done = bc.event();
+    // every view's device PSF and output stay alive until its download is done
+    std::vector<float*> k((size_t)n_views), o((size_t)n_views);
+    for (int v = 0; v < n_views; ++v) {
+        k[(size_t)v] = bc.alloc<float>(elems(params[v].kdims));
+        o[(size_t)v] = bc.alloc<float>(kept_elems(params[v].dims, params[v].inc));
     }
     // Count transport (MVSIM_OPT_COUNT_TRANSPORT, views with Poisson noise): the sampler also writes the counts as uint16; those
     // cross the link into a pinned staging buffer and host threads widen them into the caller's float32 buffer while later views
     // still compute / copy.  A view whose counts exceed 65535 (flag) is fetched again as float32.
     struct U16View { unsigned short* d16; unsigned short* h16; int* d_flag; int* h_flag; cudaEvent_t copied; bool on; };
     std::vector<U16View> u16((size_t)n_views, U16View{ nullptr, nullptr, nullptr, nullptr, nullptr, false });
-    int* h_flags = nullptr;
-    if (st == MVSIM_OK && ctx->count_transport == 1) {
-        void* hf = nullptr;
-        st = staging_buffer(ctx, 0, (size_t)n_views * sizeof(int) + 64, &hf);
-        h_flags = static_cast<int*>(hf);
-        for (int v = 0; v < n_views && st == MVSIM_OK; ++v) {
+    if (bc.st == MVSIM_OK && ctx->count_transport == 1) {
+        void* h_flags = nullptr;
+        bc.st = staging_buffer(ctx, 0, (size_t)n_views * sizeof(int) + 64, &h_flags);
+        for (int v = 0; v < n_views && bc.st == MVSIM_OK; ++v) {
             if (!(params[v].snr >= 0.0f)) continue;
-            const size_t n_out = (size_t)(params[v].dims[0] * params[v].dims[1] * ((params[v].dims[2] - 1) / params[v].inc + 1));
-            void *d16 = nullptr, *dflag = nullptr, *h16 = nullptr;
-            if ((st = dev_alloc(ctx, &d16, n_out * sizeof(unsigned short))) != MVSIM_OK) break;
-            held.push_back(d16);
-            if ((st = dev_alloc(ctx, &dflag, 16)) != MVSIM_OK) break;
-            held.push_back(dflag);
-            if ((st = staging_buffer(ctx, (size_t)v + 1, n_out * sizeof(unsigned short), &h16)) != MVSIM_OK) break;
+            const size_t n_out = kept_elems(params[v].dims, params[v].inc);
             U16View& u = u16[(size_t)v];
-            u.d16 = static_cast<unsigned short*>(d16); u.h16 = static_cast<unsigned short*>(h16);
-            u.d_flag = static_cast<int*>(dflag); u.h_flag = h_flags + v;
-            if (cudaEventCreateWithFlags(&u.copied, cudaEventDisableTiming) != cudaSuccess) { st = set_error(ctx, MVSIM_ECUDA, "simulate_views: cannot create events"); break; }
-            u.on = true;
+            u.d16 = bc.alloc<unsigned short>(n_out);
+            u.d_flag = bc.alloc<int>(4);
+            void* h16 = nullptr;
+            if (bc.st == MVSIM_OK) bc.st = staging_buffer(ctx, (size_t)v + 1, n_out * sizeof(unsigned short), &h16);
+            u.h16 = static_cast<unsigned short*>(h16);
+            u.h_flag = static_cast<int*>(h_flags) + v;
+            u.copied = bc.event();
+            u.on = bc.st == MVSIM_OK;
         }
     }
     int next_u16 = 0;
@@ -857,11 +936,10 @@ static int simulate_views_impl(mvsim_ctx* ctx, int n_views, const mvsim_view_par
         U16View& u = u16[(size_t)v];
         if (!u.on) return MVSIM_OK;
         if (cudaEventSynchronize(u.copied) != cudaSuccess) return set_error(ctx, MVSIM_ECUDA, "simulate_views: download failed");
-        const mvsim_view_params* p = &params[v];
-        const size_t n_out = (size_t)(p->dims[0] * p->dims[1] * ((p->dims[2] - 1) / p->inc + 1));
+        const size_t n_out = kept_elems(params[v].dims, params[v].inc);
         if (*u.h_flag) {
             // counts beyond uint16: this view travels as float32 after all
-            cudaError_t e = cudaMemcpyAsync(outs[v], held[2 * v + 1], n_out * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
+            cudaError_t e = cudaMemcpyAsync(outs[v], o[(size_t)v], n_out * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
             if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->copy_stream);
             if (e != cudaSuccess) return cuda_fail(ctx, e, "simulate_views: float32 fallback download");
         } else {
@@ -874,70 +952,49 @@ static int simulate_views_impl(mvsim_ctx* ctx, int n_views, const mvsim_view_par
         }
         return MVSIM_OK;
     };
-    if (st == MVSIM_OK) {
-        // upload gate: two contexts never share the host->device link, so the second caller's upload runs at full rate
-        // under the first caller's kernels instead of both uploads at half rate followed by both kernel phases.  ALL of
-        // this call's uploads happen here: a PSF upload issued later would queue on the copy engine behind the other
-        // caller's 2 GB ground truth and stall this context's kernels for the length of that transfer.
-        std::lock_guard<std::mutex> lk(gates.upload);
-        stamp("upload gate");
-        if (!d_gt) st = h2d(ctx, g.p, gt, bytes);
-        for (int v = 0; v < n_views && st == MVSIM_OK; ++v) st = h2d(ctx, held[2 * v], psfs[v], elems(params[v].kdims) * sizeof(float));
-        if (st == MVSIM_OK && (cudaEventRecord(done, ctx->stream) != cudaSuccess || cudaEventSynchronize(done) != cudaSuccess))
-            st = set_error(ctx, MVSIM_ECUDA, "simulate_views: upload failed");
-    }
-    if (st == MVSIM_OK) {
-        stamp("upload done");
-        std::lock_guard<std::mutex> lk(gates.compute);
-        stamp("compute gate");
+    bc.upload([&]() -> int {
+        int st = MVSIM_OK;
+        for (int v = 0; v < n_views && st == MVSIM_OK; ++v) st = h2d(ctx, k[(size_t)v], psfs[v], elems(params[v].kdims) * sizeof(float));
+        return st;
+    });
+    bc.compute([&](cudaEvent_t* last) -> int {
+        int st = MVSIM_OK;
         for (int v = 0; v < n_views && st == MVSIM_OK; ++v) {
             const mvsim_view_params* p = &params[v];
-            const size_t kbytes = elems(p->kdims) * sizeof(float);
-            const size_t n_out = (size_t)(p->dims[0] * p->dims[1] * ((p->dims[2] - 1) / p->inc + 1));
-            void *k = held[2 * v], *o = held[2 * v + 1];
+            const size_t n_out = kept_elems(p->dims, p->inc);
             U16View& u = u16[(size_t)v];
             cudaError_t e = cudaSuccess;
             if (u.on) e = cudaMemsetAsync(u.d_flag, 0, sizeof(int), ctx->stream);
             if (e != cudaSuccess) { st = cuda_fail(ctx, e, "simulate_views: flag"); break; }
-            if ((st = dev_simulate_view(ctx, p, gt_dev, static_cast<float*>(k), static_cast<float*>(o), u.on ? u.d16 : nullptr, u.on ? u.d_flag : nullptr)) != MVSIM_OK) break;
+            if ((st = dev_simulate_view(ctx, p, gt_dev, k[(size_t)v], o[(size_t)v], u.on ? u.d16 : nullptr, u.on ? u.d_flag : nullptr)) != MVSIM_OK) break;
             e = cudaEventRecord(done, ctx->stream);
             if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->copy_stream, done, 0);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(psfs[v], k, kbytes, cudaMemcpyDeviceToHost, ctx->copy_stream);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(psfs[v], k[(size_t)v], elems(p->kdims) * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
             if (u.on) {
                 if (e == cudaSuccess) e = cudaMemcpyAsync(u.h_flag, u.d_flag, sizeof(int), cudaMemcpyDeviceToHost, ctx->copy_stream);
                 if (e == cudaSuccess) e = cudaMemcpyAsync(u.h16, u.d16, n_out * sizeof(unsigned short), cudaMemcpyDeviceToHost, ctx->copy_stream);
                 if (e == cudaSuccess) e = cudaEventRecord(u.copied, ctx->copy_stream);
             } else if (e == cudaSuccess) {
-                e = cudaMemcpyAsync(outs[v], o, n_out * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
+                e = cudaMemcpyAsync(outs[v], o[(size_t)v], n_out * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
             }
             if (e != cudaSuccess) st = cuda_fail(ctx, e, "simulate_views: download");
         }
-        stamp("enqueued");
+        bc.stamp("enqueued");
         // uint16 views: as each copy lands, widen it into the caller's buffer while the later views still compute / copy -- but
         // only until this call's last kernel has run: then the gate opens and the rest is finished outside it
         while (st == MVSIM_OK && next_u16 < n_views - 1 && cudaEventQuery(done) == cudaErrorNotReady) st = finish_u16(next_u16++);
         cudaGetLastError();     // cudaErrorNotReady from the query is not an error
-        // the gate opens when the last kernel has run; the tail of the downloads overlaps the next caller's kernels
-        if (st == MVSIM_OK && cudaEventSynchronize(done) != cudaSuccess) st = set_error(ctx, MVSIM_ECUDA, "simulate_views: kernels failed");
-        stamp("kernels done");
-    }
-    while (st == MVSIM_OK && next_u16 < n_views) st = finish_u16(next_u16++);
-    // the main stream waits for the copy stream before the buffers go back to the pool
-    if (cudaEventRecord(copied, ctx->copy_stream) == cudaSuccess) cudaStreamWaitEvent(ctx->stream, copied, 0);
-    for (void* q : held) dev_free(ctx, q);
-    const int st2 = sync(ctx);
-    stamp("downloads done");
-    for (auto& u : u16) if (u.copied) cudaEventDestroy(u.copied);
-    cudaEventDestroy(done);
-    cudaEventDestroy(copied);
-    return st != MVSIM_OK ? st : st2;
+        *last = done;
+        return st;
+    });
+    while (bc.st == MVSIM_OK && next_u16 < n_views) bc.st = finish_u16(next_u16++);
+    return bc.finish();
 }
 
 int mvsim_simulate_views(mvsim_ctx* ctx, int n_views, const mvsim_view_params* params, const float* gt,
                          float* const* psfs, float* const* outs)
 {
     MVSIM_ENTER(ctx);
-    if (n_views > 0 && !gt) return set_error(ctx, MVSIM_EINVAL, "simulate_views: null ground truth");
     return simulate_views_impl(ctx, n_views, params, gt, nullptr, psfs, outs);
 }
 
@@ -945,11 +1002,7 @@ int mvsim_dev_simulate_views(mvsim_ctx* ctx, int n_views, const mvsim_view_param
                              float* const* psfs, float* const* outs)
 {
     MVSIM_ENTER(ctx);
-    if (n_views > 0 && !gt) return set_error(ctx, MVSIM_EINVAL, "simulate_views: null ground truth");
-    if (n_views > 0 && params)
-        for (int d = 0; d < 3; ++d)
-            if (gt->dims[d] != params[0].dims[d]) return set_error(ctx, MVSIM_EINVAL, "simulate_views: ground truth volume dims differ from the view params");
-    return simulate_views_impl(ctx, n_views, params, nullptr, gt ? gt->d : nullptr, psfs, outs);
+    return simulate_views_impl(ctx, n_views, params, nullptr, gt, psfs, outs);
 }
 
 // ---- post-acquisition chain ---------------------------------------------------------------------
@@ -988,28 +1041,19 @@ int mvsim_normalize_weights(mvsim_ctx* ctx, float* const* weights, int n_views, 
     MVSIM_ENTER(ctx);
     if (!weights || n_views < 1 || n_views > MVSIM_MAX_WEIGHT_VIEWS) return set_error(ctx, MVSIM_EINVAL, "normalize_weights: 1..%d views", MVSIM_MAX_WEIGHT_VIEWS);
     MVSIM_TRY(check_dims(ctx, dims, "normalize_weights"));
+    for (int v = 0; v < n_views; ++v)
+        if (!weights[v]) return set_error(ctx, MVSIM_EINVAL, "normalize_weights: null buffer");
     const size_t n = elems(dims), bytes = n * sizeof(float);
-    std::vector<void*> held;
+    DevBufs bufs(ctx);
     float* d[MVSIM_MAX_WEIGHT_VIEWS] = {};
-    int st = MVSIM_OK;
-    for (int v = 0; v < n_views && st == MVSIM_OK; ++v) {
-        if (!weights[v]) { st = set_error(ctx, MVSIM_EINVAL, "normalize_weights: null buffer"); break; }
-        void* q = nullptr;
-        if ((st = dev_alloc(ctx, &q, bytes)) != MVSIM_OK) break;
-        held.push_back(q);
-        d[v] = static_cast<float*>(q);
-        st = h2d(ctx, q, weights[v], bytes);
-    }
-    float* dsum = nullptr;
-    if (st == MVSIM_OK && sum_out) {
-        void* q = nullptr;
-        if ((st = dev_alloc(ctx, &q, bytes)) == MVSIM_OK) { held.push_back(q); dsum = static_cast<float*>(q); }
-    }
+    for (int v = 0; v < n_views; ++v) d[v] = bufs.alloc<float>(n);
+    float* dsum = sum_out ? bufs.alloc<float>(n) : nullptr;
+    int st = bufs.st;
+    for (int v = 0; v < n_views && st == MVSIM_OK; ++v) st = h2d(ctx, d[v], weights[v], bytes);
     if (st == MVSIM_OK) st = k_normalize_weights(ctx, d, n_views, n, osem, dsum);
     for (int v = 0; v < n_views && st == MVSIM_OK; ++v) st = d2h(ctx, weights[v], d[v], bytes);
     if (st == MVSIM_OK && sum_out) st = d2h(ctx, sum_out, dsum, bytes);
     const int st2 = sync(ctx);
-    for (void* q : held) dev_free(ctx, q);
     return st != MVSIM_OK ? st : st2;
 }
 
@@ -1330,7 +1374,7 @@ int mvsim_dev_extract_slices(mvsim_ctx* ctx, const mvsim_volume* in, int inc, fl
 {
     MVSIM_ENTER(ctx);
     if (!in || !out || inc < 1) return set_error(ctx, MVSIM_EINVAL, "dev_extract_slices: bad argument");
-    if (out->dims[0] != in->dims[0] || out->dims[1] != in->dims[1] || out->dims[2] != (in->dims[2] - 1) / inc + 1)
+    if (out->dims[0] != in->dims[0] || out->dims[1] != in->dims[1] || out->dims[2] != kept_planes(in->dims, inc))
         return set_error(ctx, MVSIM_EINVAL, "dev_extract_slices: out dims must be (X, Y, (Z-1)/inc+1)");
     StageTimer t(ctx, MVSIM_T_SAMPLE);
     return k_extract(ctx, in->d, in->dims, inc, nullptr, 0.f, snr, seed, stream, out->d);
@@ -1357,7 +1401,7 @@ int mvsim_dev_simulate_view(mvsim_ctx* ctx, const mvsim_view_params* p, const mv
     if (!gt || !psf || !out) return set_error(ctx, MVSIM_EINVAL, "dev_simulate_view: null volume");
     for (int d = 0; d < 3; ++d)
         if (gt->dims[d] != p->dims[d] || psf->dims[d] != p->kdims[d]) return set_error(ctx, MVSIM_EINVAL, "dev_simulate_view: params do not match the volumes");
-    if (out->dims[0] != p->dims[0] || out->dims[1] != p->dims[1] || out->dims[2] != (p->dims[2] - 1) / p->inc + 1)
+    if (out->dims[0] != p->dims[0] || out->dims[1] != p->dims[1] || out->dims[2] != kept_planes(p->dims, p->inc))
         return set_error(ctx, MVSIM_EINVAL, "dev_simulate_view: out dims must be (X, Y, (Z-1)/inc+1)");
     return dev_simulate_view(ctx, p, gt->d, psf->d, out->d);
 }
@@ -1428,65 +1472,48 @@ int mvsim_dev_aligned_weights(mvsim_ctx* ctx, const int64_t dims[3], int n_all, 
 // aligned view, the view's own normalised weights and the rotated-back PSF, into one of TWO device output sets; the downloads of
 // view i run on the copy stream under the kernels of view i + 1, and view i + 2 waits for them before it reuses the set.
 static int simulate_dataset_impl(mvsim_ctx* ctx, int n_all, const mvsim_view_params* params, const int32_t* align_degrees, float osem,
-                                 int n_views, const int32_t* views, const float* gt, const float* d_gt, float* const* psfs,
+                                 int n_views, const int32_t* views, const float* gt, const mvsim_volume* vol, float* const* psfs,
                                  const mvsim_dataset_outputs* outs, float* sum_weights)
 {
     MVSIM_TRY(check_view_list(ctx, n_all, n_views, views, "simulate_dataset"));
     if (!params || !align_degrees) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: null params or angles");
-    for (int k = 0; k < n_all; ++k) {
-        MVSIM_TRY(check_view(ctx, &params[k]));
+    MVSIM_TRY(check_views(ctx, n_all, params, vol, "simulate_dataset"));
+    for (int k = 0; k < n_all; ++k)
         if (params[k].axis != 0) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: main() rotates about x only (axis 0)");
-        for (int d = 0; d < 3; ++d)
-            if (params[k].dims[d] != params[0].dims[d]) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: all views share the ground truth dims");
-    }
-    if (n_views > 0 && (!psfs || !outs || (!gt && !d_gt))) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: null argument");
+    if (n_views > 0 && (!psfs || !outs || (!gt && !vol))) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: null argument");
     for (int i = 0; i < n_views; ++i)
         if (!psfs[i]) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: null PSF for view %d", (int)views[i]);
     if (n_views == 0 && !sum_weights) return MVSIM_OK;
-    if (!ctx->copy_stream) MVSIM_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
     const int64_t* dims = params[0].dims;
     const size_t n = elems(dims);
     double inv_w[12 * MVSIM_MAX_WEIGHT_VIEWS];
     weight_inverses(dims, n_all, align_degrees, inv_w);
-    auto acq_elems = [&](const mvsim_view_params* p) { return (size_t)(p->dims[0] * p->dims[1] * ((p->dims[2] - 1) / p->inc + 1)); };
-    auto iso_elems = [&](const mvsim_view_params* p) { return (size_t)(p->dims[0] * p->dims[1] * (((p->dims[2] - 1) / p->inc) * p->inc + 1)); };
+    auto iso_elems = [&](const mvsim_view_params* p) { return (size_t)(p->dims[0] * p->dims[1] * ((kept_planes(p->dims, p->inc) - 1) * p->inc + 1)); };
     // sizes of a device output set: the largest of its views
     size_t acq_max = 0, iso_max = 0, k_max = 0;
     bool any_iso = false, any_kpsf = false, any_w = false;
     for (int i = 0; i < n_views; ++i) {
         const mvsim_view_params* p = &params[views[i]];
-        acq_max = std::max(acq_max, acq_elems(p));
+        acq_max = std::max(acq_max, kept_elems(p->dims, p->inc));
         iso_max = std::max(iso_max, iso_elems(p));
         k_max = std::max(k_max, elems(p->kdims));
         any_iso |= outs[i].aligned != nullptr;
         any_kpsf |= outs[i].aligned_psf != nullptr;
         any_w |= outs[i].weights != nullptr;
     }
-    DeviceGates& gates = gates_for(ctx->device);
-    cudaEvent_t done[2] = {}, freed[2] = {}, copied = nullptr;
-    int st = MVSIM_OK;
-    for (int s = 0; s < 2 && st == MVSIM_OK; ++s)
-        if (cudaEventCreateWithFlags(&done[s], cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&freed[s], cudaEventDisableTiming) != cudaSuccess)
-            st = set_error(ctx, MVSIM_ECUDA, "simulate_dataset: cannot create events");
-    if (st == MVSIM_OK && cudaEventCreateWithFlags(&copied, cudaEventDisableTiming) != cudaSuccess) st = set_error(ctx, MVSIM_ECUDA, "simulate_dataset: cannot create events");
-    std::vector<void*> held;
-    auto alloc = [&](size_t bytes) -> float* {
-        void* q = nullptr;
-        if (st == MVSIM_OK && (st = dev_alloc(ctx, &q, bytes)) == MVSIM_OK) held.push_back(q);
-        return static_cast<float*>(q);
-    };
-    float* g = d_gt || n_views == 0 ? nullptr : alloc(n * sizeof(float));
-    const float* gt_dev = d_gt ? d_gt : g;
+    BatchCall bc(ctx, "simulate_dataset");
+    const cudaEvent_t done[2] = { bc.event(), bc.event() }, freed[2] = { bc.event(), bc.event() };
+    const float* gt_dev = n_views > 0 ? bc.ground_truth(gt, vol, n) : nullptr;
     std::vector<float*> kpsf((size_t)n_views, nullptr);
-    for (int i = 0; i < n_views; ++i) kpsf[(size_t)i] = alloc(elems(params[views[i]].kdims) * sizeof(float));
+    for (int i = 0; i < n_views; ++i) kpsf[(size_t)i] = bc.alloc<float>(elems(params[views[i]].kdims));
     struct OutSet { float *acq, *iso, *kpsf, *w; } set[2] = {};
     for (int s = 0; s < 2 && s < n_views; ++s) {
-        set[s].acq = alloc(acq_max * sizeof(float));
-        if (any_iso) set[s].iso = alloc(iso_max * sizeof(float));
-        if (any_kpsf) set[s].kpsf = alloc(k_max * sizeof(float));
-        if (any_w) set[s].w = alloc(n * sizeof(float));
+        set[s].acq = bc.alloc<float>(acq_max);
+        if (any_iso) set[s].iso = bc.alloc<float>(iso_max);
+        if (any_kpsf) set[s].kpsf = bc.alloc<float>(k_max);
+        if (any_w) set[s].w = bc.alloc<float>(n);
     }
-    float* dsum = sum_weights ? alloc(n * sizeof(float)) : nullptr;
+    float* dsum = sum_weights ? bc.alloc<float>(n) : nullptr;
     // downloads of view i (psfs are normalised in place, :255)
     auto download = [&](int i) -> int {
         const int s = i % 2;
@@ -1494,23 +1521,21 @@ static int simulate_dataset_impl(mvsim_ctx* ctx, int n_all, const mvsim_view_par
         const mvsim_dataset_outputs& o = outs[i];
         cudaError_t e = cudaStreamWaitEvent(ctx->copy_stream, done[s], 0);
         if (e == cudaSuccess) e = cudaMemcpyAsync(psfs[i], kpsf[(size_t)i], elems(p->kdims) * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
-        if (e == cudaSuccess && o.acq) e = cudaMemcpyAsync(o.acq, set[s].acq, acq_elems(p) * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
+        if (e == cudaSuccess && o.acq) e = cudaMemcpyAsync(o.acq, set[s].acq, kept_elems(p->dims, p->inc) * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
         if (e == cudaSuccess && o.aligned) e = cudaMemcpyAsync(o.aligned, set[s].iso, iso_elems(p) * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
         if (e == cudaSuccess && o.aligned_psf) e = cudaMemcpyAsync(o.aligned_psf, set[s].kpsf, elems(p->kdims) * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
         if (e == cudaSuccess && o.weights) e = cudaMemcpyAsync(o.weights, set[s].w, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->copy_stream);
         if (e == cudaSuccess) e = cudaEventRecord(freed[s], ctx->copy_stream);
         return e == cudaSuccess ? MVSIM_OK : cuda_fail(ctx, e, "simulate_dataset: download");
     };
-    if (st == MVSIM_OK && n_views > 0) {
-        // all uploads under the upload gate, as in simulate_views_impl
-        std::lock_guard<std::mutex> lk(gates.upload);
-        if (!d_gt) st = h2d(ctx, g, gt, n * sizeof(float));
-        for (int i = 0; i < n_views && st == MVSIM_OK; ++i) st = h2d(ctx, kpsf[(size_t)i], psfs[i], elems(params[views[i]].kdims) * sizeof(float));
-        if (st == MVSIM_OK && (cudaEventRecord(done[0], ctx->stream) != cudaSuccess || cudaEventSynchronize(done[0]) != cudaSuccess))
-            st = set_error(ctx, MVSIM_ECUDA, "simulate_dataset: upload failed");
-    }
-    if (st == MVSIM_OK) {
-        std::lock_guard<std::mutex> lk(gates.compute);
+    if (n_views > 0)
+        bc.upload([&]() -> int {
+            int st = MVSIM_OK;
+            for (int i = 0; i < n_views && st == MVSIM_OK; ++i) st = h2d(ctx, kpsf[(size_t)i], psfs[i], elems(params[views[i]].kdims) * sizeof(float));
+            return st;
+        });
+    bc.compute([&](cudaEvent_t* last) -> int {
+        int st = MVSIM_OK;
         // the sum image depends on the dims and the angles alone (:648-663)
         if (dsum) st = k_aligned_weights(ctx, dims, n_all, inv_w, osem, 0, nullptr, nullptr, dsum);
         for (int i = 0; i < n_views && st == MVSIM_OK; ++i) {
@@ -1519,7 +1544,7 @@ static int simulate_dataset_impl(mvsim_ctx* ctx, int n_all, const mvsim_view_par
             const mvsim_dataset_outputs& o = outs[i];
             if (i >= 2 && cudaStreamWaitEvent(ctx->stream, freed[s], 0) != cudaSuccess) { st = set_error(ctx, MVSIM_ECUDA, "simulate_dataset: wait"); break; }
             if ((st = dev_simulate_view(ctx, p, gt_dev, kpsf[(size_t)i], set[s].acq)) != MVSIM_OK) break;                 // :570-585
-            const int64_t acq_dims[3] = { p->dims[0], p->dims[1], (p->dims[2] - 1) / p->inc + 1 };
+            const int64_t acq_dims[3] = { p->dims[0], p->dims[1], kept_planes(p->dims, p->inc) };
             if (o.aligned && (st = dev_align_view(ctx, set[s].acq, acq_dims, p->inc, align_degrees[v], set[s].iso)) != MVSIM_OK) break;   // :588, :591
             if (o.weights && (st = k_aligned_weights(ctx, dims, n_all, inv_w, osem, 1, &v, &set[s].w, nullptr)) != MVSIM_OK) break;      // :576, :592, :615-646
             if (o.aligned_psf && (st = dev_rotate(ctx, kpsf[(size_t)i], set[s].kpsf, p->kdims, 0, align_degrees[v])) != MVSIM_OK) break; // :593
@@ -1528,19 +1553,10 @@ static int simulate_dataset_impl(mvsim_ctx* ctx, int n_all, const mvsim_view_par
         }
         if (st == MVSIM_OK && n_views > 0) st = download(n_views - 1);
         if (st == MVSIM_OK && dsum) st = d2h(ctx, sum_weights, dsum, n * sizeof(float));
-        // the gate opens when this call's last kernel has run; the tail of the downloads overlaps the next caller's kernels
-        if (st == MVSIM_OK && n_views > 0 && cudaEventSynchronize(done[(n_views - 1) % 2]) != cudaSuccess) st = set_error(ctx, MVSIM_ECUDA, "simulate_dataset: kernels failed");
-    }
-    // the main stream waits for the copy stream before the buffers go back to the pool
-    if (copied && cudaEventRecord(copied, ctx->copy_stream) == cudaSuccess) cudaStreamWaitEvent(ctx->stream, copied, 0);
-    for (void* q : held) dev_free(ctx, q);
-    const int st2 = sync(ctx);
-    for (int s = 0; s < 2; ++s) {
-        if (done[s]) cudaEventDestroy(done[s]);
-        if (freed[s]) cudaEventDestroy(freed[s]);
-    }
-    if (copied) cudaEventDestroy(copied);
-    return st != MVSIM_OK ? st : st2;
+        *last = n_views > 0 ? done[(n_views - 1) % 2] : nullptr;
+        return st;
+    });
+    return bc.finish();
 }
 
 int mvsim_simulate_dataset(mvsim_ctx* ctx, int n_all, const mvsim_view_params* params, const int32_t* align_degrees, float osem,
@@ -1548,7 +1564,6 @@ int mvsim_simulate_dataset(mvsim_ctx* ctx, int n_all, const mvsim_view_params* p
                            float* sum_weights)
 {
     MVSIM_ENTER(ctx);
-    if (n_views > 0 && !gt) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: null ground truth");
     return simulate_dataset_impl(ctx, n_all, params, align_degrees, osem, n_views, views, gt, nullptr, psfs, outs, sum_weights);
 }
 
@@ -1557,11 +1572,7 @@ int mvsim_dev_simulate_dataset(mvsim_ctx* ctx, int n_all, const mvsim_view_param
                                const mvsim_dataset_outputs* outs, float* sum_weights)
 {
     MVSIM_ENTER(ctx);
-    if (n_views > 0 && !gt) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: null ground truth");
-    if (gt && params && n_all >= 1)
-        for (int d = 0; d < 3; ++d)
-            if (gt->dims[d] != params[0].dims[d]) return set_error(ctx, MVSIM_EINVAL, "simulate_dataset: ground truth volume dims differ from the view params");
-    return simulate_dataset_impl(ctx, n_all, params, align_degrees, osem, n_views, views, nullptr, gt ? gt->d : nullptr, psfs, outs, sum_weights);
+    return simulate_dataset_impl(ctx, n_all, params, align_degrees, osem, n_views, views, nullptr, gt, psfs, outs, sum_weights);
 }
 
 

@@ -357,14 +357,6 @@ int conv_device(mvsim_ctx* ctx, const float* img, const int64_t dims[3], const f
 // ---- slab-decomposed convolution of the largest single volume (SURVEY section 8e, BASELINE config 5) ----------------
 // One plan per rank.  The exchange buffers are owned by the caller (torch tensors in the Python
 // orchestrator, so torch.distributed / NCCL can run the two all-to-all transposes on them).
-namespace {
-struct DeviceGuard {
-    int prev;
-    explicit DeviceGuard(int dev) : prev(-1) { cudaGetDevice(&prev); cudaSetDevice(dev); }
-    ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
-}  // namespace
-
 struct mvsim_slabconv {
     mvsim::ConvPlan pl;
     mvsim::SlabGeom g;
@@ -389,6 +381,7 @@ int mvsim_slabconv_create(mvsim_ctx* ctx, const int64_t dims[3], const int64_t k
 {
     if (!ctx || !dims || !kdims || !out) return set_error(ctx, MVSIM_EINVAL, "slabconv_create: null argument");
     *out = nullptr;
+    MVSIM_ENTER(ctx);
     mvsim_slabconv* p = new mvsim_slabconv();
     p->lanes = strided_lanes();
     p->n_owned = 0;
@@ -408,9 +401,6 @@ int mvsim_slabconv_create(mvsim_ctx* ctx, const int64_t dims[3], const int64_t k
         p->owned[p->n_owned++] = q;
         *dst = static_cast<float2*>(q);
     };
-    int prev = -1;
-    cudaGetDevice(&prev);
-    cudaSetDevice(ctx->device);
     if ((st = get_tables(ctx, p->pl.sx.n, &tx)) == MVSIM_OK && (st = get_tables(ctx, p->pl.sy.n, &ty)) == MVSIM_OK &&
         (st = get_tables(ctx, p->pl.sz.n, &tz)) == MVSIM_OK) {
         p->ws = ConvWorkspace{};
@@ -422,7 +412,6 @@ int mvsim_slabconv_create(mvsim_ctx* ctx, const int64_t dims[3], const int64_t k
         grab(&p->ws.p2, (size_t)p->pl.p2_elems(p->lanes, p->g.tiles_own));
         p->ws.tw_x = tx.tw; p->ws.twist_x = tx.twist; p->ws.tw_y = ty.tw; p->ws.tw_z = tz.tw;
     }
-    if (prev >= 0) cudaSetDevice(prev);
     if (st != MVSIM_OK) {
         for (int i = 0; i < p->n_owned; ++i) cudaFree(p->owned[i]);
         delete p;
@@ -435,7 +424,7 @@ int mvsim_slabconv_create(mvsim_ctx* ctx, const int64_t dims[3], const int64_t k
 int mvsim_slabconv_destroy(mvsim_ctx* ctx, mvsim_slabconv* p)
 {
     if (!p) return MVSIM_OK;
-    DeviceGuard guard(ctx ? ctx->device : 0);
+    DeviceScope scope(ctx ? ctx->device : 0);
     if (ctx) cudaStreamSynchronize(ctx->stream);
     for (int i = 0; i < p->n_opened; ++i) cudaIpcCloseMemHandle(p->opened[i]);
     for (int i = 0; i < p->n_owned; ++i) cudaFree(p->owned[i]);
@@ -449,7 +438,7 @@ int mvsim_slabconv_p2p_alloc(mvsim_ctx* ctx, mvsim_slabconv* p, int nbuf, unsign
     if (!ctx || !p || !handles_out || nbuf < 1 || nbuf > 2) return set_error(ctx, MVSIM_EINVAL, "slabconv_p2p_alloc: bad argument");
     if (p->g.world > kMaxRanks) return set_error(ctx, MVSIM_EUNSUPPORTED, "slabconv_p2p: at most %d ranks", kMaxRanks);
     if (p->p2p_sets) return set_error(ctx, MVSIM_EINVAL, "slabconv_p2p_alloc: already allocated");
-    DeviceGuard guard(ctx->device);
+    MVSIM_ENTER(ctx);
     const size_t bytes = (size_t)p->pl.u2_elems(p->lanes, p->g.z_local) * sizeof(float2);
     for (int i = 0; i < nbuf; ++i)
         for (int k = 0; k < 2; ++k) {
@@ -469,7 +458,7 @@ int mvsim_slabconv_p2p_alloc(mvsim_ctx* ctx, mvsim_slabconv* p, int nbuf, unsign
 int mvsim_slabconv_p2p_open(mvsim_ctx* ctx, mvsim_slabconv* p, const unsigned char* all_handles)
 {
     if (!ctx || !p || !all_handles || !p->p2p_sets) return set_error(ctx, MVSIM_EINVAL, "slabconv_p2p_open: allocate first");
-    DeviceGuard guard(ctx->device);
+    MVSIM_ENTER(ctx);
     const int per_rank = p->p2p_sets * 2;
     for (int r = 0; r < p->g.world; ++r) {
         if (r == p->g.rank) continue;
@@ -518,11 +507,10 @@ int mvsim_slabconv_bind(mvsim_slabconv* p, void* send_buffer, void* recv_buffer)
     return MVSIM_OK;
 }
 
-// every entry point that launches kernels runs with the context's device current (the caller's current device may differ)
 #define MVSIM_SLAB_ENTER(ctx, p)                                                                   \
     if (!(ctx) || !(p)) return mvsim::set_error((ctx), MVSIM_EINVAL, "slabconv: null argument");   \
     if (!(p)->send) return mvsim::set_error((ctx), MVSIM_EINVAL, "slabconv: bind the exchange buffers first"); \
-    DeviceGuard guard__((ctx)->device)
+    MVSIM_ENTER(ctx)
 
 int mvsim_slabconv_prepare(mvsim_ctx* ctx, mvsim_slabconv* p, const float* d_psf, const float* d_img_slab)
 {

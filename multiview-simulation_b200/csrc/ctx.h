@@ -74,6 +74,27 @@ int cuda_fail(mvsim_ctx* ctx, cudaError_t e, const char* what);
         if (s__ != MVSIM_OK) return s__;   \
     } while (0)
 
+// Every exported function that touches a device runs inside one of these: it makes `device` current (ok tells whether that
+// worked) and gives the caller's current device back on exit.  It also drops a stale, non-sticky error an earlier call of this
+// host thread left behind (ours or the caller's): the launch checks of the entry point read cudaGetLastError() and must report
+// their own failures only.
+struct DeviceScope {
+    int prev = -1;
+    bool ok = false;
+    explicit DeviceScope(int device)
+    {
+        if (cudaGetDevice(&prev) != cudaSuccess) { prev = -1; return; }
+        ok = cudaSetDevice(device) == cudaSuccess;
+        if (ok) cudaGetLastError();
+    }
+    ~DeviceScope() { if (prev >= 0) cudaSetDevice(prev); }
+};
+
+#define MVSIM_ENTER(ctx)                                                                     \
+    if (!(ctx)) return mvsim::set_error(nullptr, MVSIM_EINVAL, "null context");             \
+    mvsim::DeviceScope scope__((ctx)->device);                                               \
+    if (!scope__.ok) return mvsim::set_error((ctx), MVSIM_ECUDA, "cannot select CUDA device %d", (ctx)->device)
+
 // RAII-less scoped stage timer: begin() before the launches of a stage, end() after.
 struct StageTimer {
     mvsim_ctx* ctx; int idx;
