@@ -170,30 +170,51 @@ static int sync(mvsim_ctx* ctx)
     return MVSIM_OK;
 }
 
-// scoped device buffer
-struct DevBuf {
-    mvsim_ctx* ctx; void* p;
-    explicit DevBuf(mvsim_ctx* c) : ctx(c), p(nullptr) {}
-    ~DevBuf() { dev_free(ctx, p); }
-    int alloc(size_t bytes) { return dev_alloc(ctx, &p, bytes); }
-    float* f() { return static_cast<float*>(p); }
-};
+// d_scalars[slot] -> *out, enqueued: valid after the next synchronisation of the stream
+static int fetch_scalar(mvsim_ctx* ctx, int slot, double* out)
+{
+    MVSIM_CUDA(ctx, cudaMemcpyAsync(out, ctx->d_scalars + slot, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    return MVSIM_OK;
+}
 
-// device buffers of one call with a deferred failure: after the first failed allocation alloc() returns null and st keeps that
-// status, so a call allocates all it needs and checks once
-struct DevBufs {
-    mvsim_ctx* ctx;
-    int st = MVSIM_OK;
-    std::vector<void*> held;
-    explicit DevBufs(mvsim_ctx* c) : ctx(c) {}
-    ~DevBufs() { free_all(); }
-    template <class T> T* alloc(size_t n)
+static int read_scalar(mvsim_ctx* ctx, int slot, double* out)
+{
+    MVSIM_TRY(fetch_scalar(ctx, slot, out));
+    return sync(ctx);
+}
+
+// The staging of a host-buffer entry point: in() / out() / inout() allocate a device buffer for n floats of a host buffer at
+// once; run(body) then uploads the in / inout buffers, runs body(), downloads the out / inout buffers and the scalar() slots,
+// and synchronises the stream once.  A failure skips the later steps (the synchronisation still runs) and run() returns it.
+class HostCall : public DevBufs {
+public:
+    explicit HostCall(mvsim_ctx* c) : DevBufs(c) {}
+    float* in(const float* host, size_t n) { return stage(const_cast<float*>(host), n, true, false); }
+    float* out(float* host, size_t n) { return stage(host, n, false, true); }
+    float* inout(float* host, size_t n) { return stage(host, n, true, true); }
+    void scalar(int slot, double* host) { if (host) scalars_.push_back({ slot, host }); }
+
+    template <class Body> int run(Body body)
     {
-        void* q = nullptr;
-        if (st == MVSIM_OK && (st = dev_alloc(ctx, &q, n * sizeof(T))) == MVSIM_OK) held.push_back(q);
-        return static_cast<T*>(q);
+        int s = st;
+        for (const Copy& c : copies_) if (s == MVSIM_OK && c.up) s = h2d(ctx, c.dev, c.host, c.bytes);
+        if (s == MVSIM_OK) s = body();
+        for (const Copy& c : copies_) if (s == MVSIM_OK && c.down) s = d2h(ctx, c.host, c.dev, c.bytes);
+        for (const auto& sc : scalars_) if (s == MVSIM_OK) s = fetch_scalar(ctx, sc.first, sc.second);
+        const int s2 = sync(ctx);
+        return s != MVSIM_OK ? s : s2;
     }
-    void free_all() { for (void* q : held) dev_free(ctx, q); held.clear(); }
+
+private:
+    struct Copy { float* dev; float* host; size_t bytes; bool up, down; };
+    float* stage(float* host, size_t n, bool up, bool down)
+    {
+        float* d = alloc<float>(n);
+        copies_.push_back({ d, host, n * sizeof(float), up, down });
+        return d;
+    }
+    std::vector<Copy> copies_;
+    std::vector<std::pair<int, double*>> scalars_;
 };
 
 // planes z = 0, inc, 2 inc, ... that the sampler keeps of a view of dims, and the voxels they hold
@@ -337,12 +358,6 @@ static int dev_psf_normalize(mvsim_ctx* ctx, float* psf, size_t n)
     return k_divide_by_sum(ctx, psf, n, ctx->d_scalars + 0);
 }
 
-static int read_scalar(mvsim_ctx* ctx, int slot, double* out)
-{
-    MVSIM_CUDA(ctx, cudaMemcpyAsync(out, ctx->d_scalars + slot, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    return sync(ctx);
-}
-
 static int dev_adjust(mvsim_ctx* ctx, float* img, size_t n, float min_value, float target_avg)
 {
     StageTimer t(ctx, MVSIM_T_ADJUST);
@@ -361,36 +376,55 @@ static int check_view(mvsim_ctx* ctx, const mvsim_view_params* p)
     return MVSIM_OK;
 }
 
+// dims and plane step of extractSlices and makeIsotropic
+static int check_sampling(mvsim_ctx* ctx, const int64_t dims[3], int inc, const char* what)
+{
+    MVSIM_TRY(check_dims(ctx, dims, what));
+    if (inc < 1) return set_error(ctx, MVSIM_EINVAL, "%s: inc must be >= 1", what);
+    return MVSIM_OK;
+}
+
+static int dev_extract_slices(mvsim_ctx* ctx, const float* in, const int64_t dims[3], int inc, float snr, uint64_t seed, uint64_t stream,
+                              float* out)
+{
+    StageTimer t(ctx, MVSIM_T_SAMPLE);
+    return k_extract(ctx, in, dims, inc, nullptr, 0.f, snr, seed, stream, out);
+}
+
+// rotate (axis: the caller's to check) and attenuate in one pass; MVSIM_EUNSUPPORTED, without an error text, when the rotation
+// is not the axis-0 fast path.  z_local > 0: only the output planes [z0, z0 + z_local) (out = that slab)
+static int dev_rotate_attenuate(mvsim_ctx* ctx, const float* in, float* out, const int64_t dims[3], int axis, int degrees, double delta,
+                                int strict, int64_t z0 = 0, int64_t z_local = 0)
+{
+    double inv[12];
+    int steps = 0;
+    axis_rotation(dims, axis, degrees, nullptr, inv);
+    MVSIM_TRY(attenuate_steps(ctx, dims, strict, &steps));
+    StageTimer t(ctx, MVSIM_T_ROTATE);
+    return k_rotate_attenuate(ctx, in, out, dims, axis, inv, delta, steps, z0, z_local);
+}
+
 // loop body S/SimulateMultiViewDataset.java:570-585 on device pointers
 static int dev_simulate_view(mvsim_ctx* ctx, const mvsim_view_params* p, const float* gt, float* psf, float* out,
                              unsigned short* out16 = nullptr, int* d_overflow = nullptr)
 {
     const size_t n = elems(p->dims);
-    DevBuf a(ctx), b(ctx);
-    MVSIM_TRY(a.alloc(n * sizeof(float)));
-    MVSIM_TRY(b.alloc(n * sizeof(float)));
-    {
-        // :570 + :573 in one pass (the rotated volume is not part of this entry point's output)
-        double inv[12];
-        int steps = 0;
-        if (axis_rotation(p->dims, p->axis, p->degrees, nullptr, inv)) return set_error(ctx, MVSIM_EINVAL, "simulate_view: bad axis");
-        MVSIM_TRY(attenuate_steps(ctx, p->dims, p->strict_reference, &steps));
-        int st;
-        {
-            StageTimer t(ctx, MVSIM_T_ROTATE);
-            st = k_rotate_attenuate(ctx, gt, b.f(), p->dims, p->axis, inv, p->delta, steps);
-        }
-        if (st == MVSIM_EUNSUPPORTED) {
-            MVSIM_TRY(dev_rotate(ctx, gt, a.f(), p->dims, p->axis, p->degrees));
-            MVSIM_TRY(dev_attenuate(ctx, a.f(), b.f(), p->dims, p->delta, p->strict_reference));
-        } else if (st != MVSIM_OK) return st;
-    }
+    DevBufs bufs(ctx);
+    float* a = bufs.alloc<float>(n);
+    float* b = bufs.alloc<float>(n);
+    MVSIM_TRY(bufs.st);
+    // :570 + :573 in one pass (the rotated volume is not part of this entry point's output)
+    const int st = dev_rotate_attenuate(ctx, gt, b, p->dims, p->axis, p->degrees, p->delta, p->strict_reference);
+    if (st == MVSIM_EUNSUPPORTED) {
+        MVSIM_TRY(dev_rotate(ctx, gt, a, p->dims, p->axis, p->degrees));
+        MVSIM_TRY(dev_attenuate(ctx, a, b, p->dims, p->delta, p->strict_reference));
+    } else if (st != MVSIM_OK) return st;
     // (Measured and dropped in round 2: the PSF chain -- normalise, x and y transforms, 0.26 ms -- on a side stream under
     // rotate_attenuate and the image's forward passes: 6.385 -> 6.345 ms per view with tools/time_view.py, but 6.2 -> 8.1 ms inside
     // bench.py's loop on a torch stream; the saturating main-stream kernels leave it nothing to hide behind.)
     MVSIM_TRY(dev_psf_normalize(ctx, psf, elems(p->kdims)));                                   // :255
     int planes = 0;
-    MVSIM_TRY(conv_device(ctx, b.f(), p->dims, psf, p->kdims, a.f(), ctx->d_scalars + 1, p->inc, &planes));   // :580
+    MVSIM_TRY(conv_device(ctx, b, p->dims, psf, p->kdims, a, ctx->d_scalars + 1, p->inc, &planes));   // :580
     {
         StageTimer t(ctx, MVSIM_T_ADJUST);                                                     // :582, applied inside the sampler
         MVSIM_TRY(k_adjust_corr(ctx, ctx->d_scalars + 1, n, p->min_value, p->target_avg, ctx->d_scalars + 2));
@@ -399,9 +433,9 @@ static int dev_simulate_view(mvsim_ctx* ctx, const mvsim_view_params* p, const f
     if (planes != p->dims[2]) {
         // the convolution already delivered the kept slices compacted (plus the sum plane, unused here)
         const int64_t kept[3] = { p->dims[0], p->dims[1], kept_planes(p->dims, p->inc) };
-        return k_extract_u16(ctx, a.f(), kept, 1, ctx->d_scalars + 2, p->min_value, p->snr, p->seed, p->stream, out, out16, d_overflow);
+        return k_extract_u16(ctx, a, kept, 1, ctx->d_scalars + 2, p->min_value, p->snr, p->seed, p->stream, out, out16, d_overflow);
     }
-    return k_extract_u16(ctx, a.f(), p->dims, p->inc, ctx->d_scalars + 2, p->min_value, p->snr, p->seed, p->stream, out, out16, d_overflow);
+    return k_extract_u16(ctx, a, p->dims, p->inc, ctx->d_scalars + 2, p->min_value, p->snr, p->seed, p->stream, out, out16, d_overflow);
 }
 
 // every view of a batch valid, all of them on the dims of the one ground truth (and of its resident volume, if there is one)
@@ -757,14 +791,10 @@ int mvsim_rotate_axis(mvsim_ctx* ctx, const float* in, float* out, const int64_t
     MVSIM_ENTER(ctx);
     if (!in || !out) return set_error(ctx, MVSIM_EINVAL, "rotate: null buffer");
     MVSIM_TRY(check_dims(ctx, dims, "rotate"));
-    const size_t bytes = elems(dims) * sizeof(float);
-    DevBuf a(ctx), b(ctx);
-    MVSIM_TRY(a.alloc(bytes));
-    MVSIM_TRY(b.alloc(bytes));
-    MVSIM_TRY(h2d(ctx, a.p, in, bytes));
-    MVSIM_TRY(dev_rotate(ctx, a.f(), b.f(), dims, axis, degrees));
-    MVSIM_TRY(d2h(ctx, out, b.p, bytes));
-    return sync(ctx);
+    HostCall hc(ctx);
+    const float* a = hc.in(in, elems(dims));
+    float* b = hc.out(out, elems(dims));
+    return hc.run([&] { return dev_rotate(ctx, a, b, dims, axis, degrees); });
 }
 
 int mvsim_attenuate(mvsim_ctx* ctx, const float* in, float* out, const int64_t dims[3], double delta, int strict_reference)
@@ -772,14 +802,10 @@ int mvsim_attenuate(mvsim_ctx* ctx, const float* in, float* out, const int64_t d
     MVSIM_ENTER(ctx);
     if (!in || !out) return set_error(ctx, MVSIM_EINVAL, "attenuate: null buffer");
     MVSIM_TRY(check_dims(ctx, dims, "attenuate"));
-    const size_t bytes = elems(dims) * sizeof(float);
-    DevBuf a(ctx), b(ctx);
-    MVSIM_TRY(a.alloc(bytes));
-    MVSIM_TRY(b.alloc(bytes));
-    MVSIM_TRY(h2d(ctx, a.p, in, bytes));
-    MVSIM_TRY(dev_attenuate(ctx, a.f(), b.f(), dims, delta, strict_reference));
-    MVSIM_TRY(d2h(ctx, out, b.p, bytes));
-    return sync(ctx);
+    HostCall hc(ctx);
+    const float* a = hc.in(in, elems(dims));
+    float* b = hc.out(out, elems(dims));
+    return hc.run([&] { return dev_attenuate(ctx, a, b, dims, delta, strict_reference); });
 }
 
 int mvsim_psf_normalize(mvsim_ctx* ctx, float* psf, const int64_t kdims[3], double* sum_out)
@@ -787,16 +813,10 @@ int mvsim_psf_normalize(mvsim_ctx* ctx, float* psf, const int64_t kdims[3], doub
     MVSIM_ENTER(ctx);
     if (!psf) return set_error(ctx, MVSIM_EINVAL, "psf_normalize: null buffer");
     MVSIM_TRY(check_dims(ctx, kdims, "psf_normalize"));
-    const size_t bytes = elems(kdims) * sizeof(float);
-    DevBuf a(ctx);
-    MVSIM_TRY(a.alloc(bytes));
-    MVSIM_TRY(h2d(ctx, a.p, psf, bytes));
-    MVSIM_TRY(dev_psf_normalize(ctx, a.f(), elems(kdims)));
-    MVSIM_TRY(d2h(ctx, psf, a.p, bytes));
-    double s = 0;
-    MVSIM_TRY(read_scalar(ctx, 0, &s));
-    if (sum_out) *sum_out = s;
-    return MVSIM_OK;
+    HostCall hc(ctx);
+    float* a = hc.inout(psf, elems(kdims));
+    hc.scalar(0, sum_out);
+    return hc.run([&] { return dev_psf_normalize(ctx, a, elems(kdims)); });
 }
 
 int mvsim_convolve(mvsim_ctx* ctx, const float* img, const int64_t dims[3], float* psf, const int64_t kdims[3], float* out)
@@ -805,18 +825,14 @@ int mvsim_convolve(mvsim_ctx* ctx, const float* img, const int64_t dims[3], floa
     if (!img || !psf || !out) return set_error(ctx, MVSIM_EINVAL, "convolve: null buffer");
     MVSIM_TRY(check_dims(ctx, dims, "convolve dims"));
     MVSIM_TRY(check_dims(ctx, kdims, "convolve kdims"));
-    const size_t bytes = elems(dims) * sizeof(float), kbytes = elems(kdims) * sizeof(float);
-    DevBuf a(ctx), b(ctx), k(ctx);
-    MVSIM_TRY(a.alloc(bytes));
-    MVSIM_TRY(b.alloc(bytes));
-    MVSIM_TRY(k.alloc(kbytes));
-    MVSIM_TRY(h2d(ctx, a.p, img, bytes));
-    MVSIM_TRY(h2d(ctx, k.p, psf, kbytes));
-    MVSIM_TRY(dev_psf_normalize(ctx, k.f(), elems(kdims)));
-    MVSIM_TRY(conv_device(ctx, a.f(), dims, k.f(), kdims, b.f(), nullptr));
-    MVSIM_TRY(d2h(ctx, psf, k.p, kbytes));          // in-place normalisation is part of the contract (:255)
-    MVSIM_TRY(d2h(ctx, out, b.p, bytes));
-    return sync(ctx);
+    HostCall hc(ctx);
+    const float* a = hc.in(img, elems(dims));
+    float* b = hc.out(out, elems(dims));
+    float* k = hc.inout(psf, elems(kdims));          // in-place normalisation is part of the contract (:255)
+    return hc.run([&] {
+        MVSIM_TRY(dev_psf_normalize(ctx, k, elems(kdims)));
+        return conv_device(ctx, a, dims, k, kdims, b, nullptr);
+    });
 }
 
 int mvsim_adjust(mvsim_ctx* ctx, float* img, const int64_t dims[3], float min_value, float target_avg, double* correction_out)
@@ -824,36 +840,21 @@ int mvsim_adjust(mvsim_ctx* ctx, float* img, const int64_t dims[3], float min_va
     MVSIM_ENTER(ctx);
     if (!img) return set_error(ctx, MVSIM_EINVAL, "adjust: null buffer");
     MVSIM_TRY(check_dims(ctx, dims, "adjust"));
-    const size_t bytes = elems(dims) * sizeof(float);
-    DevBuf a(ctx);
-    MVSIM_TRY(a.alloc(bytes));
-    MVSIM_TRY(h2d(ctx, a.p, img, bytes));
-    MVSIM_TRY(dev_adjust(ctx, a.f(), elems(dims), min_value, target_avg));
-    MVSIM_TRY(d2h(ctx, img, a.p, bytes));
-    double c = 0;
-    MVSIM_TRY(read_scalar(ctx, 2, &c));
-    if (correction_out) *correction_out = c;
-    return MVSIM_OK;
+    HostCall hc(ctx);
+    float* a = hc.inout(img, elems(dims));
+    hc.scalar(2, correction_out);
+    return hc.run([&] { return dev_adjust(ctx, a, elems(dims), min_value, target_avg); });
 }
 
 int mvsim_extract_slices(mvsim_ctx* ctx, const float* in, const int64_t dims[3], int inc, float snr, uint64_t seed, uint64_t stream, float* out)
 {
     MVSIM_ENTER(ctx);
     if (!in || !out) return set_error(ctx, MVSIM_EINVAL, "extract_slices: null buffer");
-    MVSIM_TRY(check_dims(ctx, dims, "extract_slices"));
-    if (inc < 1) return set_error(ctx, MVSIM_EINVAL, "extract_slices: inc must be >= 1");
-    const size_t bytes = elems(dims) * sizeof(float);
-    const size_t obytes = kept_elems(dims, inc) * sizeof(float);
-    DevBuf a(ctx), b(ctx);
-    MVSIM_TRY(a.alloc(bytes));
-    MVSIM_TRY(b.alloc(obytes));
-    MVSIM_TRY(h2d(ctx, a.p, in, bytes));
-    {
-        StageTimer t(ctx, MVSIM_T_SAMPLE);
-        MVSIM_TRY(k_extract(ctx, a.f(), dims, inc, nullptr, 0.f, snr, seed, stream, b.f()));
-    }
-    MVSIM_TRY(d2h(ctx, out, b.p, obytes));
-    return sync(ctx);
+    MVSIM_TRY(check_sampling(ctx, dims, inc, "extract_slices"));
+    HostCall hc(ctx);
+    const float* a = hc.in(in, elems(dims));
+    float* b = hc.out(out, kept_elems(dims, inc));
+    return hc.run([&] { return dev_extract_slices(ctx, a, dims, inc, snr, seed, stream, b); });
 }
 
 int mvsim_poisson(mvsim_ctx* ctx, float* inout, size_t n, double snr, uint64_t seed, uint64_t stream)
@@ -861,15 +862,12 @@ int mvsim_poisson(mvsim_ctx* ctx, float* inout, size_t n, double snr, uint64_t s
     MVSIM_ENTER(ctx);
     if (!inout && n) return set_error(ctx, MVSIM_EINVAL, "poisson: null buffer");
     if (n == 0) return MVSIM_OK;
-    DevBuf a(ctx);
-    MVSIM_TRY(a.alloc(n * sizeof(float)));
-    MVSIM_TRY(h2d(ctx, a.p, inout, n * sizeof(float)));
-    {
+    HostCall hc(ctx);
+    float* a = hc.inout(inout, n);
+    return hc.run([&] {
         StageTimer t(ctx, MVSIM_T_SAMPLE);
-        MVSIM_TRY(k_poisson(ctx, a.f(), n, snr, seed, stream));
-    }
-    MVSIM_TRY(d2h(ctx, inout, a.p, n * sizeof(float)));
-    return sync(ctx);
+        return k_poisson(ctx, a, n, snr, seed, stream);
+    });
 }
 
 int mvsim_simulate_view(mvsim_ctx* ctx, const mvsim_view_params* p, const float* gt, float* psf, float* out)
@@ -877,18 +875,11 @@ int mvsim_simulate_view(mvsim_ctx* ctx, const mvsim_view_params* p, const float*
     MVSIM_ENTER(ctx);
     MVSIM_TRY(check_view(ctx, p));
     if (!gt || !psf || !out) return set_error(ctx, MVSIM_EINVAL, "simulate_view: null buffer");
-    const size_t bytes = elems(p->dims) * sizeof(float), kbytes = elems(p->kdims) * sizeof(float);
-    const size_t obytes = kept_elems(p->dims, p->inc) * sizeof(float);
-    DevBuf g(ctx), k(ctx), o(ctx);
-    MVSIM_TRY(g.alloc(bytes));
-    MVSIM_TRY(k.alloc(kbytes));
-    MVSIM_TRY(o.alloc(obytes));
-    MVSIM_TRY(h2d(ctx, g.p, gt, bytes));
-    MVSIM_TRY(h2d(ctx, k.p, psf, kbytes));
-    MVSIM_TRY(dev_simulate_view(ctx, p, g.f(), k.f(), o.f()));
-    MVSIM_TRY(d2h(ctx, psf, k.p, kbytes));
-    MVSIM_TRY(d2h(ctx, out, o.p, obytes));
-    return sync(ctx);
+    HostCall hc(ctx);
+    const float* g = hc.in(gt, elems(p->dims));
+    float* k = hc.inout(psf, elems(p->kdims));
+    float* o = hc.out(out, kept_elems(p->dims, p->inc));
+    return hc.run([&] { return dev_simulate_view(ctx, p, g, k, o); });
 }
 
 // gt: host ground truth (uploaded under the upload gate) or, when vol is given, already resident on the device
@@ -1010,17 +1001,11 @@ int mvsim_make_isotropic(mvsim_ctx* ctx, const float* in, const int64_t dims[3],
 {
     MVSIM_ENTER(ctx);
     if (!in || !out) return set_error(ctx, MVSIM_EINVAL, "make_isotropic: null buffer");
-    MVSIM_TRY(check_dims(ctx, dims, "make_isotropic"));
-    if (inc < 1) return set_error(ctx, MVSIM_EINVAL, "make_isotropic: inc must be >= 1");
-    const size_t bytes = elems(dims) * sizeof(float);
-    const size_t obytes = (size_t)(dims[0] * dims[1] * ((dims[2] - 1) * inc + 1)) * sizeof(float);
-    DevBuf a(ctx), b(ctx);
-    MVSIM_TRY(a.alloc(bytes));
-    MVSIM_TRY(b.alloc(obytes));
-    MVSIM_TRY(h2d(ctx, a.p, in, bytes));
-    MVSIM_TRY(k_make_isotropic(ctx, a.f(), dims, inc, b.f()));
-    MVSIM_TRY(d2h(ctx, out, b.p, obytes));
-    return sync(ctx);
+    MVSIM_TRY(check_sampling(ctx, dims, inc, "make_isotropic"));
+    HostCall hc(ctx);
+    const float* a = hc.in(in, elems(dims));
+    float* b = hc.out(out, (size_t)(dims[0] * dims[1] * ((dims[2] - 1) * inc + 1)));
+    return hc.run([&] { return k_make_isotropic(ctx, a, dims, inc, b); });
 }
 
 int mvsim_weight_image(mvsim_ctx* ctx, const int64_t dims[3], float* out)
@@ -1028,12 +1013,9 @@ int mvsim_weight_image(mvsim_ctx* ctx, const int64_t dims[3], float* out)
     MVSIM_ENTER(ctx);
     if (!out) return set_error(ctx, MVSIM_EINVAL, "weight_image: null buffer");
     MVSIM_TRY(check_dims(ctx, dims, "weight_image"));
-    const size_t bytes = elems(dims) * sizeof(float);
-    DevBuf a(ctx);
-    MVSIM_TRY(a.alloc(bytes));
-    MVSIM_TRY(k_weight_image(ctx, dims, a.f()));
-    MVSIM_TRY(d2h(ctx, out, a.p, bytes));
-    return sync(ctx);
+    HostCall hc(ctx);
+    float* a = hc.out(out, elems(dims));
+    return hc.run([&] { return k_weight_image(ctx, dims, a); });
 }
 
 int mvsim_normalize_weights(mvsim_ctx* ctx, float* const* weights, int n_views, const int64_t dims[3], float osem, float* sum_out)
@@ -1043,18 +1025,11 @@ int mvsim_normalize_weights(mvsim_ctx* ctx, float* const* weights, int n_views, 
     MVSIM_TRY(check_dims(ctx, dims, "normalize_weights"));
     for (int v = 0; v < n_views; ++v)
         if (!weights[v]) return set_error(ctx, MVSIM_EINVAL, "normalize_weights: null buffer");
-    const size_t n = elems(dims), bytes = n * sizeof(float);
-    DevBufs bufs(ctx);
+    HostCall hc(ctx);
     float* d[MVSIM_MAX_WEIGHT_VIEWS] = {};
-    for (int v = 0; v < n_views; ++v) d[v] = bufs.alloc<float>(n);
-    float* dsum = sum_out ? bufs.alloc<float>(n) : nullptr;
-    int st = bufs.st;
-    for (int v = 0; v < n_views && st == MVSIM_OK; ++v) st = h2d(ctx, d[v], weights[v], bytes);
-    if (st == MVSIM_OK) st = k_normalize_weights(ctx, d, n_views, n, osem, dsum);
-    for (int v = 0; v < n_views && st == MVSIM_OK; ++v) st = d2h(ctx, weights[v], d[v], bytes);
-    if (st == MVSIM_OK && sum_out) st = d2h(ctx, sum_out, dsum, bytes);
-    const int st2 = sync(ctx);
-    return st != MVSIM_OK ? st : st2;
+    for (int v = 0; v < n_views; ++v) d[v] = hc.inout(weights[v], elems(dims));
+    float* dsum = sum_out ? hc.out(sum_out, elems(dims)) : nullptr;
+    return hc.run([&] { return k_normalize_weights(ctx, d, n_views, elems(dims), osem, dsum); });
 }
 
 // ---- input generators either side of the path (SURVEY section 8f rows 2-4) -------------------------
@@ -1129,10 +1104,17 @@ static int dev_simulate_phantom(mvsim_ctx* ctx, int size, int half_pixel, int64_
     const int scale = 2;
     const int64_t big = (int64_t)(size + 1) * scale;
     const int64_t dims[3] = { big, big, big };
-    DevBuf a(ctx);
-    MVSIM_TRY(a.alloc((size_t)(big * big * big) * sizeof(float)));
-    MVSIM_TRY(dev_draw_spheres(ctx, dims, 0.0, 1.0, scale, half_pixel, seed, a.f(), n_small));
-    return k_downsample2x(ctx, a.f(), dims, d_out);
+    DevBufs bufs(ctx);
+    float* a = bufs.alloc<float>((size_t)(big * big * big));
+    MVSIM_TRY(bufs.st);
+    MVSIM_TRY(dev_draw_spheres(ctx, dims, 0.0, 1.0, scale, half_pixel, seed, a, n_small));
+    return k_downsample2x(ctx, a, dims, d_out);
+}
+
+static int check_phantom_size(mvsim_ctx* ctx, int size)
+{
+    if (size < 1 || size > 2047) return set_error(ctx, MVSIM_EINVAL, "simulate_phantom: size must be in 1..2047");
+    return MVSIM_OK;
 }
 }  // namespace mvsim
 using namespace mvsim;
@@ -1177,11 +1159,9 @@ int mvsim_render_beads(mvsim_ctx* ctx, const double* points, int n, const double
     int64_t dims[3];
     MVSIM_TRY(check_bead_args(ctx, points, n, sigma, imin, imax, dims));
     if (!out) return set_error(ctx, MVSIM_EINVAL, "render_beads: null buffer");
-    DevBuf a(ctx);
-    MVSIM_TRY(a.alloc(elems(dims) * sizeof(float)));
-    MVSIM_TRY(k_render_beads(ctx, points, n, sigma, imin, imax, a.f()));
-    MVSIM_TRY(d2h(ctx, out, a.p, elems(dims) * sizeof(float)));
-    return sync(ctx);
+    HostCall hc(ctx);
+    float* a = hc.out(out, elems(dims));
+    return hc.run([&] { return k_render_beads(ctx, points, n, sigma, imin, imax, a); });
 }
 
 int mvsim_dev_render_beads(mvsim_ctx* ctx, const double* points, int n, const double sigma[3], const int64_t imin[3], const int64_t imax[3], mvsim_volume* out)
@@ -1200,11 +1180,9 @@ int mvsim_draw_spheres(mvsim_ctx* ctx, const int64_t dims[3], double min_value, 
     MVSIM_ENTER(ctx);
     if (!out) return set_error(ctx, MVSIM_EINVAL, "draw_spheres: null buffer");
     MVSIM_TRY(check_dims(ctx, dims, "draw_spheres"));
-    DevBuf a(ctx);
-    MVSIM_TRY(a.alloc(elems(dims) * sizeof(float)));
-    MVSIM_TRY(dev_draw_spheres(ctx, dims, min_value, max_value, scale, half_pixel, seed, a.f(), n_small));
-    MVSIM_TRY(d2h(ctx, out, a.p, elems(dims) * sizeof(float)));
-    return sync(ctx);
+    HostCall hc(ctx);
+    float* a = hc.out(out, elems(dims));
+    return hc.run([&] { return dev_draw_spheres(ctx, dims, min_value, max_value, scale, half_pixel, seed, a, n_small); });
 }
 
 int mvsim_downsample2x(mvsim_ctx* ctx, const float* in, const int64_t dims[3], float* out)
@@ -1213,33 +1191,26 @@ int mvsim_downsample2x(mvsim_ctx* ctx, const float* in, const int64_t dims[3], f
     if (!in || !out) return set_error(ctx, MVSIM_EINVAL, "downsample2x: null buffer");
     MVSIM_TRY(check_dims(ctx, dims, "downsample2x"));
     if (dims[0] < 4 || dims[1] < 4 || dims[2] < 4) return set_error(ctx, MVSIM_EINVAL, "downsample2x: dims must be >= 4 (output is dims/2 - 1)");
-    const size_t obytes = (size_t)((dims[0] / 2 - 1) * (dims[1] / 2 - 1) * (dims[2] / 2 - 1)) * sizeof(float);
-    DevBuf a(ctx), b(ctx);
-    MVSIM_TRY(a.alloc(elems(dims) * sizeof(float)));
-    MVSIM_TRY(b.alloc(obytes));
-    MVSIM_TRY(h2d(ctx, a.p, in, elems(dims) * sizeof(float)));
-    MVSIM_TRY(k_downsample2x(ctx, a.f(), dims, b.f()));
-    MVSIM_TRY(d2h(ctx, out, b.p, obytes));
-    return sync(ctx);
+    HostCall hc(ctx);
+    const float* a = hc.in(in, elems(dims));
+    float* b = hc.out(out, (size_t)((dims[0] / 2 - 1) * (dims[1] / 2 - 1) * (dims[2] / 2 - 1)));
+    return hc.run([&] { return k_downsample2x(ctx, a, dims, b); });
 }
 
 int mvsim_simulate_phantom(mvsim_ctx* ctx, int size, int half_pixel, int64_t seed, float* out, int64_t* n_small)
 {
     MVSIM_ENTER(ctx);
     if (!out) return set_error(ctx, MVSIM_EINVAL, "simulate_phantom: null buffer");
-    if (size < 1 || size > 2047) return set_error(ctx, MVSIM_EINVAL, "simulate_phantom: size must be in 1..2047");
-    const size_t obytes = (size_t)size * size * size * sizeof(float);
-    DevBuf b(ctx);
-    MVSIM_TRY(b.alloc(obytes));
-    MVSIM_TRY(dev_simulate_phantom(ctx, size, half_pixel, seed, b.f(), n_small));
-    MVSIM_TRY(d2h(ctx, out, b.p, obytes));
-    return sync(ctx);
+    MVSIM_TRY(check_phantom_size(ctx, size));
+    HostCall hc(ctx);
+    float* b = hc.out(out, (size_t)size * size * size);
+    return hc.run([&] { return dev_simulate_phantom(ctx, size, half_pixel, seed, b, n_small); });
 }
 
 int mvsim_dev_simulate_phantom(mvsim_ctx* ctx, int size, int half_pixel, int64_t seed, mvsim_volume* out, int64_t* n_small)
 {
     MVSIM_ENTER(ctx);
-    if (size < 1 || size > 2047) return set_error(ctx, MVSIM_EINVAL, "simulate_phantom: size must be in 1..2047");
+    MVSIM_TRY(check_phantom_size(ctx, size));
     if (!out || out->dims[0] != size || out->dims[1] != size || out->dims[2] != size)
         return set_error(ctx, MVSIM_EINVAL, "simulate_phantom: output volume must be size^3");
     return dev_simulate_phantom(ctx, size, half_pixel, seed, out->d, n_small);
@@ -1252,13 +1223,10 @@ int mvsim_make_square(mvsim_ctx* ctx, const float* in, const int64_t dims[3], fl
     MVSIM_TRY(check_dims(ctx, dims, "make_square"));
     const int64_t m = dims[0] > dims[1] ? (dims[0] > dims[2] ? dims[0] : dims[2]) : (dims[1] > dims[2] ? dims[1] : dims[2]);
     if (m > 4096) return set_error(ctx, MVSIM_EINVAL, "make_square: dims too large");
-    DevBuf a(ctx), b(ctx);
-    MVSIM_TRY(a.alloc(elems(dims) * sizeof(float)));
-    MVSIM_TRY(b.alloc((size_t)(m * m * m) * sizeof(float)));
-    MVSIM_TRY(h2d(ctx, a.p, in, elems(dims) * sizeof(float)));
-    MVSIM_TRY(k_make_square(ctx, a.f(), dims, b.f()));
-    MVSIM_TRY(d2h(ctx, out, b.p, (size_t)(m * m * m) * sizeof(float)));
-    return sync(ctx);
+    HostCall hc(ctx);
+    const float* a = hc.in(in, elems(dims));
+    float* b = hc.out(out, (size_t)(m * m * m));
+    return hc.run([&] { return k_make_square(ctx, a, dims, b); });
 }
 
 // ---- device-resident volumes ------------------------------------------------------------------
@@ -1373,11 +1341,11 @@ int mvsim_dev_adjust(mvsim_ctx* ctx, mvsim_volume* img, float min_value, float t
 int mvsim_dev_extract_slices(mvsim_ctx* ctx, const mvsim_volume* in, int inc, float snr, uint64_t seed, uint64_t stream, mvsim_volume* out)
 {
     MVSIM_ENTER(ctx);
-    if (!in || !out || inc < 1) return set_error(ctx, MVSIM_EINVAL, "dev_extract_slices: bad argument");
+    if (!in || !out) return set_error(ctx, MVSIM_EINVAL, "dev_extract_slices: null volume");
+    MVSIM_TRY(check_sampling(ctx, in->dims, inc, "dev_extract_slices"));
     if (out->dims[0] != in->dims[0] || out->dims[1] != in->dims[1] || out->dims[2] != kept_planes(in->dims, inc))
         return set_error(ctx, MVSIM_EINVAL, "dev_extract_slices: out dims must be (X, Y, (Z-1)/inc+1)");
-    StageTimer t(ctx, MVSIM_T_SAMPLE);
-    return k_extract(ctx, in->d, in->dims, inc, nullptr, 0.f, snr, seed, stream, out->d);
+    return dev_extract_slices(ctx, in->d, in->dims, inc, snr, seed, stream, out->d);
 }
 
 int mvsim_dev_extract_interval(mvsim_ctx* ctx, const mvsim_volume* in, const int64_t min[3], const int64_t max[3], int inc,
@@ -1585,12 +1553,8 @@ int mvsim_slab_rotate_attenuate(mvsim_ctx* ctx, const float* d_gt, const int64_t
     if (!d_gt || !d_out_slab) return set_error(ctx, MVSIM_EINVAL, "slab_rotate_attenuate: null buffer");
     MVSIM_TRY(check_dims(ctx, dims, "slab_rotate_attenuate"));
     if (z0 < 0 || z_local < 1 || z0 + z_local > dims[2]) return set_error(ctx, MVSIM_EINVAL, "slab_rotate_attenuate: slab outside the volume");
-    double inv[12];
-    int steps = 0;
-    if (axis_rotation(dims, axis, degrees, nullptr, inv)) return set_error(ctx, MVSIM_EINVAL, "slab_rotate_attenuate: axis must be 0, 1 or 2");
-    MVSIM_TRY(attenuate_steps(ctx, dims, strict_reference, &steps));
-    StageTimer t(ctx, MVSIM_T_ROTATE);
-    const int st = k_rotate_attenuate(ctx, d_gt, d_out_slab, dims, axis, inv, delta, steps, z0, z_local);
+    if (axis < 0 || axis > 2) return set_error(ctx, MVSIM_EINVAL, "slab_rotate_attenuate: axis must be 0, 1 or 2");
+    const int st = dev_rotate_attenuate(ctx, d_gt, d_out_slab, dims, axis, degrees, delta, strict_reference, z0, z_local);
     if (st == MVSIM_EUNSUPPORTED) return set_error(ctx, MVSIM_EUNSUPPORTED, "slab_rotate_attenuate: only rotations about axis 0 (the reference's) are decomposed");
     return st;
 }

@@ -232,23 +232,6 @@ struct CudaLauncher {
     }
 };
 
-struct Buffers {
-    mvsim_ctx* ctx;
-    void* p[8];
-    int n;
-    explicit Buffers(mvsim_ctx* c) : ctx(c), n(0) {}
-    ~Buffers() { for (int i = 0; i < n; ++i) dev_free(ctx, p[i]); }
-    template <class T> int get(T** out, size_t elems)
-    {
-        void* q = nullptr;
-        int st = dev_alloc(ctx, &q, elems * sizeof(T));
-        if (st) return st;
-        p[n++] = q;
-        *out = static_cast<T*>(q);
-        return MVSIM_OK;
-    }
-};
-
 }  // namespace
 
 int strided_lanes() { return 8; }
@@ -315,14 +298,13 @@ int conv_device(mvsim_ctx* ctx, const float* img, const int64_t dims[3], const f
     MVSIM_TRY(get_tables(ctx, pl.sy.n, &ty));
     MVSIM_TRY(get_tables(ctx, pl.sz.n, &tz));
 
-    Buffers buf(ctx);
+    DevBufs buf(ctx);
     ConvWorkspace ws = {};
-    MVSIM_TRY(buf.get(&ws.u1, (size_t)pl.u1_elems(g.z_local)));
-    ws.u1o = ws.u1;
-    if (pl.y_blocks > 1) MVSIM_TRY(buf.get(&ws.u1o, (size_t)pl.u1_elems(g.z_local)));   // blocks still read halo rows of u1
-    MVSIM_TRY(buf.get(&ws.u2, (size_t)pl.u2_elems(lanes, g.z_local)));
-    ws.ex = ws.u2;
-    if (!otf_default()) MVSIM_TRY(buf.get(&ws.h, (size_t)pl.h_elems(lanes, g.tiles_own)));
+    ws.u1 = ws.u1o = buf.alloc<float2>((size_t)pl.u1_elems(g.z_local));
+    if (pl.y_blocks > 1) ws.u1o = buf.alloc<float2>((size_t)pl.u1_elems(g.z_local));   // blocks still read halo rows of u1
+    ws.u2 = ws.ex = buf.alloc<float2>((size_t)pl.u2_elems(lanes, g.z_local));
+    if (!otf_default()) ws.h = buf.alloc<float2>((size_t)pl.h_elems(lanes, g.tiles_own));
+    MVSIM_TRY(buf.st);
     // PSF partial spectrum: from the cache when this (normalised) PSF has been seen with this plan, else computed -- into a
     // cache-owned buffer when the cache is on, into a pool buffer otherwise
     bool psf_hit = false;
@@ -331,17 +313,16 @@ int conv_device(mvsim_ctx* ctx, const float* img, const int64_t dims[3], const f
         StageTimer t(ctx, MVSIM_T_PSF);
         MVSIM_TRY(psf_cache_lookup(ctx, psf, pl, lanes, (size_t)pl.p2_elems(lanes, g.tiles_own), &cached, &psf_hit));
     }
-    if (cached) ws.p2 = cached;
-    else MVSIM_TRY(buf.get(&ws.p2, (size_t)pl.p2_elems(lanes, g.tiles_own)));
-    if (!psf_hit) MVSIM_TRY(buf.get(&ws.p1, (size_t)pl.p1_elems()));
+    ws.p2 = cached ? cached : buf.alloc<float2>((size_t)pl.p2_elems(lanes, g.tiles_own));
+    if (!psf_hit) ws.p1 = buf.alloc<float2>((size_t)pl.p1_elems());
     ws.tw_x = tx.tw; ws.twist_x = tx.twist; ws.tw_y = ty.tw; ws.tw_z = tz.tw;
 
     CudaLauncher l = { ctx, true, lanes };
-    double* partials = nullptr;
     const int planes = conv_out_planes(pl, g, keep_inc);
     if (out_planes) *out_planes = planes;
     const int nblocks = CudaLauncher::x_blocks(pl.sx, pl.dims[1] * planes, true);      // per-block sums of the inverse x pass
-    if (d_sum) MVSIM_TRY(buf.get(&partials, (size_t)nblocks));
+    double* partials = d_sum ? buf.alloc<double>((size_t)nblocks) : nullptr;
+    MVSIM_TRY(buf.st);
     if (!psf_hit) MVSIM_TRY(conv_psf_spectrum(l, pl, g, ws, psf));
     l.psf_phase = false;
     MVSIM_TRY(conv_apply(l, pl, g, ws, img, out, partials, keep_inc));

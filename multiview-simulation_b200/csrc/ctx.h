@@ -106,6 +106,23 @@ int dev_alloc(mvsim_ctx* ctx, void** p, size_t bytes);      // stream-ordered (c
 void dev_free(mvsim_ctx* ctx, void* p);
 int get_tables(mvsim_ctx* ctx, int n, mvsim_tables* t);
 
+// device buffers of one call with a deferred failure: after the first failed allocation alloc() returns null and st keeps that
+// status, so a call allocates all it needs and checks once
+struct DevBufs {
+    mvsim_ctx* ctx;
+    int st = MVSIM_OK;
+    std::vector<void*> held;
+    explicit DevBufs(mvsim_ctx* c) : ctx(c) {}
+    ~DevBufs() { free_all(); }
+    template <class T> T* alloc(size_t n)
+    {
+        void* q = nullptr;
+        if (st == MVSIM_OK && (st = dev_alloc(ctx, &q, n * sizeof(T))) == MVSIM_OK) held.push_back(q);
+        return static_cast<T*>(q);
+    }
+    void free_all() { for (void* q : held) dev_free(ctx, q); held.clear(); }
+};
+
 // stage kernels (stages.cu); all enqueue on ctx->stream
 int k_rotate(mvsim_ctx* ctx, const float* in, float* out, const int64_t dims[3], int axis, const double inv[12]);
 // fused; MVSIM_EUNSUPPORTED when the rotation is not the axis-0 fast path.  z_local > 0: only the output planes [z0, z0 + z_local)
